@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark of the B200 duplicate-detection hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload of the headline line (BASELINE.json configs[1]): batched fingerprint forward of 10 000 synthetic clips x 64
 frames @ 64x64 per GPU, bf16 frames resident in HBM, random-init weights of the reference architecture. One "step" = one
@@ -24,6 +24,9 @@ One JSON line on stdout (rank 0):
   cfg4_join    BASELINE configs[3]: 1 048 576 rows in total, row-block sharded, NCCL all-gather overlapped with the
                local block (strong scaling), parity spot-check against an fp32 matmul
   cfg5_topk    BASELINE configs[4]: top-10 of 100 000 queries (sharded) against 10 000 000 database rows
+`--dump-outputs DIR` (git ignores bench_outputs/) writes the embeddings the last timed step returned (rank 0) as
+DIR/embeddings.npy, float32; the inputs are seeded, so two builds run with the same arguments can be compared output for
+output.
 `--impl reference` times the reference algorithm's CPU path (oracle port; the reference itself is not installable on the
 GPU box) on the same config.
 """
@@ -484,6 +487,22 @@ def bench_cfg5_topk(vfp, world, rank, dev, peaks, n_db: int, n_q: int, k: int, r
     }
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Each array as float32 out_dir/<name>.npy. An array larger than its share of 64 MB is reduced to a fixed sample of
+    its rows (seeded: the same rows in every run for the same shape)."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            rows = np.random.default_rng(0).choice(a.shape[0], share // (a.nbytes // a.shape[0]), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------------------------------
 # our arm
 # --------------------------------------------------------------------------------------------------
@@ -643,6 +662,8 @@ def run_ours(args):
         sampler.stop()
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"embeddings": emb})
     # ---- roofline of the dominant kernel ----
     known = [k for k in stages if (k in STAGE_FLOPS or k in STAGE_BYTES) and stages[k] > 0]
     dom = max(known, key=lambda k: stages[k])
@@ -724,7 +745,12 @@ def main():
     ap.add_argument("--no-cfg4", action="store_true")
     ap.add_argument("--no-cfg5", action="store_true")
     ap.add_argument("--forward-only", action="store_true", help="skip e2e, joins, cfg 3-5 and the CPU baseline (kernel experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the embeddings of the last timed step to DIR/embeddings.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.forward_only:
         args.no_e2e = args.no_join = args.no_cpu = args.no_cfg3 = args.no_cfg4 = args.no_cfg5 = True
     if args.impl == "reference":

@@ -16,10 +16,9 @@ reference's attention-model inference forward:
     /root/reference/fingerprint.py:232-270  per-video B=1 semantics -> ``fingerprint_clips``
     /root/reference/fingerprint.py:90-101   frame subsampling rule   -> ``subsample_indices``
 
-Parity pin: ``tests/golden/make_golden.py`` runs the UNMODIFIED reference module (imported from
-/root/reference in the build container) on seeded weights/inputs and stores its outputs under
-``tests/golden/``; ``tests/test_oracle.py`` checks this restatement against those files (and, when
-/root/reference is present, against the live reference as well).
+Parity pin: ``tests/golden/make_golden.py`` runs the UNMODIFIED reference module on seeded weights/inputs
+and stores its outputs (embeddings and pooled features) under ``tests/golden/``; ``tests/test_oracle.py``
+checks this restatement against those files.
 """
 from __future__ import annotations
 

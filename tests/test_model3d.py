@@ -1,9 +1,12 @@
 """3-D CNN fingerprint model (SURVEY.md section 8f rank 4; /root/reference/model.py:406-512).
 
-CPU: the fp32 oracle against the golden embeddings of the UNMODIFIED reference module (tests/golden/forward3d.npz), state_dict
-layout / default initialisation of the host mirror against the reference. GPU (-m gpu): vfp3d_forward through the C ABI against the
+CPU: the fp32 oracle against the golden embeddings of the UNMODIFIED reference module (tests/golden/forward3d.npz); the
+host mirror's default initialisation against the reference through the refinit case of that file, and its state_dict layout
+against the oracle's and against the recorded layout and initial values of a non-default configuration
+(tests/golden/host_mirror_3d.json). GPU (-m gpu): vfp3d_forward through the C ABI against the
 golden file and the oracle. Tolerance: cosine >= 0.9999 per embedding (bf16 operands, fp32 accumulation), like the attention model.
 """
+import json
 import os
 import sys
 
@@ -14,6 +17,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import forward3d_oracle as fo  # noqa: E402
+from oracle.weights import state_dict_digest  # noqa: E402
 
 GOLD = np.load(os.path.join(ROOT, "tests", "golden", "forward3d.npz"))
 COS_BAR = 0.9999
@@ -53,16 +57,13 @@ def test_host_mirror_layout():
     want = fo.make_state_dict_3d(1, 16)
     assert set(sd) == set(want) and all(sd[k].shape == want[k].shape for k in sd)
     m.load_state_dict(want, strict=True)
-    if os.path.exists("/root/reference/model.py"):
-        sys.path.insert(0, "/root/reference")
-        import model as ref_model
-
-        torch.manual_seed(3)
-        r = ref_model.create_model("3d", frame_stride=32, embedding_dim=128)
-        torch.manual_seed(3)
-        o = vfp.create_model("3d", frame_stride=32, embedding_dim=128)
-        assert list(r.state_dict()) == list(o.state_dict())
-        assert all(torch.equal(a, b) for a, b in zip(r.state_dict().values(), o.state_dict().values()))
+    # non-default factory arguments: key order, shapes and initial values as recorded in tests/golden/host_mirror_3d.json
+    with open(os.path.join(ROOT, "tests", "golden", "host_mirror_3d.json")) as f:
+        rec = json.load(f)
+    torch.manual_seed(3)
+    o = vfp.create_model("3d", frame_stride=32, embedding_dim=128).state_dict()
+    assert list(o) == rec["keys"] and [list(v.shape) for v in o.values()] == rec["shapes"]
+    assert state_dict_digest(o) == rec["weights_sha256"]
 
 
 @pytest.mark.gpu
