@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define VFP_ABI_VERSION 2
+#define VFP_ABI_VERSION 3
 
 /* frame element types accepted by vfp_forward (planar (T,3,64,64) frames as produced by
  * _preprocess_frames, fingerprint.py:186-214; U8 values are scaled by 1/255 on the device) */
@@ -123,6 +123,21 @@ int vfp3d_weights_embedding_dim(const vfp3d_weights* w);
 size_t vfp3d_forward_workspace_bytes(const vfp3d_weights* w, int64_t clips_per_pass, int n_frames);
 int vfp3d_forward(const vfp3d_weights* w, const void* frames, int frame_dtype, int64_t n_clips, int n_frames,
                   float* emb_out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Variable-length batches of the 3-D model, with the conventions of vfp_forward: `frames` is the packed device tensor
+ * (sum T, 3, 64, 64) planar u8 / bf16 / fp32 (VFP_FRAME_U8_HWC is rejected), clips back to back; `cu_seqlens_host` holds
+ * n_clips+1 int32 prefix sums of the clip lengths (HOST memory, cu_seqlens_host[0] = 0). Writes unit-norm embeddings
+ * (n_clips, D) fp32 to `emb_out`. Every clip is treated exactly like a B=1 vfp3d_forward on that clip alone, with the same
+ * bits: its zero padding up to a multiple of frame_stride and its temporal padding stop at its own ends, whatever surrounds
+ * it. A clip may have 1 .. 64 * frame_stride frames (at most 32 temporal positions after the strides); a clip of length 0,
+ * a longer clip, decreasing prefix sums, or a workspace too small for a clip are errors naming the clip.
+ * The call splits the input into passes on clip boundaries that fit `workspace_bytes`; results do not depend on the split.
+ * vfp3d_forward_packed_workspace_bytes bounds one pass of up to `frames_per_pass` frames in up to `clips_per_pass` clips
+ * (from sum ceil(T/fs) <= F/fs + C and sum T3 <= (sum G + C)/2); the minimum useful value is that of the longest clip
+ * (frames_per_pass = its length, clips_per_pass = 1). vfp3d_forward is this path with uniform lengths. */
+size_t vfp3d_forward_packed_workspace_bytes(const vfp3d_weights* w, int64_t frames_per_pass, int64_t clips_per_pass);
+int vfp3d_forward_packed(const vfp3d_weights* w, const void* frames, int frame_dtype, const int32_t* cu_seqlens_host,
+                         int n_clips, float* emb_out, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Frame preprocessing of the scanner (/root/reference/fingerprint.py:186-214 _preprocess_frames): cv2.resize(frame,
  * INTER_AREA) so that the short side becomes 64 (new size truncated with int() like the reference), then the centre

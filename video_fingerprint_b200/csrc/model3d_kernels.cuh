@@ -15,28 +15,35 @@
 
 namespace vfp {
 
+// Every kernel below works on a PACKED pass: clips of any lengths back to back, each activation the concatenation of the
+// clips' own activations in clip order (layer 1: sum G * 1024 rows, layer 2: sum G * 256, layer 3: sum T3 * 64, layer 4:
+// sum T3 * 16, with G = ceil(T / fs) and T3 = (G - 1) / 2 + 1 per clip). A row or CTA finds its clip through a small table the
+// host builds per pass; the arithmetic is the same as for the clip alone, so packed results equal B = 1 results bit for bit.
+// An equal-length batch is the special case of uniform clip lengths.
+
 // Layer 1: Conv3d(3 -> 16, kernel (fs, 5, 5), stride (fs, 2, 2), padding (0, 2, 2)) + folded BatchNorm3d + ReLU over planar
-// frames (B*T, 3, 64, 64) of any accepted dtype; T is zero-padded to a multiple of fs like model.py:468-471.
+// frames (sum T, 3, 64, 64) of any accepted dtype; each clip's T is zero-padded to a multiple of fs like model.py:468-471.
 // C_in = 3 makes this the same problem as the attention model's conv1 (6-byte pixels are not TMA / UMMA addressable), with
 // the same answer: the register-fragment tensor path. Per (kt, kh) the 5 x 3 (kw, c) taps of an output position are 15
 // CONSECUTIVE bf16 of a pixel-interleaved (HWC) copy of the input row (+ 1 don't-care with zero weight), so one A register of
 // mma.sync m16n8k16 is one aligned 32-bit shared load: K = 16 * 5 * fs, k = (kt*5 + kh)*16 + kw*3 + c.
-// One CTA per (b, g, oh) = 32 output positions x 16 channels: the 5 input rows x fs frames it needs are staged in shared memory
-// (68 pixels: zero halo of 2 on both sides; rows outside the image and frames past the clip end are zero), the four warps
-// split the 5*fs K runs, partial sums meet in shared memory, bias + ReLU, bf16 channels-last output [position][32] (channels
-// 16..31 zero: the 32-column box of the next layer's GEMM). An earlier version materialised the im2col matrix (2.6 GB written
+// One CTA per (global group, oh) = 32 output positions x 16 channels. groups[global group] = {first frame of the group, frames
+// of its clip from there on}: frames at or past the clip's own end read as zero, never as the next clip's first frames. The
+// 5 input rows x fs frames a CTA needs are staged in shared memory (68 pixels: zero halo of 2 on both sides; rows outside the
+// image and frames past the clip end are zero), the four warps split the 5*fs K runs, partial sums meet in shared memory,
+// bias + ReLU, bf16 channels-last output [position][32] (channels 16..31 zero: the 32-column box of the next layer's GEMM). An earlier version materialised the im2col matrix (2.6 GB written
 // and read back per 256 clips): 1.05 ms per 256 clips against 0.1 ms here.
 // wpack: [5*fs runs][2 n-tiles][32 lanes] x uint2 = the B fragments of the folded weights; bias [16].
-__global__ void __launch_bounds__(128) conv3d_l1_kernel(const void* __restrict__ frames, int frame_dtype, int T, int fs, int groups,
-                                                        const uint2* __restrict__ wpack, const float* __restrict__ bias,
+__global__ void __launch_bounds__(128) conv3d_l1_kernel(const void* __restrict__ frames, int frame_dtype, const int2* __restrict__ groups,
+                                                        int fs, const uint2* __restrict__ wpack, const float* __restrict__ bias,
                                                         __nv_bfloat16* __restrict__ out) {
   extern __shared__ __align__(16) uint8_t smem3d[];
   __nv_bfloat16* tile = reinterpret_cast<__nv_bfloat16*>(smem3d);   // [fs*5 runs][68 pixels][3 channels] (+ 2 pad elements)
   const int runs = fs * 5;
   float* part = reinterpret_cast<float*>(smem3d + (((size_t)runs * 204 * 2 + 4 + 15) & ~size_t(15)));   // [4 warps][16][32 lanes]
   const int oh = blockIdx.x & 31;
-  const int g_idx = (blockIdx.x >> 5) % groups;
-  const long long b = (blockIdx.x >> 5) / groups;
+  const unsigned gg = blockIdx.x >> 5;
+  const int2 grp = __ldg(groups + gg);   // {first frame, frames left in the clip}
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   // halo pixels (x = -2, -1, 64, 65) of every run
   for (int i = tid; i < runs * 12; i += 128) {
@@ -49,12 +56,12 @@ __global__ void __launch_bounds__(128) conv3d_l1_kernel(const void* __restrict__
   for (int i = tid; i < runs * 24; i += 128) {
     const int x0 = (i & 7) * 8, c = (i >> 3) % 3, run = i / 24;
     const int kh = run % 5, kt = run / 5;
-    const int t = g_idx * fs + kt, ih = 2 * oh + kh - 2;
+    const int ih = 2 * oh + kh - 2;
     float v[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) v[j] = 0.0f;
-    if (t < T && ih >= 0 && ih < 64) {
-      const size_t idx = (((size_t)(b * T + t) * 3 + c) * 64 + ih) * 64 + x0;
+    if (kt < grp.y && ih >= 0 && ih < 64) {
+      const size_t idx = (((size_t)(grp.x + kt) * 3 + c) * 64 + ih) * 64 + x0;
       if (frame_dtype == kFrameBF16) {
         const uint4 q = *reinterpret_cast<const uint4*>(static_cast<const __nv_bfloat16*>(frames) + idx);
         const uint32_t w[4] = {q.x, q.y, q.z, q.w};
@@ -115,7 +122,7 @@ __global__ void __launch_bounds__(128) conv3d_l1_kernel(const void* __restrict__
       for (int i = 0; i < 4; ++i) part[(warp * 16 + (mt * 2 + nt) * 4 + i) * 32 + lane] = acc[mt][nt][i];
   __syncthreads();
   // ---- reduce the four partial sums, bias + ReLU, channels-last bf16 rows of 32 (16 real channels + 16 zeros) ----
-  __nv_bfloat16* orow = out + ((size_t)(b * groups + g_idx) * 1024 + (size_t)oh * 32) * 32;
+  __nv_bfloat16* orow = out + ((size_t)gg * 1024 + (size_t)oh * 32) * 32;
   for (int o = tid; o < 32 * 8; o += 128) {         // one item = channel pair (2 * cp, 2 * cp + 1) of one position
     const int ow = o >> 3, cp = o & 7;
     // fragment coordinates of (position ow, channels 2cp, 2cp+1): mt = ow / 16, row r = ow % 16 -> g = r % 8, upper = r / 8;
@@ -134,12 +141,14 @@ __global__ void __launch_bounds__(128) conv3d_l1_kernel(const void* __restrict__
     *reinterpret_cast<uint4*>(orow + (o >> 1) * 32 + 16 + (o & 1) * 8) = make_uint4(0u, 0u, 0u, 0u);
 }
 
-// Layers 2-4: Conv3d(C -> *, kernel 3x3x3, stride (st, 2, 2), padding 1) over a channels-last activation [B][Ti][Hi][Wi][C]
-// (C a multiple of 8). Row = (b, to, oh, ow), column k = ((kt*3 + kh)*3 + kw)*C + c; one thread moves 8 channels (16 bytes).
-__global__ void im2col3d_ndhwc_kernel(const __nv_bfloat16* __restrict__ in, int B, int Ti, int Hi, int Wi, int C, int st, int To,
-                                      int Ho, int Wo, int kp, __nv_bfloat16* __restrict__ out) {
+// Layers 2-4: Conv3d(C -> *, kernel 3x3x3, stride (st, 2, 2), padding 1) over a packed channels-last activation
+// [sum Ti][Hi][Wi][C] (C a multiple of 8). Row = (output slot, oh, ow), column k = ((kt*3 + kh)*3 + kw)*C + c; one thread
+// moves 8 channels (16 bytes). slots[output slot] = {first input slot of the clip, the clip's input positions Ti, first input
+// position of the window (to * st - 1, clip-local), 0}: the temporal zero padding and the stride stop at the clip's own ends.
+__global__ void im2col3d_ndhwc_kernel(const __nv_bfloat16* __restrict__ in, const int4* __restrict__ slots, long long n_slots, int Hi,
+                                      int Wi, int C, int Ho, int Wo, int kp, __nv_bfloat16* __restrict__ out) {
   const int k8n = kp / 8;
-  const long long rows = (long long)B * To * Ho * Wo;
+  const long long rows = n_slots * Ho * Wo;
   const long long total = rows * k8n;
   const int kreal = 27 * C;
   for (long long it = (long long)blockIdx.x * blockDim.x + threadIdx.x; it < total; it += (long long)gridDim.x * blockDim.x) {
@@ -152,37 +161,38 @@ __global__ void im2col3d_ndhwc_kernel(const __nv_bfloat16* __restrict__ in, int 
       long long r = row;
       const int ow = (int)(r % Wo); r /= Wo;
       const int oh = (int)(r % Ho); r /= Ho;
-      const int to = (int)(r % To);
-      const long long b = r / To;
-      const int t = to * st + kt - 1, ih = 2 * oh + kh - 1, iw = 2 * ow + kw - 1;
-      if (t >= 0 && t < Ti && ih >= 0 && ih < Hi && iw >= 0 && iw < Wi)
-        v = *reinterpret_cast<const uint4*>(in + ((((size_t)b * Ti + t) * Hi + ih) * Wi + iw) * C + c0);
+      const int4 s = __ldg(slots + r);
+      const int t = s.z + kt, ih = 2 * oh + kh - 1, iw = 2 * ow + kw - 1;
+      if (t >= 0 && t < s.y && ih >= 0 && ih < Hi && iw >= 0 && iw < Wi)
+        v = *reinterpret_cast<const uint4*>(in + ((((size_t)s.x + t) * Hi + ih) * Wi + iw) * C + c0);
     }
     *reinterpret_cast<uint4*>(out + row * kp + k0) = v;
   }
 }
 
 struct Head3dParams {
-  const __nv_bfloat16* act;   // layer-4 output [B][T3][16][128]
-  int T3;
+  const __nv_bfloat16* act;   // packed layer-4 output [sum T3][16][128]
+  const int2* clips;          // per clip {first temporal slot in act, T3}
   const float *tc_w, *tc_b;   // temporal_conv (128, 128, 3), (128)
   const float *ta_w, *ta_b;   // temporal_attention (1, 128, 1), (1)
   const float *p0_w, *p0_b;   // projector.0 (128, 128)
   const float *p3_w, *p3_b;   // projector.3 (D, 128)
   int D;
-  float* out;                 // [B][D]
+  float* out;                 // [clips][D]
 };
 constexpr int kHead3dMaxT = 32;   // temporal positions after the two temporal strides (clips of up to 32 * 2 * fs frames)
 
-// model.py:476-509 for one clip per CTA (128 threads = one per channel)
+// model.py:476-509 for one clip per CTA (128 threads = one per channel); pooling, Conv1d padding and softmax see only that clip
 __global__ void __launch_bounds__(128) head3d_kernel(const Head3dParams p) {
   __shared__ float feat[kHead3dMaxT + 2][128];   // spatial means, rows 0 and T3+1 are the Conv1d zero padding
   __shared__ float tc[kHead3dMaxT][128];
   __shared__ float prob[kHead3dMaxT];
   __shared__ float vec[128], hid[128];
   __shared__ float red[4];
-  const int b = blockIdx.x, c = threadIdx.x, T3 = p.T3;
-  const __nv_bfloat16* a = p.act + (size_t)b * T3 * 16 * 128;
+  const int b = blockIdx.x, c = threadIdx.x;
+  const int2 clip = p.clips[b];
+  const int T3 = clip.y;
+  const __nv_bfloat16* a = p.act + (size_t)clip.x * 16 * 128;
   feat[0][c] = 0.0f;
   feat[T3 + 1][c] = 0.0f;
   for (int t = 0; t < T3; ++t) {

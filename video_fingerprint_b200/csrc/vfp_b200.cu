@@ -1342,13 +1342,140 @@ int upload3d(vfp3d_weights* w, const std::vector<T>& host, T** dev) {
   *dev = static_cast<T*>(p);
   return 0;
 }
-struct Dims3d { int G, T3; long long m[4]; };
-Dims3d dims3d(long long B, int T, int fs) {
+// temporal positions of one clip of T frames: G groups of fs frames after layer 1 (and 2), T3 after the stride-2 layer 3
+struct Dims3d { int G, T3; };
+Dims3d dims3d(int T, int fs) {
   Dims3d d;
   d.G = (T + fs - 1) / fs;
   d.T3 = (d.G - 1) / 2 + 1;
-  d.m[0] = B * d.G * 1024; d.m[1] = B * d.G * 256; d.m[2] = B * d.T3 * 64; d.m[3] = B * d.T3 * 16;
   return d;
+}
+// Workspace of one packed pass whose clips sum to sG groups and sT3 layer-3 positions:
+// [tables][im2col matrix A (layers 2-4, reused)][act 0][act 1][act 2][act 3]. Tables, in int32 units: layer-1 groups (int2 x sG),
+// then 16-byte aligned the im2col slots of layers 2, 3, 4 (int4 x sG, sT3, sT3) and the head's clips (int2 x C).
+struct Ws3d {
+  long long m[4];             // packed rows of the four conv layers
+  size_t t_slots[3], t_head;  // table offsets (int32 units)
+  size_t tables, a, act[4], total;   // byte offsets / sizes
+};
+Ws3d ws3d(const vfp3d_weights* w, long long sG, long long sT3, long long C) {
+  Ws3d L;
+  L.m[0] = sG * 1024; L.m[1] = sG * 256; L.m[2] = sT3 * 64; L.m[3] = sT3 * 16;
+  L.t_slots[0] = ((size_t)sG * 2 + 3) / 4 * 4;
+  L.t_slots[1] = L.t_slots[0] + (size_t)sG * 4;
+  L.t_slots[2] = L.t_slots[1] + (size_t)sT3 * 4;
+  L.t_head = L.t_slots[2] + (size_t)sT3 * 4;
+  L.tables = align_up((L.t_head + (size_t)C * 2) * 4, 1024);
+  size_t a_bytes = 0;
+  for (int l = 1; l < 4; ++l) a_bytes = std::max(a_bytes, align_up((size_t)L.m[l] * w->kp[l] * 2, 1024));   // layer 1 needs no im2col matrix
+  L.a = L.tables;
+  size_t off = L.a + a_bytes;
+  for (int l = 0; l < 4; ++l) { L.act[l] = off; off += align_up((size_t)L.m[l] * k3dNp[l] * 2, 1024); }
+  L.total = off + 1024;
+  return L;
+}
+
+// One packed pass: clips [c0, c1) of the input, frames cu[c0] .. cu[c1].
+int forward3d_pass(const vfp3d_weights* w, const uint8_t* frames_base, int frame_dtype, size_t frame_bytes, const int32_t* cu,
+                   int c0, int c1, float* emb_out, uint8_t* ws, cudaStream_t st) {
+  const int C = c1 - c0, fs = w->fs;
+  long long sG = 0, sT3 = 0;
+  for (int i = c0; i < c1; ++i) { const Dims3d d = dims3d(cu[i + 1] - cu[i], fs); sG += d.G; sT3 += d.T3; }
+  const Ws3d L = ws3d(w, sG, sT3, C);
+  // the per-pass tables (pageable host memory: the copy is staged before cudaMemcpyAsync returns, so the vector may go)
+  std::vector<int32_t> tab(L.t_head + (size_t)C * 2, 0);
+  int32_t* groups = tab.data();
+  int32_t* slots[3] = {tab.data() + L.t_slots[0], tab.data() + L.t_slots[1], tab.data() + L.t_slots[2]};
+  int32_t* head = tab.data() + L.t_head;
+  long long gb = 0, tb = 0;   // first group / layer-3 position of the clip in the pass
+  for (int i = c0; i < c1; ++i) {
+    const int f = cu[i] - cu[c0], T = cu[i + 1] - cu[i];
+    const Dims3d d = dims3d(T, fs);
+    for (int g = 0; g < d.G; ++g) { groups[(gb + g) * 2] = f + g * fs; groups[(gb + g) * 2 + 1] = T - g * fs; }
+    auto slot = [](int32_t* s, long long in_base, int Ti, int t0) { s[0] = (int32_t)in_base; s[1] = Ti; s[2] = t0; s[3] = 0; };
+    for (int to = 0; to < d.G; ++to) slot(slots[0] + (gb + to) * 4, gb, d.G, to - 1);         // layer 2: G -> G, stride 1
+    for (int to = 0; to < d.T3; ++to) slot(slots[1] + (tb + to) * 4, gb, d.G, 2 * to - 1);    // layer 3: G -> T3, stride 2
+    for (int to = 0; to < d.T3; ++to) slot(slots[2] + (tb + to) * 4, tb, d.T3, to - 1);       // layer 4: T3 -> T3, stride 1
+    head[(i - c0) * 2] = (int32_t)tb; head[(i - c0) * 2 + 1] = d.T3;
+    gb += d.G; tb += d.T3;
+  }
+  VFP_CUDA(cudaMemcpyAsync(ws, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice, st));
+  const int32_t* dtab = reinterpret_cast<const int32_t*>(ws);
+  __nv_bfloat16* A = reinterpret_cast<__nv_bfloat16*>(ws + L.a);
+  __nv_bfloat16* act[4];
+  for (int l = 0; l < 4; ++l) act[l] = reinterpret_cast<__nv_bfloat16*>(ws + L.act[l]);
+  const uint8_t* fr = frames_base + (size_t)cu[c0] * frame_bytes;
+  for (int l = 0; l < 4; ++l) {
+    if (l == 0) {   // layer 1 straight from the frames on the register-fragment tensor path, no im2col matrix
+      const size_t smem = (((size_t)fs * 5 * 204 * 2 + 4 + 15) & ~size_t(15)) + 4 * 16 * 32 * 4;
+      VFP_CUDA(ensure_dynamic_smem(reinterpret_cast<const void*>(conv3d_l1_kernel), 64 * 5 * 204 * 2 + 32 + 4 * 16 * 32 * 4));
+      conv3d_l1_kernel<<<(unsigned)(sG * 32), 128, smem, st>>>(fr, frame_dtype, reinterpret_cast<const int2*>(dtab), fs, w->l1_pack,
+                                                             w->b[0], act[0]);
+      continue;
+    }
+    const long long items = L.m[l] * (w->kp[l] / 8);
+    const unsigned grid = (unsigned)std::min<long long>((items + 255) / 256, (long long)device_sm_count() * 32);
+    const int Hi = 64 >> l;
+    im2col3d_ndhwc_kernel<<<grid, 256, 0, st>>>(act[l - 1], reinterpret_cast<const int4*>(dtab + L.t_slots[l - 1]), l == 1 ? sG : sT3,
+                                                Hi, Hi, k3dCinPad[l], Hi / 2, Hi / 2, w->kp[l], A);
+    CUtensorMap ta;
+    if (make_tmap_rows_bf16(&ta, A, (uint64_t)L.m[l], (uint64_t)w->kp[l], (uint64_t)w->kp[l], 128, 64)) return fail("vfp3d_forward: tensor map encode failed (A)");
+    EpiBiasActTma<true>::Params ep{};
+    if (make_tmap_out(&ep.tmap_out, act[l], (uint64_t)L.m[l], (uint64_t)k3dNp[l], true)) return fail("vfp3d_forward: tensor map encode failed (out)");
+    ep.bias = w->b[l]; ep.N = k3dNp[l]; ep.act = 1;
+    GemmShape s = plain_shape(L.m[l], k3dNp[l], w->kp[l], k3dNp[l], 64, 32);
+    if (l <= 1) VFP_CUDA((launch_gemm<32, 64, 4, EpiBiasActTma<true>>(ta, w->tm[l], s, ep, st)));
+    else if (l == 2) VFP_CUDA((launch_gemm<64, 64, 4, EpiBiasActTma<true>>(ta, w->tm[l], s, ep, st)));
+    else VFP_CUDA((launch_gemm<128, 64, 4, EpiBiasActTma<true>>(ta, w->tm[l], s, ep, st)));
+  }
+  Head3dParams hp{};
+  hp.act = act[3]; hp.clips = reinterpret_cast<const int2*>(dtab + L.t_head);
+  hp.tc_w = w->tc_w; hp.tc_b = w->tc_b; hp.ta_w = w->ta_w; hp.ta_b = w->ta_b;
+  hp.p0_w = w->p0_w; hp.p0_b = w->p0_b; hp.p3_w = w->p3_w; hp.p3_b = w->p3_b; hp.D = w->embedding_dim;
+  hp.out = emb_out + (size_t)c0 * w->embedding_dim;
+  head3d_kernel<<<(unsigned)C, 128, 0, st>>>(hp);
+  VFP_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// Checks a packed input and runs it in passes cut on clip boundaries, each as large as the workspace holds.
+int forward3d_packed(const char* who, const vfp3d_weights* w, const void* frames, int frame_dtype, const int32_t* cu, int n_clips,
+                     float* emb_out, void* workspace, size_t workspace_bytes, void* stream) {
+  const std::string name(who);
+  if (!w || !frames || !cu || !emb_out || !workspace) return fail(name + ": null argument");
+  if (n_clips <= 0) return fail(name + ": n_clips must be positive");
+  if (frame_dtype == VFP_FRAME_U8_HWC) return fail(name + ": decoder-layout (HWC) frames are not supported by the 3-D model; pass planar (T, 3, 64, 64) frames");
+  if (frame_dtype != VFP_FRAME_U8 && frame_dtype != VFP_FRAME_BF16 && frame_dtype != VFP_FRAME_F32) return fail(name + ": planar u8 / bf16 / fp32 frames only");
+  if (cu[0] != 0) return fail(name + ": cu_seqlens[0] must be 0");
+  for (int i = 0; i < n_clips; ++i) {
+    const int T = cu[i + 1] - cu[i];
+    if (cu[i + 1] < cu[i]) return fail(name + ": cu_seqlens is not monotone (decreases at clip " + std::to_string(i) + ")");
+    if (T == 0) return fail(name + ": clip " + std::to_string(i) + " has length 0");
+    const Dims3d d = dims3d(T, w->fs);
+    if (d.T3 > kHead3dMaxT)
+      return fail(name + ": clip " + std::to_string(i) + " too long: " + std::to_string(T) + " frames give " + std::to_string(d.T3) +
+                  " temporal positions after the strides (at most 32, i.e. " + std::to_string(64 * w->fs) + " frames)");
+    const size_t need = ws3d(w, d.G, d.T3, 1).total;
+    if (need > workspace_bytes)
+      return fail(name + ": workspace of " + std::to_string(workspace_bytes) + " bytes is too small for clip " + std::to_string(i) + " (" +
+                  std::to_string(T) + " frames need " + std::to_string(need) + ")");
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t frame_bytes = (size_t)12288 * (frame_dtype == VFP_FRAME_BF16 ? 2 : frame_dtype == VFP_FRAME_F32 ? 4 : 1);
+  for (int c0 = 0; c0 < n_clips;) {
+    int c1 = c0;   // every clip fits on its own (checked above): add clips while the pass still fits
+    long long sG = 0, sT3 = 0;
+    while (c1 < n_clips) {
+      const Dims3d d = dims3d(cu[c1 + 1] - cu[c1], w->fs);
+      if (c1 > c0 && ws3d(w, sG + d.G, sT3 + d.T3, c1 - c0 + 1).total > workspace_bytes) break;
+      sG += d.G; sT3 += d.T3; ++c1;
+    }
+    if (int rc = forward3d_pass(w, static_cast<const uint8_t*>(frames), frame_dtype, frame_bytes, cu, c0, c1, emb_out,
+                                static_cast<uint8_t*>(workspace), st))
+      return rc;
+    c0 = c1;
+  }
+  return 0;
 }
 }  // namespace
 
@@ -1432,69 +1559,33 @@ int vfp3d_weights_create(const vfp_tensor_desc* tensors, int n_tensors, int fram
 
 size_t vfp3d_forward_workspace_bytes(const vfp3d_weights* w, int64_t clips_per_pass, int n_frames) {
   if (!w || clips_per_pass <= 0 || n_frames <= 0) return 0;
-  const Dims3d d = dims3d(clips_per_pass, n_frames, w->fs);
-  size_t a = 0, act = 0;
-  for (int l = 0; l < 4; ++l) {
-    if (l > 0) a = std::max(a, align_up((size_t)d.m[l] * w->kp[l] * 2, 1024));   // layer 1 needs no im2col matrix
-    act += align_up((size_t)d.m[l] * k3dNp[l] * 2, 1024);
-  }
-  return a + act + 1024;
+  const Dims3d d = dims3d(n_frames, w->fs);
+  return ws3d(w, clips_per_pass * d.G, clips_per_pass * d.T3, clips_per_pass).total;
 }
 
+size_t vfp3d_forward_packed_workspace_bytes(const vfp3d_weights* w, int64_t frames_per_pass, int64_t clips_per_pass) {
+  if (!w || frames_per_pass <= 0 || clips_per_pass <= 0) return 0;
+  const int64_t C = std::min(clips_per_pass, frames_per_pass);                  // a clip has at least one frame
+  const int64_t G = std::min(frames_per_pass, frames_per_pass / w->fs + C);     // sum ceil(T/fs) <= F/fs + C, and <= F
+  const int64_t T3 = std::min(G, (G + C) / 2);                                  // sum ceil(G/2) <= (sum G + C) / 2
+  return ws3d(w, G, T3, C).total;
+}
+
+// The equal-length batch is the packed path with uniform clip lengths: one kernel set, one indexing scheme.
 int vfp3d_forward(const vfp3d_weights* w, const void* frames, int frame_dtype, int64_t n_clips, int n_frames, float* emb_out,
                   void* workspace, size_t workspace_bytes, void* stream) {
   if (!w || !frames || !emb_out || !workspace) return fail("vfp3d_forward: null argument");
   if (n_clips <= 0 || n_frames <= 0) return fail("vfp3d_forward: empty input");
-  if (frame_dtype != VFP_FRAME_U8 && frame_dtype != VFP_FRAME_BF16 && frame_dtype != VFP_FRAME_F32) return fail("vfp3d_forward: planar u8 / bf16 / fp32 frames only");
-  const Dims3d one = dims3d(1, n_frames, w->fs);
-  if (one.T3 > kHead3dMaxT) return fail("vfp3d_forward: clip too long (more than 32 temporal positions after the strides)");
-  // largest pass that fits the workspace
-  int64_t per = n_clips;
-  while (per > 1 && vfp3d_forward_workspace_bytes(w, per, n_frames) > workspace_bytes) per = (per + 1) / 2;
-  if (vfp3d_forward_workspace_bytes(w, per, n_frames) > workspace_bytes) return fail("vfp3d_forward: workspace too small for one clip; see vfp3d_forward_workspace_bytes");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t frame_bytes = (size_t)12288 * (frame_dtype == VFP_FRAME_BF16 ? 2 : frame_dtype == VFP_FRAME_F32 ? 4 : 1);
-  for (int64_t c0 = 0; c0 < n_clips; c0 += per) {
-    const int64_t B = std::min<int64_t>(per, n_clips - c0);
-    const Dims3d d = dims3d(B, n_frames, w->fs);
-    uint8_t* ws = static_cast<uint8_t*>(workspace);
-    size_t a_bytes = 0;
-    for (int l = 1; l < 4; ++l) a_bytes = std::max(a_bytes, align_up((size_t)d.m[l] * w->kp[l] * 2, 1024));
-    __nv_bfloat16* A = reinterpret_cast<__nv_bfloat16*>(ws);
-    __nv_bfloat16* act[4];
-    size_t off = a_bytes;
-    for (int l = 0; l < 4; ++l) { act[l] = reinterpret_cast<__nv_bfloat16*>(ws + off); off += align_up((size_t)d.m[l] * k3dNp[l] * 2, 1024); }
-    const uint8_t* fr = static_cast<const uint8_t*>(frames) + (size_t)c0 * n_frames * frame_bytes;
-    for (int l = 0; l < 4; ++l) {
-      const long long items = d.m[l] * (w->kp[l] / 8);
-      const unsigned grid = (unsigned)std::min<long long>((items + 255) / 256, (long long)device_sm_count() * 32);
-      if (l == 0) {   // layer 1 straight from the frames on the register-fragment tensor path, no im2col matrix
-        const size_t smem = (((size_t)w->fs * 5 * 204 * 2 + 4 + 15) & ~size_t(15)) + 4 * 16 * 32 * 4;
-        VFP_CUDA(ensure_dynamic_smem(reinterpret_cast<const void*>(conv3d_l1_kernel), 64 * 5 * 204 * 2 + 32 + 4 * 16 * 32 * 4));
-        conv3d_l1_kernel<<<(unsigned)(B * d.G * 32), 128, smem, st>>>(fr, frame_dtype, n_frames, w->fs, d.G, w->l1_pack, w->b[0], act[0]);
-        continue;
-      } else {
-        const int Ti = l == 3 ? d.T3 : d.G, Hi = 64 >> l, st_t = l == 2 ? 2 : 1, To = l == 1 ? d.G : d.T3;
-        im2col3d_ndhwc_kernel<<<grid, 256, 0, st>>>(act[l - 1], (int)B, Ti, Hi, Hi, k3dCinPad[l], st_t, To, Hi / 2, Hi / 2, w->kp[l], A);
-      }
-      CUtensorMap ta;
-      if (make_tmap_rows_bf16(&ta, A, (uint64_t)d.m[l], (uint64_t)w->kp[l], (uint64_t)w->kp[l], 128, 64)) return fail("vfp3d_forward: tensor map encode failed (A)");
-      EpiBiasActTma<true>::Params ep{};
-      if (make_tmap_out(&ep.tmap_out, act[l], (uint64_t)d.m[l], (uint64_t)k3dNp[l], true)) return fail("vfp3d_forward: tensor map encode failed (out)");
-      ep.bias = w->b[l]; ep.N = k3dNp[l]; ep.act = 1;
-      GemmShape s = plain_shape(d.m[l], k3dNp[l], w->kp[l], k3dNp[l], 64, 32);
-      if (l <= 1) VFP_CUDA((launch_gemm<32, 64, 4, EpiBiasActTma<true>>(ta, w->tm[l], s, ep, st)));
-      else if (l == 2) VFP_CUDA((launch_gemm<64, 64, 4, EpiBiasActTma<true>>(ta, w->tm[l], s, ep, st)));
-      else VFP_CUDA((launch_gemm<128, 64, 4, EpiBiasActTma<true>>(ta, w->tm[l], s, ep, st)));
-    }
-    Head3dParams hp{};
-    hp.act = act[3]; hp.T3 = d.T3; hp.tc_w = w->tc_w; hp.tc_b = w->tc_b; hp.ta_w = w->ta_w; hp.ta_b = w->ta_b;
-    hp.p0_w = w->p0_w; hp.p0_b = w->p0_b; hp.p3_w = w->p3_w; hp.p3_b = w->p3_b; hp.D = w->embedding_dim;
-    hp.out = emb_out + (size_t)c0 * w->embedding_dim;
-    head3d_kernel<<<(unsigned)B, 128, 0, st>>>(hp);
-    VFP_CUDA(cudaGetLastError());
-  }
-  return 0;
+  if (n_clips > INT32_MAX || n_clips * (int64_t)n_frames > INT32_MAX) return fail("vfp3d_forward: more than 2^31 - 1 frames in one call");
+  std::vector<int32_t> cu((size_t)n_clips + 1);
+  for (int64_t i = 0; i <= n_clips; ++i) cu[i] = (int32_t)(i * n_frames);
+  return forward3d_packed("vfp3d_forward", w, frames, frame_dtype, cu.data(), (int)n_clips, emb_out, workspace, workspace_bytes, stream);
+}
+
+int vfp3d_forward_packed(const vfp3d_weights* w, const void* frames, int frame_dtype, const int32_t* cu_seqlens_host, int n_clips,
+                         float* emb_out, void* workspace, size_t workspace_bytes, void* stream) {
+  return forward3d_packed("vfp3d_forward_packed", w, frames, frame_dtype, cu_seqlens_host, n_clips, emb_out, workspace, workspace_bytes,
+                          stream);
 }
 
 }  // extern "C"

@@ -326,6 +326,35 @@ class VideoFingerprintScanner:
         final = np.mean(emb, axis=0)
         return final / np.linalg.norm(final)
 
+    def extract_fingerprints_3d_from_frames(self, videos: Sequence[torch.Tensor]) -> List[Optional[np.ndarray]]:
+        """Batched form of the reference's per-video 3-D scan loop (fingerprint.py:272-320, driven per video at :377-434):
+        preprocessed (T_v, 3, 64, 64) videos of one dtype -> one embedding per video, with the rule of
+        `extract_fingerprint_3d_from_frames` (< 10 frames -> None; at most clip_length frames -> one clip of the video's own
+        length; longer -> the window_starts_3d windows, averaged and re-normalised). The clips of ALL videos go through one
+        packed forward, so a corpus of short videos of many different lengths costs one launch sequence, not one per video."""
+        clip_length = self.config.get("clip_length", 128)
+        pieces: List[torch.Tensor] = []
+        spans: List[Tuple[int, int, int]] = []   # (video, first row, rows) in the packed result
+        for v, frames in enumerate(videos):
+            total = int(frames.shape[0])
+            if total < 10:
+                continue
+            starts = self.window_starts_3d(total)
+            span = total if total <= clip_length else clip_length
+            spans.append((v, len(pieces), len(starts)))
+            pieces += [frames[s : s + span] for s in starts]
+        result: List[Optional[np.ndarray]] = [None] * len(videos)
+        if not pieces:
+            return result
+        emb = self.model.fingerprint_clips(pieces).cpu().numpy()
+        for v, row, k in spans:
+            if int(videos[v].shape[0]) <= clip_length:
+                result[v] = emb[row]
+            else:
+                final = np.mean(np.ascontiguousarray(emb[row : row + k]), axis=0)
+                result[v] = final / np.linalg.norm(final)
+        return result
+
     def extract_fingerprint_from_frames(self, clip: torch.Tensor) -> Optional[np.ndarray]:
         """clip: (T,3,64,64) preprocessed frames (what _preprocess_frames returns). <10 frames -> None."""
         out = self.extract_fingerprints_from_frames([clip])

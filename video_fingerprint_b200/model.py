@@ -311,10 +311,20 @@ class Conv3DBlock(_ParamsOnly):
         self.relu = nn.ReLU(inplace=True)
 
 
+def _frame_code(frames: torch.Tensor) -> Tuple[int, torch.Tensor]:
+    """Native frame type of planar (.., 3, 64, 64) frames: uint8 (0..255, scaled on the device), bf16, anything else as fp32."""
+    if frames.dtype == torch.uint8:
+        return _native.FRAME_U8, frames
+    if frames.dtype == torch.bfloat16:
+        return _native.FRAME_BF16, frames
+    return _native.FRAME_F32, frames.float()
+
+
 class VideoFingerprint3D(nn.Module):
     """The reference's 3-D CNN fingerprint model (model.py:406-512), inference only: same constructor arguments, same
     state_dict keys / shapes / default initialisation, same forward contract ((B,T,3,64,64) or (B,3,T,64,64) in [0,1] ->
-    unit-norm (B, embedding_dim)); the compute is `vfp3d_forward` in libvfp_b200.so (im2col + tcgen05 GEMMs + a fused tail)."""
+    unit-norm (B, embedding_dim)); the compute is `vfp3d_forward` in libvfp_b200.so (im2col + tcgen05 GEMMs + a fused tail).
+    `fingerprint_packed` / `fingerprint_clips` take clips of different lengths in one call (`vfp3d_forward_packed`)."""
 
     def __init__(self, embedding_dim=256, frame_stride=32, dropout=0.2):
         super().__init__()
@@ -401,27 +411,76 @@ class VideoFingerprint3D(nn.Module):
             raise ValueError("the sm_100a kernels are specialised for 3 x 64 x 64 frames")
         if not video.is_cuda:
             video = video.cuda()
-        if video.dtype == torch.uint8:
-            code = _native.FRAME_U8
-        elif video.dtype == torch.bfloat16:
-            code = _native.FRAME_BF16
-        else:
-            code, video = _native.FRAME_F32, video.float()
+        code, video = _frame_code(video)
         frames = video.contiguous()
         dev = frames.device
         lib = _native.load()
         with torch.cuda.device(dev):
             weights = self._ensure_native()
             per = max(1, min(B, self.clips_per_pass))
-            nbytes = lib.vfp3d_forward_workspace_bytes(C.c_void_p(weights), per, T)
-            if self._workspace is None or self._workspace.numel() < nbytes or self._workspace.device != dev:
-                self._workspace = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            ws = self._get_workspace(lib.vfp3d_forward_workspace_bytes(C.c_void_p(weights), per, T), dev)
             emb = torch.empty((B, self.embedding_dim), dtype=torch.float32, device=dev)
             rc = lib.vfp3d_forward(C.c_void_p(weights), C.c_void_p(frames.data_ptr()), code, B, T, C.c_void_p(emb.data_ptr()),
-                                   C.c_void_p(self._workspace.data_ptr()), self._workspace.numel(),
-                                   C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+                                   C.c_void_p(ws.data_ptr()), ws.numel(), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
             _native.check(rc, "vfp3d_forward")
         return emb
+
+    def _get_workspace(self, nbytes: int, dev) -> torch.Tensor:
+        """One cached device workspace, grown on demand and shared by `forward` and `fingerprint_packed`."""
+        if self._workspace is None or self._workspace.numel() < nbytes or self._workspace.device != dev:
+            self._workspace = None
+            self._workspace = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        return self._workspace
+
+    # ------------------------------------------------------------------ packed (variable-length) entry
+    @torch.no_grad()
+    def fingerprint_packed(self, frames: torch.Tensor, lengths: Sequence[int]) -> torch.Tensor:
+        """frames: (sum T, 3, 64, 64) uint8 / bf16 / fp32, clips back to back (host frames are uploaded once); lengths: frames
+        per clip, each 1 .. 64 * frame_stride. Returns (n, embedding_dim) fp32 on the device; row i has exactly the bits
+        `forward` gives for clip i alone. Passes hold about `clips_per_pass` clips."""
+        _native.require_cuda()
+        if self.training:
+            raise RuntimeError("inference only: call .eval() first")
+        lengths = [int(t) for t in lengths]
+        n, total = len(lengths), sum(lengths)
+        if frames.dim() != 4 or tuple(frames.shape[1:]) != (3, 64, 64) or frames.shape[0] != total:
+            raise ValueError(f"frames must be (sum(lengths)={total}, 3, 64, 64), got {tuple(frames.shape)}")
+        if not frames.is_cuda:
+            frames = frames.cuda()
+        code, frames = _frame_code(frames)
+        frames = frames.contiguous()
+        dev = frames.device
+        lib = _native.load()
+        with torch.cuda.device(dev):
+            weights = self._ensure_native()
+            cu = (C.c_int32 * (n + 1))()
+            acc = 0
+            for i, t in enumerate(lengths):
+                cu[i] = acc
+                acc += t
+            cu[n] = acc
+            # workspace for passes of clips_per_pass clips of the batch's mean length (at least the longest clip)
+            per = max(1, min(n, self.clips_per_pass))
+            pass_frames = total if per == n else max(max(lengths), -(-total * per // n))
+            ws = self._get_workspace(lib.vfp3d_forward_packed_workspace_bytes(C.c_void_p(weights), max(1, pass_frames), per), dev)
+            emb = torch.empty((n, self.embedding_dim), dtype=torch.float32, device=dev)
+            rc = lib.vfp3d_forward_packed(C.c_void_p(weights), C.c_void_p(frames.data_ptr()), code, C.cast(cu, C.c_void_p), n,
+                                          C.c_void_p(emb.data_ptr()), C.c_void_p(ws.data_ptr()), ws.numel(),
+                                          C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+            _native.check(rc, "vfp3d_forward_packed")
+        return emb
+
+    def fingerprint_clips(self, clips: Sequence[torch.Tensor]) -> torch.Tensor:
+        """List of (T_i, 3, 64, 64) clips of one dtype -> (n, D) embeddings, one packed launch sequence (no padding, no masks).
+        Clips that are all on one device (or all on the host, then uploaded once) are concatenated there."""
+        if len({c.dtype for c in clips}) > 1:
+            raise ValueError("clips must share one dtype (uint8 frames are scaled by 1/255, float frames are not)")
+        lengths = [int(c.shape[0]) for c in clips]
+        devices = {c.device for c in clips}
+        if len(devices) > 1:
+            dev = next(d for d in devices if d.type == "cuda")
+            clips = [c.to(dev) for c in clips]
+        return self.fingerprint_packed(torch.cat(list(clips), dim=0), lengths)
 
     def compute_loss(self, *a, **k):
         raise NotImplementedError("training (model.py:514-582) is outside the B200 inference hot path")
