@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define VFP_ABI_VERSION 3
+#define VFP_ABI_VERSION 4
 
 /* frame element types accepted by vfp_forward (planar (T,3,64,64) frames as produced by
  * _preprocess_frames, fingerprint.py:186-214; U8 values are scaled by 1/255 on the device) */
@@ -130,7 +130,9 @@ int vfp3d_forward(const vfp3d_weights* w, const void* frames, int frame_dtype, i
  * (n_clips, D) fp32 to `emb_out`. Every clip is treated exactly like a B=1 vfp3d_forward on that clip alone, with the same
  * bits: its zero padding up to a multiple of frame_stride and its temporal padding stop at its own ends, whatever surrounds
  * it. A clip may have 1 .. 64 * frame_stride frames (at most 32 temporal positions after the strides); a clip of length 0,
- * a longer clip, decreasing prefix sums, or a workspace too small for a clip are errors naming the clip.
+ * a longer clip, decreasing prefix sums, or a workspace too small for a clip are errors naming the clip. `frames` must be
+ * 16-byte aligned (the frames are read in 8- and 16-byte vectors); so must vfp3d_forward's. Every torch allocation and
+ * every whole-frame view of one is.
  * The call splits the input into passes on clip boundaries that fit `workspace_bytes`; results do not depend on the split.
  * vfp3d_forward_packed_workspace_bytes bounds one pass of up to `frames_per_pass` frames in up to `clips_per_pass` clips
  * (from sum ceil(T/fs) <= F/fs + C and sum T3 <= (sum G + C)/2); the minimum useful value is that of the longest clip
@@ -139,11 +141,23 @@ size_t vfp3d_forward_packed_workspace_bytes(const vfp3d_weights* w, int64_t fram
 int vfp3d_forward_packed(const vfp3d_weights* w, const void* frames, int frame_dtype, const int32_t* cu_seqlens_host,
                          int n_clips, float* emb_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Clips that sit anywhere in device memory, with the conventions of vfp3d_forward_packed: `clip_frames_host` is a HOST
+ * array of n_clips device pointers, each at its clip's first frame, and clip i is `lengths_host[i]` contiguous frames from
+ * there, planar (T, 3, 64, 64) u8 / bf16 / fp32 or decoder-layout (T, 64, 64, 3) u8 (VFP_FRAME_U8_HWC, the output of
+ * vfp_preprocess_frames; it gives the same bits as the same frames permuted to planar u8). Clips may be separate
+ * allocations, overlapping windows of one buffer, or the same frames listed twice; no frame is copied. Row i of `emb_out`
+ * has the bits of a B=1 vfp3d_forward on clip i alone. Size the workspace with vfp3d_forward_packed_workspace_bytes
+ * (frames_per_pass = the sum of the lengths of a pass). A null or not 16-byte aligned pointer, a length below 1 or above
+ * 64 * frame_stride, a workspace too small for a clip and an unknown frame_dtype are errors naming the clip; beyond that
+ * the pointers are not validated (each must address lengths_host[i] readable frames on the current device). */
+int vfp3d_forward_clips(const vfp3d_weights* w, const void* const* clip_frames_host, const int32_t* lengths_host,
+                        int n_clips, int frame_dtype, float* emb_out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Frame preprocessing of the scanner (/root/reference/fingerprint.py:186-214 _preprocess_frames): cv2.resize(frame,
  * INTER_AREA) so that the short side becomes 64 (new size truncated with int() like the reference), then the centre
  * 64 x 64 crop. `frames_hwc`: device uint8 (n_frames, height, width, 3), all frames of one size; `out_hwc64`: device
- * uint8 (n_frames, 64, 64, 3), which vfp_forward accepts as VFP_FRAME_U8_HWC (the /255 and the HWC->CHW permute of
- * fingerprint.py:210-212 happen inside the stem kernel). Bit-exact with OpenCV 4.x INTER_AREA: down-scaling (general,
+ * uint8 (n_frames, 64, 64, 3), which vfp_forward and vfp3d_forward_clips accept as VFP_FRAME_U8_HWC (the /255 and the
+ * HWC->CHW permute of fingerprint.py:210-212 happen inside the first layer's loader). Bit-exact with OpenCV 4.x INTER_AREA: down-scaling (general,
  * integer-factor and 2 x 2 code paths) and, for frames with a side below 64 pixels, the up-scaling branch (8-bit fixed-point
  * bilinear kernels with the area coefficient rule). */
 size_t vfp_preprocess_workspace_bytes(int height, int width);

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, _LIB_NAME)
 LIB_PATH = os.environ.get("VFP_B200_LIB", LIB_PATH)  # development aid: load an experimental build
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 FRAME_U8, FRAME_BF16, FRAME_F32, FRAME_U8_HWC = 0, 1, 2, 3
 
 # every symbol include/vfp_b200.h declares (tests check the library exports exactly these)
@@ -36,6 +36,7 @@ EXPORTED_SYMBOLS = (
     "vfp3d_forward",
     "vfp3d_forward_packed_workspace_bytes",
     "vfp3d_forward_packed",
+    "vfp3d_forward_clips",
     "vfp_preprocess_workspace_bytes",
     "vfp_preprocess_frames",
     "vfp_pair_scores",
@@ -111,6 +112,8 @@ def load() -> C.CDLL:
     lib.vfp3d_forward_packed_workspace_bytes.argtypes = [vp, i64, i64]
     lib.vfp3d_forward_packed.restype = i32
     lib.vfp3d_forward_packed.argtypes = [vp, vp, i32, vp, i32, vp, vp, sz, vp]
+    lib.vfp3d_forward_clips.restype = i32
+    lib.vfp3d_forward_clips.argtypes = [vp, vp, vp, i32, i32, vp, vp, sz, vp]
     lib.vfp_preprocess_workspace_bytes.restype = sz
     lib.vfp_preprocess_workspace_bytes.argtypes = [i32, i32]
     lib.vfp_preprocess_frames.restype = i32

@@ -21,21 +21,29 @@ namespace vfp {
 // host builds per pass; the arithmetic is the same as for the clip alone, so packed results equal B = 1 results bit for bit.
 // An equal-length batch is the special case of uniform clip lengths.
 
-// Layer 1: Conv3d(3 -> 16, kernel (fs, 5, 5), stride (fs, 2, 2), padding (0, 2, 2)) + folded BatchNorm3d + ReLU over planar
-// frames (sum T, 3, 64, 64) of any accepted dtype; each clip's T is zero-padded to a multiple of fs like model.py:468-471.
+// Layer 1: Conv3d(3 -> 16, kernel (fs, 5, 5), stride (fs, 2, 2), padding (0, 2, 2)) + folded BatchNorm3d + ReLU over frames
+// of any accepted type: planar (T, 3, 64, 64) u8 / bf16 / fp32 or decoder-layout (T, 64, 64, 3) u8; each clip's T is
+// zero-padded to a multiple of fs like model.py:468-471.
 // C_in = 3 makes this the same problem as the attention model's conv1 (6-byte pixels are not TMA / UMMA addressable), with
 // the same answer: the register-fragment tensor path. Per (kt, kh) the 5 x 3 (kw, c) taps of an output position are 15
 // CONSECUTIVE bf16 of a pixel-interleaved (HWC) copy of the input row (+ 1 don't-care with zero weight), so one A register of
 // mma.sync m16n8k16 is one aligned 32-bit shared load: K = 16 * 5 * fs, k = (kt*5 + kh)*16 + kw*3 + c.
-// One CTA per (global group, oh) = 32 output positions x 16 channels. groups[global group] = {first frame of the group, frames
-// of its clip from there on}: frames at or past the clip's own end read as zero, never as the next clip's first frames. The
-// 5 input rows x fs frames a CTA needs are staged in shared memory (68 pixels: zero halo of 2 on both sides; rows outside the
-// image and frames past the clip end are zero), the four warps split the 5*fs K runs, partial sums meet in shared memory,
-// bias + ReLU, bf16 channels-last output [position][32] (channels 16..31 zero: the 32-column box of the next layer's GEMM). An earlier version materialised the im2col matrix (2.6 GB written
-// and read back per 256 clips): 1.05 ms per 256 clips against 0.1 ms here.
+// One CTA per (global group, oh) = 32 output positions x 16 channels. groups[global group] = {device address of the group's
+// first frame, frames of its clip from there on}: frames at or past the clip's own end read as zero, never as whatever lies
+// next in memory, so clips may sit anywhere (separate allocations, overlapping windows of one buffer, one view listed twice).
+// The 5 input rows x fs frames a CTA needs are staged in shared memory (68 pixels: zero halo of 2 on both sides; rows outside
+// the image and frames past the clip end are zero), the four warps split the 5*fs K runs, partial sums meet in shared memory,
+// bias + ReLU, bf16 channels-last output [position][32] (channels 16..31 zero: the 32-column box of the next layer's GEMM).
+// An earlier version materialised the im2col matrix (2.6 GB written and read back per 256 clips): 1.05 ms per 256 clips
+// against 0.1 ms here.
 // wpack: [5*fs runs][2 n-tiles][32 lanes] x uint2 = the B fragments of the folded weights; bias [16].
-__global__ void __launch_bounds__(128) conv3d_l1_kernel(const void* __restrict__ frames, int frame_dtype, const int2* __restrict__ groups,
-                                                        int fs, const uint2* __restrict__ wpack, const float* __restrict__ bias,
+struct __align__(16) L1Group {
+  const void* frames;   // first frame of the group; 16-byte aligned (8/16-byte vector loads)
+  int left;             // frames of the clip from this one on (>= 1)
+  int pad;
+};
+__global__ void __launch_bounds__(128) conv3d_l1_kernel(int frame_dtype, const L1Group* __restrict__ groups, int fs,
+                                                        const uint2* __restrict__ wpack, const float* __restrict__ bias,
                                                         __nv_bfloat16* __restrict__ out) {
   extern __shared__ __align__(16) uint8_t smem3d[];
   __nv_bfloat16* tile = reinterpret_cast<__nv_bfloat16*>(smem3d);   // [fs*5 runs][68 pixels][3 channels] (+ 2 pad elements)
@@ -43,7 +51,8 @@ __global__ void __launch_bounds__(128) conv3d_l1_kernel(const void* __restrict__
   float* part = reinterpret_cast<float*>(smem3d + (((size_t)runs * 204 * 2 + 4 + 15) & ~size_t(15)));   // [4 warps][16][32 lanes]
   const int oh = blockIdx.x & 31;
   const unsigned gg = blockIdx.x >> 5;
-  const int2 grp = __ldg(groups + gg);   // {first frame, frames left in the clip}
+  const L1Group grp = groups[gg];
+  const uint8_t* fbase = static_cast<const uint8_t*>(grp.frames);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   // halo pixels (x = -2, -1, 64, 65) of every run
   for (int i = tid; i < runs * 12; i += 128) {
@@ -52,40 +61,60 @@ __global__ void __launch_bounds__(128) conv3d_l1_kernel(const void* __restrict__
     tile[(run * 68 + x) * 3 + c] = __float2bfloat16(0.0f);
   }
   if (tid < 2) tile[runs * 204 + tid] = __float2bfloat16(0.0f);   // the don't-care element after the very last run
-  // load: one item = 8 consecutive pixels of one (run, plane) row: a 16-byte (bf16) / 8-byte (u8) / 32-byte (fp32) load
-  for (int i = tid; i < runs * 24; i += 128) {
-    const int x0 = (i & 7) * 8, c = (i >> 3) % 3, run = i / 24;
-    const int kh = run % 5, kt = run / 5;
-    const int ih = 2 * oh + kh - 2;
-    float v[8];
+  if (frame_dtype == kFrameU8HWC) {
+    // decoder layout: an input row (run, ih) is 192 contiguous bytes already in the tile's pixel-interleaved order, so byte b
+    // goes to element run*204 + 6 + b. One item = 16 bytes: one 16-byte load, eight 4-byte bf16x2 stores (even element offset).
+    // Same value as the planar u8 path, (float)u8 * (1/255) rounded to bf16, so both layouts give the same bits.
+    for (int i = tid; i < runs * 12; i += 128) {
+      const int q = i % 12, run = i / 12;
+      const int kh = run % 5, kt = run / 5;
+      const int ih = 2 * oh + kh - 2;
+      uint4 d = make_uint4(0u, 0u, 0u, 0u);
+      if (kt < grp.left && ih >= 0 && ih < 64) d = *reinterpret_cast<const uint4*>(fbase + (size_t)kt * 12288 + ih * 192 + q * 16);
+      const uint32_t w[4] = {d.x, d.y, d.z, d.w};
+      __nv_bfloat162* dst = reinterpret_cast<__nv_bfloat162*>(tile + run * 204 + 6 + q * 16);
 #pragma unroll
-    for (int j = 0; j < 8; ++j) v[j] = 0.0f;
-    if (kt < grp.y && ih >= 0 && ih < 64) {
-      const size_t idx = (((size_t)(grp.x + kt) * 3 + c) * 64 + ih) * 64 + x0;
-      if (frame_dtype == kFrameBF16) {
-        const uint4 q = *reinterpret_cast<const uint4*>(static_cast<const __nv_bfloat16*>(frames) + idx);
-        const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          v[2 * j] = __uint_as_float(w[j] << 16);
-          v[2 * j + 1] = __uint_as_float(w[j] & 0xFFFF0000u);
-        }
-      } else if (frame_dtype == kFrameU8) {
-        const uint2 q = *reinterpret_cast<const uint2*>(static_cast<const uint8_t*>(frames) + idx);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          v[j] = (float)((q.x >> (8 * j)) & 0xFF) * (1.0f / 255.0f);
-          v[4 + j] = (float)((q.y >> (8 * j)) & 0xFF) * (1.0f / 255.0f);
-        }
-      } else {
-        const float4 a = *reinterpret_cast<const float4*>(static_cast<const float*>(frames) + idx);
-        const float4 d = *reinterpret_cast<const float4*>(static_cast<const float*>(frames) + idx + 4);
-        v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = d.x; v[5] = d.y; v[6] = d.z; v[7] = d.w;
+      for (int j = 0; j < 8; ++j) {
+        const uint32_t b = w[j >> 1] >> (16 * (j & 1));
+        dst[j] = __floats2bfloat162_rn((float)(b & 0xFF) * (1.0f / 255.0f), (float)((b >> 8) & 0xFF) * (1.0f / 255.0f));
       }
     }
-    __nv_bfloat16* dst = tile + (run * 68 + x0 + 2) * 3 + c;
+  } else {
+    // planar: one item = 8 consecutive pixels of one (run, plane) row: a 16-byte (bf16) / 8-byte (u8) / 32-byte (fp32) load
+    for (int i = tid; i < runs * 24; i += 128) {
+      const int x0 = (i & 7) * 8, c = (i >> 3) % 3, run = i / 24;
+      const int kh = run % 5, kt = run / 5;
+      const int ih = 2 * oh + kh - 2;
+      float v[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) dst[3 * j] = __float2bfloat16(v[j]);
+      for (int j = 0; j < 8; ++j) v[j] = 0.0f;
+      if (kt < grp.left && ih >= 0 && ih < 64) {
+        const size_t idx = (((size_t)kt * 3 + c) * 64 + ih) * 64 + x0;
+        if (frame_dtype == kFrameBF16) {
+          const uint4 q = *reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(fbase) + idx);
+          const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            v[2 * j] = __uint_as_float(w[j] << 16);
+            v[2 * j + 1] = __uint_as_float(w[j] & 0xFFFF0000u);
+          }
+        } else if (frame_dtype == kFrameU8) {
+          const uint2 q = *reinterpret_cast<const uint2*>(fbase + idx);
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            v[j] = (float)((q.x >> (8 * j)) & 0xFF) * (1.0f / 255.0f);
+            v[4 + j] = (float)((q.y >> (8 * j)) & 0xFF) * (1.0f / 255.0f);
+          }
+        } else {
+          const float4 a = *reinterpret_cast<const float4*>(reinterpret_cast<const float*>(fbase) + idx);
+          const float4 d = *reinterpret_cast<const float4*>(reinterpret_cast<const float*>(fbase) + idx + 4);
+          v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = d.x; v[5] = d.y; v[6] = d.z; v[7] = d.w;
+        }
+      }
+      __nv_bfloat16* dst = tile + (run * 68 + x0 + 2) * 3 + c;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) dst[3 * j] = __float2bfloat16(v[j]);
+    }
   }
   __syncthreads();
   // ---- this warp's share of the K runs: 2 m-tiles (positions 0-15, 16-31) x 2 n-tiles (channels 0-7, 8-15) ----

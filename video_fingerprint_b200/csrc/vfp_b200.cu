@@ -1351,8 +1351,8 @@ Dims3d dims3d(int T, int fs) {
   return d;
 }
 // Workspace of one packed pass whose clips sum to sG groups and sT3 layer-3 positions:
-// [tables][im2col matrix A (layers 2-4, reused)][act 0][act 1][act 2][act 3]. Tables, in int32 units: layer-1 groups (int2 x sG),
-// then 16-byte aligned the im2col slots of layers 2, 3, 4 (int4 x sG, sT3, sT3) and the head's clips (int2 x C).
+// [tables][im2col matrix A (layers 2-4, reused)][act 0][act 1][act 2][act 3]. Tables, in int32 units: layer-1 groups (L1Group,
+// 16 bytes, x sG), the im2col slots of layers 2, 3, 4 (int4 x sG, sT3, sT3) and the head's clips (int2 x C).
 struct Ws3d {
   long long m[4];             // packed rows of the four conv layers
   size_t t_slots[3], t_head;  // table offsets (int32 units)
@@ -1361,7 +1361,7 @@ struct Ws3d {
 Ws3d ws3d(const vfp3d_weights* w, long long sG, long long sT3, long long C) {
   Ws3d L;
   L.m[0] = sG * 1024; L.m[1] = sG * 256; L.m[2] = sT3 * 64; L.m[3] = sT3 * 16;
-  L.t_slots[0] = ((size_t)sG * 2 + 3) / 4 * 4;
+  L.t_slots[0] = (size_t)sG * 4;
   L.t_slots[1] = L.t_slots[0] + (size_t)sG * 4;
   L.t_slots[2] = L.t_slots[1] + (size_t)sT3 * 4;
   L.t_head = L.t_slots[2] + (size_t)sT3 * 4;
@@ -1375,12 +1375,17 @@ Ws3d ws3d(const vfp3d_weights* w, long long sG, long long sT3, long long C) {
   return L;
 }
 
-// One packed pass: clips [c0, c1) of the input, frames cu[c0] .. cu[c1].
-int forward3d_pass(const vfp3d_weights* w, const uint8_t* frames_base, int frame_dtype, size_t frame_bytes, const int32_t* cu,
-                   int c0, int c1, float* emb_out, uint8_t* ws, cudaStream_t st) {
+size_t frame_bytes3d(int frame_dtype) {
+  return (size_t)12288 * (frame_dtype == VFP_FRAME_BF16 ? 2 : frame_dtype == VFP_FRAME_F32 ? 4 : 1);
+}
+
+// One packed pass: clips [c0, c1) of the input, clip i = len[i] frames from device address clip[i].
+int forward3d_pass(const vfp3d_weights* w, int frame_dtype, const void* const* clip, const int32_t* len, int c0, int c1,
+                   float* emb_out, uint8_t* ws, cudaStream_t st) {
   const int C = c1 - c0, fs = w->fs;
+  const size_t frame_bytes = frame_bytes3d(frame_dtype);
   long long sG = 0, sT3 = 0;
-  for (int i = c0; i < c1; ++i) { const Dims3d d = dims3d(cu[i + 1] - cu[i], fs); sG += d.G; sT3 += d.T3; }
+  for (int i = c0; i < c1; ++i) { const Dims3d d = dims3d(len[i], fs); sG += d.G; sT3 += d.T3; }
   const Ws3d L = ws3d(w, sG, sT3, C);
   // the per-pass tables (pageable host memory: the copy is staged before cudaMemcpyAsync returns, so the vector may go)
   std::vector<int32_t> tab(L.t_head + (size_t)C * 2, 0);
@@ -1389,9 +1394,13 @@ int forward3d_pass(const vfp3d_weights* w, const uint8_t* frames_base, int frame
   int32_t* head = tab.data() + L.t_head;
   long long gb = 0, tb = 0;   // first group / layer-3 position of the clip in the pass
   for (int i = c0; i < c1; ++i) {
-    const int f = cu[i] - cu[c0], T = cu[i + 1] - cu[i];
+    const int T = len[i];
     const Dims3d d = dims3d(T, fs);
-    for (int g = 0; g < d.G; ++g) { groups[(gb + g) * 2] = f + g * fs; groups[(gb + g) * 2 + 1] = T - g * fs; }
+    for (int g = 0; g < d.G; ++g) {   // L1Group {first frame of the group, frames left in the clip, 0}
+      const void* first = static_cast<const uint8_t*>(clip[i]) + (size_t)g * fs * frame_bytes;
+      memcpy(groups + (gb + g) * 4, &first, sizeof(first));
+      groups[(gb + g) * 4 + 2] = T - g * fs;
+    }
     auto slot = [](int32_t* s, long long in_base, int Ti, int t0) { s[0] = (int32_t)in_base; s[1] = Ti; s[2] = t0; s[3] = 0; };
     for (int to = 0; to < d.G; ++to) slot(slots[0] + (gb + to) * 4, gb, d.G, to - 1);         // layer 2: G -> G, stride 1
     for (int to = 0; to < d.T3; ++to) slot(slots[1] + (tb + to) * 4, gb, d.G, 2 * to - 1);    // layer 3: G -> T3, stride 2
@@ -1404,12 +1413,11 @@ int forward3d_pass(const vfp3d_weights* w, const uint8_t* frames_base, int frame
   __nv_bfloat16* A = reinterpret_cast<__nv_bfloat16*>(ws + L.a);
   __nv_bfloat16* act[4];
   for (int l = 0; l < 4; ++l) act[l] = reinterpret_cast<__nv_bfloat16*>(ws + L.act[l]);
-  const uint8_t* fr = frames_base + (size_t)cu[c0] * frame_bytes;
   for (int l = 0; l < 4; ++l) {
     if (l == 0) {   // layer 1 straight from the frames on the register-fragment tensor path, no im2col matrix
       const size_t smem = (((size_t)fs * 5 * 204 * 2 + 4 + 15) & ~size_t(15)) + 4 * 16 * 32 * 4;
       VFP_CUDA(ensure_dynamic_smem(reinterpret_cast<const void*>(conv3d_l1_kernel), 64 * 5 * 204 * 2 + 32 + 4 * 16 * 32 * 4));
-      conv3d_l1_kernel<<<(unsigned)(sG * 32), 128, smem, st>>>(fr, frame_dtype, reinterpret_cast<const int2*>(dtab), fs, w->l1_pack,
+      conv3d_l1_kernel<<<(unsigned)(sG * 32), 128, smem, st>>>(frame_dtype, reinterpret_cast<const L1Group*>(dtab), fs, w->l1_pack,
                                                              w->b[0], act[0]);
       continue;
     }
@@ -1438,19 +1446,20 @@ int forward3d_pass(const vfp3d_weights* w, const uint8_t* frames_base, int frame
   return 0;
 }
 
-// Checks a packed input and runs it in passes cut on clip boundaries, each as large as the workspace holds.
-int forward3d_packed(const char* who, const vfp3d_weights* w, const void* frames, int frame_dtype, const int32_t* cu, int n_clips,
-                     float* emb_out, void* workspace, size_t workspace_bytes, void* stream) {
-  const std::string name(who);
-  if (!w || !frames || !cu || !emb_out || !workspace) return fail(name + ": null argument");
+// The one planner of the 3-D model: checks clip i = len[i] frames at device address clip[i] (any placement: packed, separate
+// allocations, overlapping, aliased) and runs the clips in passes cut on clip boundaries, each as large as the workspace holds.
+int forward3d_clips(const std::string& name, const vfp3d_weights* w, const void* const* clip, const int32_t* len, int n_clips,
+                    int frame_dtype, float* emb_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!w || !clip || !len || !emb_out || !workspace) return fail(name + ": null argument");
   if (n_clips <= 0) return fail(name + ": n_clips must be positive");
-  if (frame_dtype == VFP_FRAME_U8_HWC) return fail(name + ": decoder-layout (HWC) frames are not supported by the 3-D model; pass planar (T, 3, 64, 64) frames");
-  if (frame_dtype != VFP_FRAME_U8 && frame_dtype != VFP_FRAME_BF16 && frame_dtype != VFP_FRAME_F32) return fail(name + ": planar u8 / bf16 / fp32 frames only");
-  if (cu[0] != 0) return fail(name + ": cu_seqlens[0] must be 0");
+  if (frame_dtype != VFP_FRAME_U8 && frame_dtype != VFP_FRAME_BF16 && frame_dtype != VFP_FRAME_F32 && frame_dtype != VFP_FRAME_U8_HWC)
+    return fail(name + ": unknown frame_dtype " + std::to_string(frame_dtype));
   for (int i = 0; i < n_clips; ++i) {
-    const int T = cu[i + 1] - cu[i];
-    if (cu[i + 1] < cu[i]) return fail(name + ": cu_seqlens is not monotone (decreases at clip " + std::to_string(i) + ")");
-    if (T == 0) return fail(name + ": clip " + std::to_string(i) + " has length 0");
+    const int T = len[i];
+    if (T <= 0) return fail(name + ": clip " + std::to_string(i) + " has length " + std::to_string(T));
+    if (!clip[i]) return fail(name + ": clip " + std::to_string(i) + " has a null frame pointer");
+    if (reinterpret_cast<uintptr_t>(clip[i]) % 16)
+      return fail(name + ": clip " + std::to_string(i) + "'s frame pointer is not 16-byte aligned (the frames are read in 16-byte vectors)");
     const Dims3d d = dims3d(T, w->fs);
     if (d.T3 > kHead3dMaxT)
       return fail(name + ": clip " + std::to_string(i) + " too long: " + std::to_string(T) + " frames give " + std::to_string(d.T3) +
@@ -1461,21 +1470,38 @@ int forward3d_packed(const char* who, const vfp3d_weights* w, const void* frames
                   std::to_string(T) + " frames need " + std::to_string(need) + ")");
   }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t frame_bytes = (size_t)12288 * (frame_dtype == VFP_FRAME_BF16 ? 2 : frame_dtype == VFP_FRAME_F32 ? 4 : 1);
   for (int c0 = 0; c0 < n_clips;) {
     int c1 = c0;   // every clip fits on its own (checked above): add clips while the pass still fits
     long long sG = 0, sT3 = 0;
     while (c1 < n_clips) {
-      const Dims3d d = dims3d(cu[c1 + 1] - cu[c1], w->fs);
+      const Dims3d d = dims3d(len[c1], w->fs);
       if (c1 > c0 && ws3d(w, sG + d.G, sT3 + d.T3, c1 - c0 + 1).total > workspace_bytes) break;
       sG += d.G; sT3 += d.T3; ++c1;
     }
-    if (int rc = forward3d_pass(w, static_cast<const uint8_t*>(frames), frame_dtype, frame_bytes, cu, c0, c1, emb_out,
-                                static_cast<uint8_t*>(workspace), st))
-      return rc;
+    if (int rc = forward3d_pass(w, frame_dtype, clip, len, c0, c1, emb_out, static_cast<uint8_t*>(workspace), st)) return rc;
     c0 = c1;
   }
   return 0;
+}
+
+// A packed input (clips back to back, prefix sums cu): the clip pointers are frames + cu[i] frames.
+int forward3d_packed(const char* who, const vfp3d_weights* w, const void* frames, int frame_dtype, const int32_t* cu, int n_clips,
+                     float* emb_out, void* workspace, size_t workspace_bytes, void* stream) {
+  const std::string name(who);
+  if (!w || !frames || !cu || !emb_out || !workspace) return fail(name + ": null argument");
+  if (n_clips <= 0) return fail(name + ": n_clips must be positive");
+  if (frame_dtype == VFP_FRAME_U8_HWC) return fail(name + ": decoder-layout (HWC) frames are not supported here; pass planar (T, 3, 64, 64) frames, or use vfp3d_forward_clips");
+  if (frame_dtype != VFP_FRAME_U8 && frame_dtype != VFP_FRAME_BF16 && frame_dtype != VFP_FRAME_F32) return fail(name + ": planar u8 / bf16 / fp32 frames only");
+  if (cu[0] != 0) return fail(name + ": cu_seqlens[0] must be 0");
+  const size_t frame_bytes = frame_bytes3d(frame_dtype);
+  std::vector<const void*> clip((size_t)n_clips);
+  std::vector<int32_t> len((size_t)n_clips);
+  for (int i = 0; i < n_clips; ++i) {
+    if (cu[i + 1] < cu[i]) return fail(name + ": cu_seqlens is not monotone (decreases at clip " + std::to_string(i) + ")");
+    clip[i] = static_cast<const uint8_t*>(frames) + (size_t)cu[i] * frame_bytes;
+    len[i] = cu[i + 1] - cu[i];
+  }
+  return forward3d_clips(name, w, clip.data(), len.data(), n_clips, frame_dtype, emb_out, workspace, workspace_bytes, stream);
 }
 }  // namespace
 
@@ -1586,6 +1612,12 @@ int vfp3d_forward_packed(const vfp3d_weights* w, const void* frames, int frame_d
                          float* emb_out, void* workspace, size_t workspace_bytes, void* stream) {
   return forward3d_packed("vfp3d_forward_packed", w, frames, frame_dtype, cu_seqlens_host, n_clips, emb_out, workspace, workspace_bytes,
                           stream);
+}
+
+int vfp3d_forward_clips(const vfp3d_weights* w, const void* const* clip_frames_host, const int32_t* lengths_host, int n_clips,
+                        int frame_dtype, float* emb_out, void* workspace, size_t workspace_bytes, void* stream) {
+  return forward3d_clips("vfp3d_forward_clips", w, clip_frames_host, lengths_host, n_clips, frame_dtype, emb_out, workspace,
+                         workspace_bytes, stream);
 }
 
 }  // extern "C"

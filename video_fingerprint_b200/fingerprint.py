@@ -347,13 +347,58 @@ class VideoFingerprintScanner:
         if not pieces:
             return result
         emb = self.model.fingerprint_clips(pieces).cpu().numpy()
+        self._combine_windows_3d(emb, spans, [int(v.shape[0]) for v in videos], result)
+        return result
+
+    def _combine_windows_3d(self, emb: np.ndarray, spans, totals: List[int], result: List[Optional[np.ndarray]]) -> None:
+        """result[v] for every (video, first row, rows) span: the row itself for a video of at most clip_length frames, else
+        the mean of its window rows, re-normalised (fingerprint.py:305-320)."""
+        clip_length = self.config.get("clip_length", 128)
         for v, row, k in spans:
-            if int(videos[v].shape[0]) <= clip_length:
+            if totals[v] <= clip_length:
                 result[v] = emb[row]
             else:
                 final = np.mean(np.ascontiguousarray(emb[row : row + k]), axis=0)
                 result[v] = final / np.linalg.norm(final)
+
+    def extract_fingerprints_3d_from_decoded(self, videos) -> List[Optional[np.ndarray]]:
+        """Decoded videos -> one embedding (or None) per video with the rule of `extract_fingerprint_3d_from_frames`, with
+        preprocessing and forward both on the device. Each video is (T_v, H_v, W_v, 3) uint8 at its own resolution, as an
+        array, a tensor or a list of frames (what `preprocess_frames_device` accepts). Only frames inside some window are
+        uploaded and resized (a 1 000-frame video at clip_length 128 needs at most 5 x 128), one decoder-layout buffer per run
+        of overlapping windows; the windows of ALL videos are views into those buffers and go through one `fingerprint_views`
+        call."""
+        _native.require_cuda()
+        clip_length = self.config.get("clip_length", 128)
+        views: List[torch.Tensor] = []
+        spans: List[Tuple[int, int, int]] = []   # (video, first row, rows) in the result of fingerprint_views
+        totals = [len(frames) for frames in videos]
+        for v, frames in enumerate(videos):
+            total = totals[v]
+            if total < 10:
+                continue
+            starts = self.window_starts_3d(total)
+            span = min(total, clip_length)
+            runs: List[List[int]] = []   # overlapping windows merged into runs [a, b) of frames
+            for s in starts:
+                if runs and s <= runs[-1][1]:
+                    runs[-1][1] = s + span
+                else:
+                    runs.append([s, s + span])
+            # a slice of an array or tensor is a view: each run is uploaded straight from the caller's frames, no host gather
+            bufs = [(a, b, preprocess_frames_device(frames[a:b], self.device)) for a, b in runs]
+            spans.append((v, len(views), len(starts)))
+            views += [u8[s - a : s - a + span] for s in starts for a, b, u8 in bufs if a <= s < b]
+        result: List[Optional[np.ndarray]] = [None] * len(totals)
+        if not views:
+            return result
+        emb = self.model.fingerprint_views(views).cpu().numpy()
+        self._combine_windows_3d(emb, spans, totals, result)
         return result
+
+    def extract_fingerprint_3d_from_decoded(self, frames) -> Optional[np.ndarray]:
+        """One decoded video (T, H, W, 3) uint8 -> its 3-D embedding, or None below 10 frames."""
+        return self.extract_fingerprints_3d_from_decoded([frames])[0]
 
     def extract_fingerprint_from_frames(self, clip: torch.Tensor) -> Optional[np.ndarray]:
         """clip: (T,3,64,64) preprocessed frames (what _preprocess_frames returns). <10 frames -> None."""

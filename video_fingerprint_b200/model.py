@@ -324,7 +324,8 @@ class VideoFingerprint3D(nn.Module):
     """The reference's 3-D CNN fingerprint model (model.py:406-512), inference only: same constructor arguments, same
     state_dict keys / shapes / default initialisation, same forward contract ((B,T,3,64,64) or (B,3,T,64,64) in [0,1] ->
     unit-norm (B, embedding_dim)); the compute is `vfp3d_forward` in libvfp_b200.so (im2col + tcgen05 GEMMs + a fused tail).
-    `fingerprint_packed` / `fingerprint_clips` take clips of different lengths in one call (`vfp3d_forward_packed`)."""
+    `fingerprint_packed` / `fingerprint_clips` take clips of different lengths in one call (`vfp3d_forward_packed`);
+    `fingerprint_views` takes device clips wherever they sit, including decoder-layout uint8 frames (`vfp3d_forward_clips`)."""
 
     def __init__(self, embedding_dim=256, frame_stride=32, dropout=0.2):
         super().__init__()
@@ -459,10 +460,7 @@ class VideoFingerprint3D(nn.Module):
                 cu[i] = acc
                 acc += t
             cu[n] = acc
-            # workspace for passes of clips_per_pass clips of the batch's mean length (at least the longest clip)
-            per = max(1, min(n, self.clips_per_pass))
-            pass_frames = total if per == n else max(max(lengths), -(-total * per // n))
-            ws = self._get_workspace(lib.vfp3d_forward_packed_workspace_bytes(C.c_void_p(weights), max(1, pass_frames), per), dev)
+            ws = self._packed_workspace(lib, weights, lengths, dev)
             emb = torch.empty((n, self.embedding_dim), dtype=torch.float32, device=dev)
             rc = lib.vfp3d_forward_packed(C.c_void_p(weights), C.c_void_p(frames.data_ptr()), code, C.cast(cu, C.c_void_p), n,
                                           C.c_void_p(emb.data_ptr()), C.c_void_p(ws.data_ptr()), ws.numel(),
@@ -470,9 +468,17 @@ class VideoFingerprint3D(nn.Module):
             _native.check(rc, "vfp3d_forward_packed")
         return emb
 
+    def _packed_workspace(self, lib, weights: int, lengths: List[int], dev) -> torch.Tensor:
+        """Workspace for passes of clips_per_pass clips of the batch's mean length (at least the longest clip)."""
+        n, total = len(lengths), sum(lengths)
+        per = max(1, min(n, self.clips_per_pass))
+        pass_frames = total if per == n else max(max(lengths), -(-total * per // n))
+        return self._get_workspace(lib.vfp3d_forward_packed_workspace_bytes(C.c_void_p(weights), max(1, pass_frames), per), dev)
+
     def fingerprint_clips(self, clips: Sequence[torch.Tensor]) -> torch.Tensor:
         """List of (T_i, 3, 64, 64) clips of one dtype -> (n, D) embeddings, one packed launch sequence (no padding, no masks).
-        Clips that are all on one device (or all on the host, then uploaded once) are concatenated there."""
+        Clips that are all on one device (or all on the host, then uploaded once) are concatenated there; for clips already
+        on the device, `fingerprint_views` gives the same bits without that copy."""
         if len({c.dtype for c in clips}) > 1:
             raise ValueError("clips must share one dtype (uint8 frames are scaled by 1/255, float frames are not)")
         lengths = [int(c.shape[0]) for c in clips]
@@ -481,6 +487,51 @@ class VideoFingerprint3D(nn.Module):
             dev = next(d for d in devices if d.type == "cuda")
             clips = [c.to(dev) for c in clips]
         return self.fingerprint_packed(torch.cat(list(clips), dim=0), lengths)
+
+    @torch.no_grad()
+    def fingerprint_views(self, clips: Sequence[torch.Tensor]) -> torch.Tensor:
+        """Device clips wherever they sit -> (n, embedding_dim) fp32 on their device, without copying a frame: each clip is a
+        contiguous CUDA tensor (T_i, 3, 64, 64) uint8 / bf16 / fp32, or decoder-layout (T_i, 64, 64, 3) uint8 (what
+        `preprocess_frames_device` returns), all of one dtype and layout on one device. Views such as `frames[s:s + L]` of
+        one buffer qualify, overlapping or repeated ones too. Row i has exactly the bits `forward` gives for clip i alone
+        (HWC and planar uint8 frames give the same bits). Raises ValueError rather than copying anything."""
+        _native.require_cuda()
+        if self.training:
+            raise RuntimeError("inference only: call .eval() first")
+        clips = list(clips)
+        if not clips:
+            raise ValueError("fingerprint_views needs at least one clip")
+        for i, c in enumerate(clips):
+            if not isinstance(c, torch.Tensor) or not c.is_cuda:
+                raise ValueError(f"clip {i} is not a CUDA tensor (fingerprint_views copies nothing; use fingerprint_clips for host clips)")
+            if not c.is_contiguous():
+                raise ValueError(f"clip {i} is not contiguous (its frames must be consecutive in memory)")
+        hwc = tuple(clips[0].shape[1:]) == (64, 64, 3)
+        dtype, dev = clips[0].dtype, clips[0].device
+        for i, c in enumerate(clips):
+            if c.dim() != 4 or tuple(c.shape[1:]) != ((64, 64, 3) if hwc else (3, 64, 64)):
+                raise ValueError(f"clip {i} has shape {tuple(c.shape)}; all clips must be (T, 3, 64, 64), or all (T, 64, 64, 3)")
+            if c.dtype != dtype:
+                raise ValueError(f"clip {i} is {c.dtype}, clip 0 is {dtype}: clips must share one dtype")
+            if c.device != dev:
+                raise ValueError(f"clip {i} is on {c.device}, clip 0 on {dev}: clips must be on one device")
+        codes = {torch.uint8: _native.FRAME_U8, torch.bfloat16: _native.FRAME_BF16, torch.float32: _native.FRAME_F32}
+        if dtype not in codes or (hwc and dtype != torch.uint8):
+            raise ValueError(f"{dtype} clips: planar clips are uint8 / bfloat16 / float32, decoder-layout clips uint8")
+        code = _native.FRAME_U8_HWC if hwc else codes[dtype]
+        n = len(clips)
+        lengths = [int(c.shape[0]) for c in clips]
+        ptrs = (C.c_void_p * n)(*[c.data_ptr() for c in clips])
+        lens = (C.c_int32 * n)(*lengths)
+        lib = _native.load()
+        with torch.cuda.device(dev):
+            weights = self._ensure_native()
+            ws = self._packed_workspace(lib, weights, lengths, dev)
+            emb = torch.empty((n, self.embedding_dim), dtype=torch.float32, device=dev)
+            rc = lib.vfp3d_forward_clips(C.c_void_p(weights), ptrs, lens, n, code, C.c_void_p(emb.data_ptr()), C.c_void_p(ws.data_ptr()),
+                                         ws.numel(), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+            _native.check(rc, "vfp3d_forward_clips")
+        return emb
 
     def compute_loss(self, *a, **k):
         raise NotImplementedError("training (model.py:514-582) is outside the B200 inference hot path")
