@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define VFP_ABI_VERSION 4
+#define VFP_ABI_VERSION 5
 
 /* frame element types accepted by vfp_forward (planar (T,3,64,64) frames as produced by
  * _preprocess_frames, fingerprint.py:186-214; U8 values are scaled by 1/255 on the device) */
@@ -81,6 +81,21 @@ size_t vfp_forward_workspace_bytes(int64_t frames_per_pass, int64_t clips_per_pa
 int vfp_forward(const vfp_weights* w, const void* frames, int frame_dtype, const int32_t* cu_seqlens_host,
                 int n_clips, float* emb_out, float* features_out, void* workspace, size_t workspace_bytes,
                 void* stream);
+
+/* Clips that sit anywhere in device memory, with the conventions of vfp_forward (asynchronous on `stream`, caller-owned
+ * buffers, the same pass planner and pipelines): `clip_frames_host` is a HOST array of n_clips device pointers, each at its
+ * clip's first frame; frame t of clip i starts `frame_pitch_bytes_host[i]` * t bytes after it (HOST array; NULL = frames back
+ * to back). Each frame is one contiguous planar (3, 64, 64) u8 / bf16 / fp32 or decoder-layout (64, 64, 3) u8 frame
+ * (VFP_FRAME_U8_HWC). Clips may be separate allocations, windows of one buffer (overlapping or repeated) or views with a
+ * frame stride such as every 3rd frame; no frame is copied. Row i of `emb_out` (and rows sum_{j<i} T_j .. of
+ * `features_out`, if non-null) have the bits vfp_forward gives for the same frames packed. Size the workspace with
+ * vfp_forward_workspace_bytes. A null or not 16-byte aligned pointer, a pitch below one frame or not a multiple of 16, a
+ * length below 1 or above the positional table, a workspace too small for the longest clip and an unknown frame_dtype are
+ * errors naming the clip, reported before anything is enqueued; beyond that the pointers are not validated (each must
+ * address lengths_host[i] readable frames on the current device). */
+int vfp_forward_clips(const vfp_weights* w, const void* const* clip_frames_host, const int64_t* frame_pitch_bytes_host,
+                      const int32_t* lengths_host, int n_clips, int frame_dtype, float* emb_out, float* features_out,
+                      void* workspace, size_t workspace_bytes, void* stream);
 
 /* All-pairs cosine/inner-product threshold join of a query row block against a database:
  * emits every (i, j, s) with s = <q_i, db_j> >= thr computed in fp32, i = q_row0 + local row (so a
@@ -156,7 +171,7 @@ int vfp3d_forward_clips(const vfp3d_weights* w, const void* const* clip_frames_h
 /* Frame preprocessing of the scanner (/root/reference/fingerprint.py:186-214 _preprocess_frames): cv2.resize(frame,
  * INTER_AREA) so that the short side becomes 64 (new size truncated with int() like the reference), then the centre
  * 64 x 64 crop. `frames_hwc`: device uint8 (n_frames, height, width, 3), all frames of one size; `out_hwc64`: device
- * uint8 (n_frames, 64, 64, 3), which vfp_forward and vfp3d_forward_clips accept as VFP_FRAME_U8_HWC (the /255 and the
+ * uint8 (n_frames, 64, 64, 3), which vfp_forward, vfp_forward_clips and vfp3d_forward_clips accept as VFP_FRAME_U8_HWC (the /255 and the
  * HWC->CHW permute of fingerprint.py:210-212 happen inside the first layer's loader). Bit-exact with OpenCV 4.x INTER_AREA: down-scaling (general,
  * integer-factor and 2 x 2 code paths) and, for frames with a side below 64 pixels, the up-scaling branch (8-bit fixed-point
  * bilinear kernels with the area coefficient rule). */

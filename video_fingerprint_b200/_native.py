@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, _LIB_NAME)
 LIB_PATH = os.environ.get("VFP_B200_LIB", LIB_PATH)  # development aid: load an experimental build
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 FRAME_U8, FRAME_BF16, FRAME_F32, FRAME_U8_HWC = 0, 1, 2, 3
 
 # every symbol include/vfp_b200.h declares (tests check the library exports exactly these)
@@ -25,6 +25,7 @@ EXPORTED_SYMBOLS = (
     "vfp_weights_embedding_dim",
     "vfp_forward_workspace_bytes",
     "vfp_forward",
+    "vfp_forward_clips",
     "vfp_join_workspace_bytes",
     "vfp_join_threshold",
     "vfp_topk_workspace_bytes",
@@ -90,6 +91,8 @@ def load() -> C.CDLL:
     lib.vfp_forward_workspace_bytes.argtypes = [i64, i64]
     lib.vfp_forward.restype = i32
     lib.vfp_forward.argtypes = [vp, vp, i32, vp, i32, vp, vp, vp, sz, vp]
+    lib.vfp_forward_clips.restype = i32
+    lib.vfp_forward_clips.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp, vp, sz, vp]
     lib.vfp_join_workspace_bytes.restype = sz
     lib.vfp_join_workspace_bytes.argtypes = [i64, i64, i64]
     lib.vfp_join_threshold.restype = i32

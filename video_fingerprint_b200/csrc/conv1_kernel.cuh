@@ -28,13 +28,13 @@ __device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
 }
 
-// Copy frame f into the padded HWC bf16 tile (interior cells only; the halo stays zero). Any of the accepted frame
-// formats: planar CHW uint8 / bf16 / fp32 (what _preprocess_frames returns, fingerprint.py:210-214) or decoder-layout
+// Copy the frame at `frame` into the padded HWC bf16 tile (interior cells only; the halo stays zero). Any of the accepted
+// frame formats: planar CHW uint8 / bf16 / fp32 (what _preprocess_frames returns, fingerprint.py:210-214) or decoder-layout
 // HWC uint8. uint8 values are divided by 255 like the reference does.
-__device__ __forceinline__ void stage_frame_hwc(const void* __restrict__ frames, int frame_dtype, long long f,
+__device__ __forceinline__ void stage_frame_hwc(const void* __restrict__ frame, int frame_dtype,
                                                 __nv_bfloat16* __restrict__ tile, int tid, int nthreads) {
   if (frame_dtype == kFrameU8) {
-    const uint32_t* src = reinterpret_cast<const uint32_t*>(static_cast<const uint8_t*>(frames) + f * 12288);
+    const uint32_t* src = reinterpret_cast<const uint32_t*>(frame);
 #pragma unroll 4
     for (int i = tid; i < 3072; i += nthreads) {
       const uint32_t q = __ldg(src + i);
@@ -49,7 +49,7 @@ __device__ __forceinline__ void stage_frame_hwc(const void* __restrict__ frames,
   } else if (frame_dtype == kFrameU8HWC) {
     // decoder layout (H, W, 3) uint8, i.e. what _preprocess_frames sees before its permute (fingerprint.py:210-212):
     // a frame row is 192 contiguous bytes = 192 contiguous elements of the padded HWC tile
-    const uint32_t* src = reinterpret_cast<const uint32_t*>(static_cast<const uint8_t*>(frames) + f * 12288);
+    const uint32_t* src = reinterpret_cast<const uint32_t*>(frame);
 #pragma unroll 4
     for (int i = tid; i < 3072; i += nthreads) {
       const uint32_t q = __ldg(src + i);
@@ -59,7 +59,7 @@ __device__ __forceinline__ void stage_frame_hwc(const void* __restrict__ frames,
       d[1] = __floats2bfloat162_rn((float)((q >> 16) & 0xFF) / 255.0f, (float)(q >> 24) / 255.0f);
     }
   } else if (frame_dtype == kFrameBF16) {
-    const uint2* src = reinterpret_cast<const uint2*>(static_cast<const __nv_bfloat16*>(frames) + f * 12288);
+    const uint2* src = reinterpret_cast<const uint2*>(frame);
 #pragma unroll 4
     for (int i = tid; i < 3072; i += nthreads) {
       const uint2 q = __ldg(src + i);
@@ -71,7 +71,7 @@ __device__ __forceinline__ void stage_frame_hwc(const void* __restrict__ frames,
       d[0] = lo.x; d[3] = lo.y; d[6] = hi.x; d[9] = hi.y;
     }
   } else {
-    const float4* src = reinterpret_cast<const float4*>(static_cast<const float*>(frames) + f * 12288);
+    const float4* src = reinterpret_cast<const float4*>(frame);
 #pragma unroll 4
     for (int i = tid; i < 3072; i += nthreads) {
       const float4 q = __ldg(src + i);
@@ -84,9 +84,10 @@ __device__ __forceinline__ void stage_frame_hwc(const void* __restrict__ frames,
   }
 }
 
-// wpack: [5 kh][4 n-tiles][32 lanes][2] packed bf16x2 B fragments, bias: [32] fp32 (BN folded)
+// frame_addr: [n_frames] device address of each frame (token_map_kernel); wpack: [5 kh][4 n-tiles][32 lanes][2] packed
+// bf16x2 B fragments, bias: [32] fp32 (BN folded)
 __global__ void __launch_bounds__(kC1Threads)
-conv1_stem_kernel(const void* __restrict__ frames, int frame_dtype, long long n_frames,
+conv1_stem_kernel(const unsigned long long* __restrict__ frame_addr, int frame_dtype, long long n_frames,
                   const uint32_t* __restrict__ wpack, const float* __restrict__ bias,
                   __nv_bfloat16* __restrict__ out) {
   __shared__ __align__(16) __nv_bfloat16 tile[kC1SmemElems];
@@ -117,7 +118,7 @@ conv1_stem_kernel(const void* __restrict__ frames, int frame_dtype, long long n_
   __syncthreads();
 
   for (long long f = blockIdx.x; f < n_frames; f += gridDim.x) {
-    stage_frame_hwc(frames, frame_dtype, f, tile, tid, kC1Threads);
+    stage_frame_hwc(reinterpret_cast<const void*>(__ldg(frame_addr + f)), frame_dtype, tile, tid, kC1Threads);
     __syncthreads();
 
     // ---- 64 m-tiles of 16 pixels, processed as 32 vertical PAIRS (output rows 2j, 2j+1; same 16 columns): in the

@@ -25,7 +25,8 @@
 // no per-element work that the tensor core can do instead (the bias).
 //
 // One CTA per SM, persistent over frames, 24 warps:
-//   WG0   warp 0        bulk-copy issuer (raw frame planes -> smem ring, L2 prefetch two frames ahead), weights once (TMA)
+//   WG0   warp 0        bulk-copy issuer (raw frame planes -> smem ring, L2 prefetch two frames ahead; each frame's address
+//                       comes from the pass's frame address table), weights once (TMA)
 //         warp 1        TMEM allocation + conv1 UMMA issuer (TS mode)
 //         warp 2        transposer (raw planes -> HWC bf16 tile), with WG5
 //         warp 3        conv2 UMMA issuer
@@ -77,7 +78,7 @@ struct StemTsParams {
   alignas(64) CUtensorMap tmap_w2;   // conv2 weights [64][320] bf16 (fused K order), box 64 x 64, SWIZZLE_128B
   alignas(64) CUtensorMap tmap_w1;   // conv1 stacked weights + bias rows [64][128] bf16, box 64 x 64, SWIZZLE_128B
   alignas(64) CUtensorMap tmap_out;  // conv2 output [frames*256][64] bf16, box 32 x 32, SWIZZLE_64B
-  const void* frames;
+  const unsigned long long* frame_addr;   // [n_frames] device address of each frame (16-byte aligned; token_map_kernel)
   int frame_dtype;
   long long n_frames;
   const float* c2_bias;  // [64]
@@ -241,15 +242,16 @@ __global__ void __launch_bounds__(kStemThreads, 1) stem_ts_kernel(const __grid_c
         mbar_arrive_expect_tx(w_full, (kStemWBlocks + 2) * 8192);
         for (int kb = 0; kb < kStemWBlocks; ++kb) tma_load_2d(&p.tmap_w2, w_full, w2buf + kb * 8192, kb * 64, 0);
         for (int kb = 0; kb < 2; ++kb) tma_load_2d(&p.tmap_w1, w_full, w1buf + kb * 8192, kb * 64, 0);
-        const uint8_t* base = static_cast<const uint8_t*>(p.frames);
-        const size_t frame_bytes = 3 * (size_t)plane_bytes;
+        const unsigned long long* addr = p.frame_addr + blockIdx.x;   // this CTA's frames: addr[li * gridDim.x]
         int slot = 0;
         uint32_t ph = 0;
         for (int li = 0; li < n_local; ++li) {
-          const uint8_t* src = base + (size_t)(blockIdx.x + (size_t)li * gridDim.x) * frame_bytes;
+          // one 8-byte load per frame: frames may sit anywhere (clip views, separate allocations), each one contiguous
+          const uint8_t* src = reinterpret_cast<const uint8_t*>(__ldg(addr + (size_t)li * gridDim.x));
           // the ring only holds one frame, so a copy is issued about one frame time before its data is needed: pull the
           // frame after next into L2 now and the copy only pays the L2 latency
-          if (li + 2 < n_local && !(kTsKnock & 4)) bulk_prefetch_l2(src + 2 * (size_t)gridDim.x * frame_bytes, 3 * plane_bytes);
+          if (li + 2 < n_local && !(kTsKnock & 4))
+            bulk_prefetch_l2(reinterpret_cast<const uint8_t*>(__ldg(addr + (size_t)(li + 2) * gridDim.x)), 3 * plane_bytes);
           for (int c = 0; c < 3; ++c) {
             mbar_wait_lazy(&raw_empty[slot], ph ^ 1);
             if (kTsKnock & 4) {

@@ -15,10 +15,18 @@ constexpr int kHeads = 8;
 constexpr int kHeadDim = 32;
 
 // ---------------------------------------------------------------------------------------------
-// token -> (clip, position) maps from the prefix sums
+// token -> (clip, position) maps from the prefix sums, and the frame address table of the pass
 // ---------------------------------------------------------------------------------------------
-__global__ void token_map_kernel(const int* __restrict__ cu, int n_clips, int n_tokens, int* __restrict__ tok_pos,
-                                 int* __restrict__ tok_len) {
+// Where a clip's frames are: frame t of the clip starts at addr + t * pitch (bytes). Clips may sit anywhere in device memory.
+struct FrameSrc {
+  unsigned long long addr;
+  long long pitch;
+};
+
+// Token t of the pass is frame tok_pos[t] of clip v; frame_addr[t] receives that frame's device address, which is all the
+// frame encoder's loaders read (the frames themselves need not be packed).
+__global__ void token_map_kernel(const int* __restrict__ cu, const FrameSrc* __restrict__ src, int n_clips, int n_tokens,
+                                 int* __restrict__ tok_pos, int* __restrict__ tok_len, unsigned long long* __restrict__ frame_addr) {
   pdl_launch_dependents();
   pdl_wait();
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -28,8 +36,11 @@ __global__ void token_map_kernel(const int* __restrict__ cu, int n_clips, int n_
     const int mid = (lo + hi) >> 1;
     if (cu[mid] <= t) lo = mid; else hi = mid;
   }
-  tok_pos[t] = t - cu[lo];
+  const int pos = t - cu[lo];
+  tok_pos[t] = pos;
   tok_len[t] = cu[lo + 1] - cu[lo];
+  const FrameSrc s = src[lo];
+  frame_addr[t] = s.addr + (unsigned long long)((long long)pos * s.pitch);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -274,7 +274,7 @@ int g_join_symmetric = 1;   // key 11: self joins screen the upper triangle only
 int g_join_panel_tiles = 512;  // key 12: database column tiles (of 128 rows) per L2 panel
 
 struct TokenWs {
-  size_t cu, att_items, tok_pos, tok_len, feat, xa, xb, xn, qkv, att, delta, delta2, h, logits, xbf, pooled, pooled_bf, head_h, total;
+  size_t cu, frame_src, att_items, frame_addr, tok_pos, tok_len, feat, xa, xb, xn, qkv, att, delta, delta2, h, logits, xbf, pooled, pooled_bf, head_h, total;
 };
 struct ConvWs {
   size_t c1, c2, c3, total;
@@ -287,8 +287,11 @@ TokenWs token_ws_layout(int64_t F, int64_t C) {
     off = align_up(off + bytes, 1024);
     return o;
   };
+  // cu, frame_src and att_items are consecutive: the host stages the three per-pass tables in one buffer, one copy
   L.cu = take((size_t)(C + 1) * 4);
+  L.frame_src = take((size_t)C * sizeof(FrameSrc));    // where each clip's frames are
   L.att_items = take((size_t)(F / 64 + C + 1) * 16);   // attention work items: <= F / 64 + C of them
+  L.frame_addr = take((size_t)F * 8);                  // device address of every frame of the pass (token_map_kernel)
   L.tok_pos = take((size_t)F * 4);
   L.tok_len = take((size_t)F * 4);
   L.feat = take((size_t)F * 256 * 2);
@@ -685,25 +688,25 @@ size_t vfp_forward_workspace_bytes(int64_t frames_per_pass, int64_t clips_per_pa
 
 namespace {
 
-// Frame encoder over frames [f0, f0 + F) of the packed input -> feat[f_rel0 + i] (bf16 [frames][256]).
-int encode_frames_pass(const vfp_weights* w, const uint8_t* frames, int frame_dtype, int64_t F, __nv_bfloat16* feat_out,
-                       uint8_t* conv_ws, cudaStream_t st) {
+// Frame encoder over the F frames at frame_addr[0 .. F) (device table, one address per frame) -> feat_out (bf16 [frames][256]).
+// `fused_ok`: every frame address is 16-byte aligned, as the fused stem's bulk copies need.
+int encode_frames_pass(const vfp_weights* w, const unsigned long long* frame_addr, int frame_dtype, bool fused_ok, int64_t F,
+                       __nv_bfloat16* feat_out, uint8_t* conv_ws, cudaStream_t st) {
   const ConvWs L = conv_ws_layout(F);
   __nv_bfloat16* c1a = reinterpret_cast<__nv_bfloat16*>(conv_ws + L.c1);
   __nv_bfloat16* c2a = reinterpret_cast<__nv_bfloat16*>(conv_ws + L.c2);
   __nv_bfloat16* c3a = reinterpret_cast<__nv_bfloat16*>(conv_ws + L.c3);
-  const size_t frame_bytes = (size_t)12288 * (frame_dtype == VFP_FRAME_BF16 ? 2 : frame_dtype == VFP_FRAME_F32 ? 4 : 1);
   // conv1 + conv2 can run in shorter "stem passes" (vfp_set_tuning key 0) so that conv1's output (64 KB per frame,
   // the largest tensor of the forward) is still in L2 when conv2 reads it; by default one stem pass = the conv pass.
   CUtensorMap ta;
   // the fused stem streams raw frame planes with 16-byte bulk copies; fp32 frames (48 KB) do not fit its smem ring
-  const bool fused = g_fused_stem && frame_dtype != VFP_FRAME_F32 && (reinterpret_cast<uintptr_t>(frames) & 15) == 0;
+  const bool fused = g_fused_stem && frame_dtype != VFP_FRAME_F32 && fused_ok;
   if (fused) {
     StemTsParams sp{};
     sp.tmap_w2 = w->tm_c2f;
     sp.tmap_w1 = w->tm_c1ts;
     if (make_tmap_out(&sp.tmap_out, c2a, (uint64_t)F * 256, 64, true)) return fail("tensor map encode failed (stem out)");
-    sp.frames = frames; sp.frame_dtype = frame_dtype; sp.n_frames = F;
+    sp.frame_addr = frame_addr; sp.frame_dtype = frame_dtype; sp.n_frames = F;
     sp.c2_bias = w->c2_b;
     VFP_CUDA(ensure_dynamic_smem(reinterpret_cast<const void*>(stem_ts_kernel), StemTsSmem::kTotal));
     g_prof.launches += 1;
@@ -716,7 +719,7 @@ int encode_frames_pass(const vfp_weights* w, const uint8_t* frames, int frame_dt
     g_prof.launches += 2;
     {
       const long long grid = std::min<long long>(n, (long long)device_sm_count() * 10);
-      conv1_stem_kernel<<<(unsigned)grid, kC1Threads, 0, st>>>(frames + (size_t)s0 * frame_bytes, frame_dtype, n, w->c1_wpack,
+      conv1_stem_kernel<<<(unsigned)grid, kC1Threads, 0, st>>>(frame_addr + s0, frame_dtype, n, w->c1_wpack,
                                                               w->c1_bias, c1a);
       g_prof.mark(kStConv1, st);
     }
@@ -781,16 +784,18 @@ int encode_frames_pass(const vfp_weights* w, const uint8_t* frames, int frame_dt
   return 0;
 }
 
-// One token pass: clips [c0, c1) = frames [f0, f0 + F) of the packed input.
-int forward_pass(const vfp_weights* w, const uint8_t* frames_base, int frame_dtype, size_t frame_bytes,
-                 const int32_t* cu_host, int c0, int c1, float* emb_out, float* features_out, uint8_t* ws,
-                 cudaStream_t st) {
+// One token pass: clips [c0, c1), whose frames are src[c0 .. c1) (host records), = rows [f0, f0 + F) of the packed
+// features (cu_host: prefix sums of the clip lengths).
+int forward_pass(const vfp_weights* w, const FrameSrc* src, int frame_dtype, bool fused_ok, const int64_t* cu_host, int c0,
+                 int c1, float* emb_out, float* features_out, uint8_t* ws, cudaStream_t st) {
   const int C = c1 - c0;
   const int64_t f0 = cu_host[c0];
   const int64_t F = cu_host[c1] - f0;
   const TokenWs L = token_ws_layout(F, C);
   uint8_t* conv_ws = ws + L.total;
   int* d_cu = reinterpret_cast<int*>(ws + L.cu);
+  const FrameSrc* d_src = reinterpret_cast<const FrameSrc*>(ws + L.frame_src);
+  unsigned long long* frame_addr = reinterpret_cast<unsigned long long*>(ws + L.frame_addr);
   int* tok_pos = reinterpret_cast<int*>(ws + L.tok_pos);
   int* tok_len = reinterpret_cast<int*>(ws + L.tok_len);
   __nv_bfloat16* feat = reinterpret_cast<__nv_bfloat16*>(ws + L.feat);
@@ -808,32 +813,35 @@ int forward_pass(const vfp_weights* w, const uint8_t* frames_base, int frame_dty
   __nv_bfloat16* pooled_bf = reinterpret_cast<__nv_bfloat16*>(ws + L.pooled_bf);
   __nv_bfloat16* head_h = reinterpret_cast<__nv_bfloat16*>(ws + L.head_h);
 
-  // clip prefix sums relative to this pass
+  // The per-pass tables, staged in one host buffer laid out like the workspace from L.cu on and copied with one call:
+  // clip prefix sums relative to this pass, the clips' frame records, and the attention work items (64 query tokens of
+  // one clip each, {first query token, clip start, clip end, 0}).
   std::vector<int32_t> cu_rel(C + 1);
-  int max_T = 0;
   for (int i = 0; i <= C; ++i) cu_rel[i] = (int32_t)(cu_host[c0 + i] - f0);
-  for (int i = 0; i < C; ++i) max_T = std::max(max_T, cu_rel[i + 1] - cu_rel[i]);
-  g_prof.mark(-1, st);
-  g_prof.launches += 8 + 7 * (unsigned long long)w->n_attn;
-  VFP_CUDA(cudaMemcpyAsync(d_cu, cu_rel.data(), (size_t)(C + 1) * 4, cudaMemcpyHostToDevice, st));
-  // attention work items: 64 query tokens of one clip each, {first query token, clip start, clip end, 0}
-  std::vector<int32_t> items_host;
-  items_host.reserve((size_t)(F / kAttRows + C) * 4);
+  size_t n_items = 0;
+  for (int i = 0; i < C; ++i) n_items += (size_t)(cu_rel[i + 1] - cu_rel[i] + kAttRows - 1) / kAttRows;
+  std::vector<uint8_t> tables(L.att_items - L.cu + n_items * 16);
+  memcpy(tables.data(), cu_rel.data(), (size_t)(C + 1) * 4);
+  memcpy(tables.data() + (L.frame_src - L.cu), src + c0, (size_t)C * sizeof(FrameSrc));
+  int32_t* items_host = reinterpret_cast<int32_t*>(tables.data() + (L.att_items - L.cu));
   for (int i = 0; i < C; ++i)
     for (int q = cu_rel[i]; q < cu_rel[i + 1]; q += kAttRows) {
-      items_host.push_back(q); items_host.push_back(cu_rel[i]); items_host.push_back(cu_rel[i + 1]); items_host.push_back(0);
+      items_host[0] = q; items_host[1] = cu_rel[i]; items_host[2] = cu_rel[i + 1]; items_host[3] = 0;
+      items_host += 4;
     }
-  const size_t n_items = items_host.size() / 4;
+  g_prof.mark(-1, st);
+  g_prof.launches += 8 + 7 * (unsigned long long)w->n_attn;
   int4* att_items = reinterpret_cast<int4*>(ws + L.att_items);
-  VFP_CUDA(cudaMemcpyAsync(att_items, items_host.data(), items_host.size() * 4, cudaMemcpyHostToDevice, st));
-  // cu_rel is pageable: the copy is staged before the call returns, so the vector may die with this scope.
-  VFP_CUDA(launch_kernel(token_map_kernel, dim3((unsigned)((F + 255) / 256)), dim3(256), 0, st, d_cu, C, (int)F, tok_pos, tok_len));
+  // pageable source: the copy is staged before the call returns, so the vector may die with this scope
+  VFP_CUDA(cudaMemcpyAsync(d_cu, tables.data(), tables.size(), cudaMemcpyHostToDevice, st));
+  VFP_CUDA(launch_kernel(token_map_kernel, dim3((unsigned)((F + 255) / 256)), dim3(256), 0, st, (const int*)d_cu, d_src, C, (int)F,
+                         tok_pos, tok_len, frame_addr));
   g_prof.mark(kStMisc, st);
 
   // ---- frame encoder, one conv pass at a time (frames are independent: slices ignore clip boundaries) ----
   for (int64_t s0 = 0; s0 < F; s0 += g_conv_pass_frames) {
     const int64_t n = std::min<int64_t>(g_conv_pass_frames, F - s0);
-    if (int rc = encode_frames_pass(w, frames_base + (size_t)(f0 + s0) * frame_bytes, frame_dtype, n, feat + s0 * 256, conv_ws, st))
+    if (int rc = encode_frames_pass(w, frame_addr + s0, frame_dtype, fused_ok, n, feat + s0 * 256, conv_ws, st))
       return rc;
   }
   // ---- token embedding: x = Wtok feat + btok + pe[pos] ----
@@ -976,25 +984,23 @@ int forward_pass(const vfp_weights* w, const uint8_t* frames_base, int frame_dty
   return 0;
 }
 
-}  // namespace
-
-extern "C" {
-
-int vfp_forward(const vfp_weights* w, const void* frames, int frame_dtype, const int32_t* cu, int n_clips,
-                float* emb_out, float* features_out, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!w || !frames || !cu || !emb_out || !workspace) return fail("vfp_forward: null argument");
-  if (n_clips <= 0) return fail("vfp_forward: n_clips must be positive");
-  if (frame_dtype < 0 || frame_dtype > 3) return fail("vfp_forward: unknown frame dtype");
-  const size_t frame_bytes = (size_t)12288 * (frame_dtype == VFP_FRAME_BF16 ? 2 : frame_dtype == VFP_FRAME_F32 ? 4 : 1);
-  if (cu[0] != 0) return fail("vfp_forward: cu_seqlens[0] must be 0");
-  int max_T = 0;
+// The one planner of the attention model. Clip i is len[i] frames, frame t at device address src[i].addr + t * src[i].pitch:
+// clips may be packed back to back, separate allocations, views with any frame stride, overlapping or repeated. Checks the
+// lengths and the workspace, then runs the clips in token passes cut on clip boundaries, dealt round-robin onto the pipelines.
+// `aligned`: every address and pitch is a multiple of 16 bytes, which the fused stem's bulk copies need.
+int forward_clips(const std::string& name, const vfp_weights* w, const FrameSrc* src, const int32_t* len, int n_clips,
+                  int frame_dtype, bool aligned, float* emb_out, float* features_out, void* workspace, size_t workspace_bytes,
+                  void* stream) {
+  std::vector<int64_t> cu((size_t)n_clips + 1, 0);   // prefix sums: clip i owns rows cu[i] .. cu[i+1] of the features
+  int max_T = 0, longest = 0;
   for (int i = 0; i < n_clips; ++i) {
-    const int T = cu[i + 1] - cu[i];
-    if (T <= 0) return fail("vfp_forward: clip " + std::to_string(i) + " has no frames");
+    const int T = len[i];
+    if (T <= 0) return fail(name + ": clip " + std::to_string(i) + " has no frames");
     if (T > w->pe_len)   // the positional table of the checkpoint (model.py:77: max_len 10000) is the only length limit
-      return fail("vfp_forward: clip " + std::to_string(i) + " has " + std::to_string(T) + " frames; the positional table holds " +
+      return fail(name + ": clip " + std::to_string(i) + " has " + std::to_string(T) + " frames; the positional table holds " +
                   std::to_string(w->pe_len));
-    max_T = std::max(max_T, T);
+    if (T > max_T) { max_T = T; longest = i; }
+    cu[i + 1] = cu[i] + T;
   }
   const int64_t total = cu[n_clips];
   // The workspace is cut into equal slices, one per pipeline; a pipeline = an internal stream that takes every
@@ -1014,8 +1020,8 @@ int vfp_forward(const vfp_weights* w, const void* frames, int frame_dtype, const
   while (n_pipes > 1 && fit(slice_bytes(n_pipes)) < max_T) --n_pipes;
   const int64_t pass_frames = fit(slice_bytes(n_pipes));
   if (pass_frames < max_T)
-    return fail("vfp_forward: workspace of " + std::to_string(workspace_bytes) + " bytes cannot hold the longest clip (" +
-                std::to_string(max_T) + " frames need " + std::to_string(forward_ws_total(max_T, 1)) + ")");
+    return fail(name + ": workspace of " + std::to_string(workspace_bytes) + " bytes cannot hold the longest clip (clip " +
+                std::to_string(longest) + ": " + std::to_string(max_T) + " frames need " + std::to_string(forward_ws_total(max_T, 1)) + ")");
   const size_t slice = slice_bytes(n_pipes);
   // passes of about equal size, a multiple of n_pipes of them
   int64_t n_pass = (total + pass_frames - 1) / pass_frames;
@@ -1034,9 +1040,9 @@ int vfp_forward(const vfp_weights* w, const void* frames, int frame_dtype, const
   int c0 = 0, pass = 0;
   while (c0 < n_clips && rc == 0) {
     int c1 = c0 + 1;   // a clip always fits (pass_frames >= max_T); add clips up to the target, never past the slice capacity
-    while (c1 < n_clips && (int64_t)cu[c1 + 1] - cu[c0] <= pass_frames && (int64_t)cu[c1] - cu[c0] < target) ++c1;
+    while (c1 < n_clips && cu[c1 + 1] - cu[c0] <= pass_frames && cu[c1] - cu[c0] < target) ++c1;
     const int p = pass % n_pipes;
-    rc = forward_pass(w, static_cast<const uint8_t*>(frames), frame_dtype, frame_bytes, cu, c0, c1, emb_out, features_out,
+    rc = forward_pass(w, src, frame_dtype, aligned, cu.data(), c0, c1, emb_out, features_out,
                       static_cast<uint8_t*>(workspace) + (size_t)p * slice, pipe[p]);
     c0 = c1;
     ++pass;
@@ -1053,6 +1059,59 @@ int vfp_forward(const vfp_weights* w, const void* frames, int frame_dtype, const
     cudaEventDestroy(fork);
   }
   return rc;
+}
+
+size_t frame_bytes_of(int frame_dtype) {
+  return (size_t)12288 * (frame_dtype == VFP_FRAME_BF16 ? 2 : frame_dtype == VFP_FRAME_F32 ? 4 : 1);
+}
+
+}  // namespace
+
+extern "C" {
+
+int vfp_forward(const vfp_weights* w, const void* frames, int frame_dtype, const int32_t* cu, int n_clips,
+                float* emb_out, float* features_out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!w || !frames || !cu || !emb_out || !workspace) return fail("vfp_forward: null argument");
+  if (n_clips <= 0) return fail("vfp_forward: n_clips must be positive");
+  if (frame_dtype < 0 || frame_dtype > 3) return fail("vfp_forward: unknown frame dtype");
+  const size_t frame_bytes = frame_bytes_of(frame_dtype);
+  if (cu[0] != 0) return fail("vfp_forward: cu_seqlens[0] must be 0");
+  // the packed frames as clip records with a dense pitch; an unaligned buffer takes the two-kernel stem, as it always has
+  std::vector<FrameSrc> src((size_t)n_clips);
+  std::vector<int32_t> len((size_t)n_clips);
+  for (int i = 0; i < n_clips; ++i) {
+    src[i].addr = reinterpret_cast<uintptr_t>(frames) + (unsigned long long)cu[i] * frame_bytes;
+    src[i].pitch = (long long)frame_bytes;
+    len[i] = cu[i + 1] - cu[i];
+  }
+  const bool aligned = (reinterpret_cast<uintptr_t>(frames) & 15) == 0;
+  return forward_clips("vfp_forward", w, src.data(), len.data(), n_clips, frame_dtype, aligned, emb_out, features_out, workspace,
+                       workspace_bytes, stream);
+}
+
+int vfp_forward_clips(const vfp_weights* w, const void* const* clip_frames_host, const int64_t* frame_pitch_bytes_host,
+                      const int32_t* lengths_host, int n_clips, int frame_dtype, float* emb_out, float* features_out,
+                      void* workspace, size_t workspace_bytes, void* stream) {
+  const std::string name = "vfp_forward_clips";
+  if (!w || !clip_frames_host || !lengths_host || !emb_out || !workspace) return fail(name + ": null argument");
+  if (n_clips <= 0) return fail(name + ": n_clips must be positive");
+  if (frame_dtype < 0 || frame_dtype > 3) return fail(name + ": unknown frame_dtype " + std::to_string(frame_dtype));
+  const long long frame_bytes = (long long)frame_bytes_of(frame_dtype);
+  std::vector<FrameSrc> src((size_t)n_clips);
+  for (int i = 0; i < n_clips; ++i) {
+    const uintptr_t a = reinterpret_cast<uintptr_t>(clip_frames_host[i]);
+    const long long pitch = frame_pitch_bytes_host ? (long long)frame_pitch_bytes_host[i] : frame_bytes;
+    if (!a) return fail(name + ": clip " + std::to_string(i) + " has a null frame pointer");
+    if (a % 16)
+      return fail(name + ": clip " + std::to_string(i) + "'s frame pointer is not 16-byte aligned (frames are read in 16-byte copies)");
+    if (pitch < frame_bytes || pitch % 16)
+      return fail(name + ": clip " + std::to_string(i) + " has a frame pitch of " + std::to_string(pitch) +
+                  " bytes; it must be a multiple of 16 and at least one frame (" + std::to_string(frame_bytes) + " bytes)");
+    src[i].addr = a;
+    src[i].pitch = pitch;
+  }
+  return forward_clips(name, w, src.data(), lengths_host, n_clips, frame_dtype, true, emb_out, features_out, workspace,
+                       workspace_bytes, stream);
 }
 
 // ---------------------------------------------------------------------------------------------

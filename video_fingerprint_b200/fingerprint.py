@@ -301,6 +301,29 @@ class VideoFingerprintScanner:
         emb = self.model.fingerprint_packed(u8, [u8.shape[0]])
         return emb[0].cpu().numpy()
 
+    def extract_fingerprints_from_decoded(self, videos) -> List[Optional[np.ndarray]]:
+        """Batched form of `extract_fingerprint_from_decoded`: decoded videos, each (T_v, H_v, W_v, 3) uint8 at its own
+        resolution as an array, a tensor or a list of frames -> one embedding per video, or None where fewer than 10 frames
+        are kept. Only the frames `subsample` keeps (a strided slice of the caller's frames) are uploaded and preprocessed on
+        the device; the decoder-layout buffers of ALL videos then go through one `fingerprint_views` call. Row for row
+        equal to `extract_fingerprint_from_decoded` on each video."""
+        _native.require_cuda()
+        views: List[torch.Tensor] = []
+        rows: List[int] = []   # videos with a row in the result of fingerprint_views
+        for v, frames in enumerate(videos):
+            keep = self.subsample(len(frames))   # range(0, total, skip)[:max_frames]
+            if len(keep) < 10:
+                continue
+            skip = keep[1] - keep[0]
+            views.append(preprocess_frames_device(frames[: keep[-1] + 1 : skip], self.device))
+            rows.append(v)
+        result: List[Optional[np.ndarray]] = [None] * len(videos)
+        if views:
+            emb = self.model.fingerprint_views(views).cpu().numpy()
+            for row, v in enumerate(rows):
+                result[v] = emb[row]
+        return result
+
     def window_starts_3d(self, total_frames: int) -> List[int]:
         """Start frames of the clip_length windows the 3-D scanner path fingerprints (fingerprint.py:293-303); one window
         starting at 0 (taking every frame) when the video is not longer than clip_length (fingerprint.py:280-291)."""

@@ -282,6 +282,73 @@ class VideoFingerprintAttention(nn.Module):
         lengths = [int(c.shape[0]) for c in clips]
         return self.fingerprint_packed(torch.cat([c.cuda() for c in clips], dim=0), lengths)
 
+    @torch.no_grad()
+    def fingerprint_views(self, clips: Sequence[torch.Tensor], return_features: bool = False):
+        """Device clips wherever they sit -> (n, embedding_dim) fp32 on their device, without copying a frame: each clip is a
+        CUDA tensor (T_i, 3, 64, 64) uint8 / bf16 / fp32, or decoder-layout (T_i, 64, 64, 3) uint8 (what
+        `preprocess_frames_device` returns), all of one dtype and layout on one device. Every frame must be contiguous; the
+        frames of a clip may be any positive stride apart, so `frames[s:s + L]`, `frames[::skip][:max_frames]` and
+        overlapping or repeated windows of one buffer all qualify. Row i has exactly the bits `fingerprint_packed` gives for
+        the same frames packed; with return_features=True the per-frame features (sum T_i, 256) follow, in clip order.
+        Raises ValueError rather than copying anything."""
+        _native.require_cuda()
+        if self.training:
+            raise RuntimeError("inference only: call .eval() first (the reference scanner does, fingerprint.py:33)")
+        clips = list(clips)
+        if not clips:
+            raise ValueError("fingerprint_views needs at least one clip")
+        for i, c in enumerate(clips):
+            if not isinstance(c, torch.Tensor) or not c.is_cuda:
+                raise ValueError(f"clip {i} is not a CUDA tensor (fingerprint_views copies nothing; use fingerprint_clips for host clips)")
+        hwc = tuple(clips[0].shape[1:]) == (64, 64, 3)
+        frame_shape = (64, 64, 3) if hwc else (3, 64, 64)
+        frame_strides = (192, 3, 1) if hwc else (4096, 64, 1)
+        dtype, dev = clips[0].dtype, clips[0].device
+        for i, c in enumerate(clips):
+            if c.dim() != 4 or tuple(c.shape[1:]) != frame_shape:
+                raise ValueError(f"clip {i} has shape {tuple(c.shape)}; all clips must be (T, 3, 64, 64), or all (T, 64, 64, 3)")
+            if c.dtype != dtype:
+                raise ValueError(f"clip {i} is {c.dtype}, clip 0 is {dtype}: clips must share one dtype")
+            if c.device != dev:
+                raise ValueError(f"clip {i} is on {c.device}, clip 0 on {dev}: clips must be on one device")
+            if c.shape[0] < 1:
+                raise ValueError(f"clip {i} has no frames")
+            if tuple(c.stride()[1:]) != frame_strides:
+                raise ValueError(f"clip {i} has strides {tuple(c.stride())}: each of its frames must be contiguous")
+            if c.shape[0] > 1 and c.stride(0) < 12288:
+                raise ValueError(f"clip {i} has a frame stride of {c.stride(0)} elements: frames must be a positive stride of "
+                                 "at least one frame (12288 elements) apart")
+        codes = {torch.uint8: _native.FRAME_U8, torch.bfloat16: _native.FRAME_BF16, torch.float32: _native.FRAME_F32}
+        if dtype not in codes or (hwc and dtype != torch.uint8):
+            raise ValueError(f"{dtype} clips: planar clips are uint8 / bfloat16 / float32, decoder-layout clips uint8")
+        code = _native.FRAME_U8_HWC if hwc else codes[dtype]
+        n = len(clips)
+        lengths = [int(c.shape[0]) for c in clips]
+        total = sum(lengths)
+        esize = clips[0].element_size()
+        # a one-frame clip has no frame stride to speak of (torch may report any value for it): dense
+        pitches = [c.stride(0) * esize if c.shape[0] > 1 else 12288 * esize for c in clips]
+        ptrs = (C.c_void_p * n)(*[c.data_ptr() for c in clips])
+        pitch = (C.c_int64 * n)(*pitches)
+        lens = (C.c_int32 * n)(*lengths)
+        lib = _native.load()
+        with torch.cuda.device(dev):
+            weights = self._ensure_native(dev.index)
+            # workspace and pipelines sized as in fingerprint_packed
+            pass_frames = max(min(total, self.frames_per_pass), max(lengths))
+            slices = max(1, min(int(self.pipelines), 4, -(-total // pass_frames)))
+            ws = self._get_workspace(slices * (lib.vfp_forward_workspace_bytes(pass_frames, min(pass_frames, n)) + 1024), dev)
+            emb = torch.empty((n, self.embedding_dim), dtype=torch.float32, device=dev)
+            feats = torch.empty((total, 256), dtype=torch.float32, device=dev) if return_features else None
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            lib.vfp_set_tuning(9, slices)
+            rc = lib.vfp_forward_clips(
+                C.c_void_p(weights), ptrs, pitch, lens, n, code, C.c_void_p(emb.data_ptr()),
+                C.c_void_p(feats.data_ptr() if feats is not None else None), C.c_void_p(ws.data_ptr()), ws.numel(), C.c_void_p(stream),
+            )
+            _native.check(rc, "vfp_forward_clips")
+        return (emb, feats) if return_features else emb
+
     # ------------------------------------------------------------------ reference-compatible forward
     def forward(self, video: torch.Tensor, return_features: bool = False):
         """Same contract as model.py:272-298, including the `(B,3,T,H,W)` layout sniff on `shape[1] == 3`."""
