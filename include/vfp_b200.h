@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define VFP_ABI_VERSION 5
+#define VFP_ABI_VERSION 6
 
 /* frame element types accepted by vfp_forward (planar (T,3,64,64) frames as produced by
  * _preprocess_frames, fingerprint.py:186-214; U8 values are scaled by 1/255 on the device) */
@@ -99,14 +99,21 @@ int vfp_forward_clips(const vfp_weights* w, const void* const* clip_frames_host,
 
 /* All-pairs cosine/inner-product threshold join of a query row block against a database:
  * emits every (i, j, s) with s = <q_i, db_j> >= thr computed in fp32, i = q_row0 + local row (so a
- * row-block shard reports global indices). `q`/`db` are device fp32 (n, dim) row-major, dim == 256.
+ * row-block shard reports global indices). `q`/`db` are device fp32 (n, dim) row-major with 16 <= dim <= 512 and
+ * dim % 16 == 0 (the width rule of vfp_pair_stats); any other dim is an error naming it. The screen runs on bf16 copies of
+ * 2 * dim bytes per row in ceil(dim / 64) K blocks of 64 columns (TMA zero-fills the columns past dim); at dim == 256 it
+ * launches the kernels of earlier versions and gives the same bits.
  * `screen_margin` must be >= 2^-8 * max|q_i| * max|db_j| (0.004 for unit vectors): the tensor-core
  * screen runs in bf16 at thr - screen_margin and survivors are re-scored in fp32.
  * counts_out (device, 2 x uint64): [0] = number of result pairs (may exceed `capacity`; only the first
  * `capacity` are stored, in no particular order), [1] = number of screen candidates (if it exceeds the
  * candidate capacity implied by the workspace the result is incomplete and the caller must retry with
- * the workspace vfp_join_workspace_bytes(..., candidates) reports). */
+ * the workspace vfp_join_workspace_bytes_dim(..., candidates, dim) reports). The workspace holds both bf16 copies and the
+ * candidates; what is left after the copies of `dim`-wide rows sets the candidate capacity, and a workspace that cannot hold
+ * them plus 1024 candidates (e.g. one sized for a smaller dim) is rejected. vfp_join_workspace_bytes is the dim == 256 size;
+ * the _dim form returns 0 for an unsupported dim. */
 size_t vfp_join_workspace_bytes(int64_t n_q, int64_t n_db, int64_t candidate_capacity);
+size_t vfp_join_workspace_bytes_dim(int64_t n_q, int64_t n_db, int64_t candidate_capacity, int dim);
 int vfp_join_threshold(const float* q, const float* db, int64_t n_q, int64_t n_db, int dim, int64_t q_row0,
                        float thr, float screen_margin, int32_t* out_i, int32_t* out_j, float* out_s,
                        int64_t capacity, uint64_t* counts_out, void* workspace, size_t workspace_bytes,
@@ -114,12 +121,15 @@ int vfp_join_threshold(const float* q, const float* db, int64_t n_q, int64_t n_d
 
 /* Exact flat inner-product top-k (the arithmetic of faiss.IndexFlatIP.search): for every query row the k
  * largest <q_i, db_j> in fp32, sorted by (score descending, index ascending). out_s (n_q, k) fp32,
- * out_idx (n_q, k) int64, device memory. k <= 32, dim == 256. The tensor-core screen keeps the 64 best bf16 scores
+ * out_idx (n_q, k) int64, device memory. k <= 32; dim follows the rule of vfp_join_threshold (16 <= dim <= 512,
+ * dim % 16 == 0), and at dim == 256 the same kernels and bits as earlier versions. The tensor-core screen keeps the 64 best bf16 scores
  * per query, which are re-scored in fp32; `flags_out` (device, 2 x uint64): [0] = query rows whose exactness could
  * not be proven from the screen bound (`screen_margin`, as for the join) and were recomputed by the exact fp32
  * scan, [1] != 0 = that fallback overflowed (more than 8192 such rows or more than 512 tied candidates for one
- * row) and the result must be discarded. */
+ * row) and the result must be discarded. vfp_topk_workspace_bytes is the dim == 256 size; the _dim form (0 for an
+ * unsupported dim) is what a call with that dim needs at least: a smaller workspace is rejected. */
 size_t vfp_topk_workspace_bytes(int64_t n_q, int64_t n_db, int k);
+size_t vfp_topk_workspace_bytes_dim(int64_t n_q, int64_t n_db, int k, int dim);
 int vfp_topk_ip(const float* q, const float* db, int64_t n_q, int64_t n_db, int dim, int k,
                 float screen_margin, float* out_s, int64_t* out_idx, uint64_t* flags_out, void* workspace,
                 size_t workspace_bytes, void* stream);

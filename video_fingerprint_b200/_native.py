@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, _LIB_NAME)
 LIB_PATH = os.environ.get("VFP_B200_LIB", LIB_PATH)  # development aid: load an experimental build
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 FRAME_U8, FRAME_BF16, FRAME_F32, FRAME_U8_HWC = 0, 1, 2, 3
 
 # every symbol include/vfp_b200.h declares (tests check the library exports exactly these)
@@ -27,8 +27,10 @@ EXPORTED_SYMBOLS = (
     "vfp_forward",
     "vfp_forward_clips",
     "vfp_join_workspace_bytes",
+    "vfp_join_workspace_bytes_dim",
     "vfp_join_threshold",
     "vfp_topk_workspace_bytes",
+    "vfp_topk_workspace_bytes_dim",
     "vfp_topk_ip",
     "vfp3d_weights_create",
     "vfp3d_weights_destroy",
@@ -95,10 +97,14 @@ def load() -> C.CDLL:
     lib.vfp_forward_clips.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp, vp, sz, vp]
     lib.vfp_join_workspace_bytes.restype = sz
     lib.vfp_join_workspace_bytes.argtypes = [i64, i64, i64]
+    lib.vfp_join_workspace_bytes_dim.restype = sz
+    lib.vfp_join_workspace_bytes_dim.argtypes = [i64, i64, i64, i32]
     lib.vfp_join_threshold.restype = i32
     lib.vfp_join_threshold.argtypes = [vp, vp, i64, i64, i32, i64, f32, f32, vp, vp, vp, i64, vp, vp, sz, vp]
     lib.vfp_topk_workspace_bytes.restype = sz
     lib.vfp_topk_workspace_bytes.argtypes = [i64, i64, i32]
+    lib.vfp_topk_workspace_bytes_dim.restype = sz
+    lib.vfp_topk_workspace_bytes_dim.argtypes = [i64, i64, i32, i32]
     lib.vfp_topk_ip.restype = i32
     lib.vfp_topk_ip.argtypes = [vp, vp, i64, i64, i32, i32, f32, vp, vp, vp, vp, sz, vp]
     lib.vfp3d_weights_create.restype = i32

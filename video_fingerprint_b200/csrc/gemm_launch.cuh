@@ -139,13 +139,13 @@ inline cudaError_t launch_gemm_bres(const CUtensorMap& ta, const CUtensorMap& tb
   return launch_kernel(kernel, dim3(grid), dim3(gemm_threads<BLOCK_N, Epi>()), kSmem, stream, ta, tb, shape, ep);
 }
 
-template <int STAGES, class Epi>
+template <int STAGES, int KB, class Epi>
 inline cudaError_t launch_gemm_ares(const CUtensorMap& ta, const CUtensorMap& tb, const AresShape& shape,
                                     const typename Epi::Params& ep, cudaStream_t stream) {
-  using L = AresSmemLayout<STAGES>;
+  using L = AresSmemLayout<STAGES, KB>;
   constexpr int kSmem = L::kTotal + Epi::kExtraSmemBytes;
   static_assert(kSmem <= 232448, "shared memory budget");
-  auto kernel = gemm_ares_tcgen05_kernel<STAGES, Epi>;
+  auto kernel = gemm_ares_tcgen05_kernel<STAGES, KB, Epi>;
   if (cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), kSmem); e != cudaSuccess) return e;
   const long long total = (long long)shape.m_super * shape.n_panels;
   if (total <= 0) return cudaSuccess;
@@ -153,13 +153,13 @@ inline cudaError_t launch_gemm_ares(const CUtensorMap& ta, const CUtensorMap& tb
   return launch_kernel(kernel, dim3(grid), dim3(gemm_threads<kAresBlockN, Epi>()), kSmem, stream, ta, tb, shape, ep);
 }
 
-template <int STAGES, class Epi>
+template <int STAGES, int KB, class Epi>
 inline cudaError_t launch_gemm_ares2(const CUtensorMap& ta, const CUtensorMap& tb, const AresShape& shape,
                                      const typename Epi::Params& ep, cudaStream_t stream) {
-  using L = Ares2SmemLayout<STAGES>;
+  using L = Ares2SmemLayout<STAGES, KB>;
   constexpr int kSmem = L::kTotal + Epi::kExtraSmemBytes;
   static_assert(kSmem <= 232448, "shared memory budget");
-  auto kernel = gemm_ares2_tcgen05_kernel<STAGES, Epi>;
+  auto kernel = gemm_ares2_tcgen05_kernel<STAGES, KB, Epi>;
   if (cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), kSmem); e != cudaSuccess) return e;
   const long long total = (long long)shape.m_super * shape.n_panels;
   if (total <= 0) return cudaSuccess;

@@ -549,9 +549,10 @@ gemm_bres_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
 // `tri` (self joins): S is symmetric, so column tiles that lie entirely below the diagonal of the item's rows are
 // skipped; the epilogue keeps j >= i and the re-score kernel emits the mirrored pair.
 // =================================================================================================
+// KB (template parameter of both kernels) = resident K blocks of 64 columns, ceil(dim / 64): 4 for the 256-wide embeddings the
+// models produce by default. Columns past dim in the last block are zero-filled by the TMA unit and add +0 to every score.
 constexpr int kAresMT = 2;
 constexpr int kAresBlockN = 128;
-constexpr int kAresKB = 4;   // K = 256 = 4 blocks of 64
 
 struct AresShape {
   int m_super;        // super-tiles of kAresMT * 128 query rows
@@ -583,21 +584,21 @@ struct AresWalk {
   }
 };
 
-template <int STAGES>
+template <int STAGES, int KB>
 struct AresSmemLayout {
   static constexpr int kABytes = kBlockM * 128;                      // one K block of one 128-row sub-tile
-  static constexpr int kAResident = kAresMT * kAresKB * kABytes;     // 128 KB
+  static constexpr int kAResident = kAresMT * KB * kABytes;          // 32 KB per K block (128 KB at KB = 4)
   static constexpr int kBBytes = kAresBlockN * 128;                  // one K block of a database tile
   static constexpr int kCore = kAResident + STAGES * kBBytes + 256;
   static constexpr int kCoreAligned = (kCore + 1023) / 1024 * 1024;
   static constexpr int kTotal = kCoreAligned + 1024;
 };
 
-template <int STAGES, class Epilogue>
+template <int STAGES, int KB, class Epilogue>
 __global__ void __launch_bounds__(gemm_threads<kAresBlockN, Epilogue>(), 1)
 gemm_ares_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                          const AresShape shape, const __grid_constant__ typename Epilogue::Params ep) {
-  using L = AresSmemLayout<STAGES>;
+  using L = AresSmemLayout<STAGES, KB>;
   constexpr int kAccCols = kAresMT * kAresBlockN;   // 256 columns per accumulator buffer
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -654,11 +655,11 @@ gemm_ares_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
 #pragma unroll
         for (int sub = 0; sub < kAresMT; ++sub)
 #pragma unroll
-          for (int kb = 0; kb < kAresKB; ++kb)
-            tma_load_2d(&tmap_a, a_full, smem_a + (sub * kAresKB + kb) * L::kABytes, kb * 64, (mts * kAresMT + sub) * kBlockM);
+          for (int kb = 0; kb < KB; ++kb)
+            tma_load_2d(&tmap_a, a_full, smem_a + (sub * KB + kb) * L::kABytes, kb * 64, (mts * kAresMT + sub) * kBlockM);
         for (int nt = nt0; nt < nt1; ++nt) {
 #pragma unroll
-          for (int kb = 0; kb < kAresKB; ++kb) {
+          for (int kb = 0; kb < KB; ++kb) {
             mbar_wait(&empty_bar[stage], phase ^ 1);
             mbar_arrive_expect_tx(&full_bar[stage], L::kBBytes);
             tma_load_2d(&tmap_b, &full_bar[stage], smem_b + stage * L::kBBytes, kb * 64, nt * kAresBlockN);
@@ -686,7 +687,7 @@ gemm_ares_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
           tc_fence_after();
           const uint32_t d_tmem = tmem_base + acc * kAccCols;
 #pragma unroll
-          for (int kb = 0; kb < kAresKB; ++kb) {
+          for (int kb = 0; kb < KB; ++kb) {
             mbar_wait(&full_bar[stage], phase);
             tc_fence_after();
             const uint64_t bdesc = umma_smem_desc_kmajor<128>(smem_u32(smem_b + stage * L::kBBytes));
@@ -694,7 +695,7 @@ gemm_ares_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
             for (int k = 0; k < 4; ++k) {
 #pragma unroll
               for (int sub = 0; sub < kAresMT; ++sub) {
-                const uint64_t adesc = umma_smem_desc_kmajor<128>(a_base + (sub * kAresKB + kb) * L::kABytes);
+                const uint64_t adesc = umma_smem_desc_kmajor<128>(a_base + (sub * KB + kb) * L::kABytes);
                 umma_bf16(d_tmem + sub * kAresBlockN, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
               }
             }
@@ -768,21 +769,21 @@ gemm_ares_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
 // =================================================================================================
 constexpr int kAres2BlockN = 256;
 
-template <int STAGES>
+template <int STAGES, int KB>
 struct Ares2SmemLayout {
   static constexpr int kABytes = kBlockM * 128;                   // one K block of this CTA's 128 query rows
-  static constexpr int kAResident = kAresKB * kABytes;            // 64 KB
+  static constexpr int kAResident = KB * kABytes;                 // 16 KB per K block (64 KB at KB = 4)
   static constexpr int kBBytes = (kAres2BlockN / 2) * 128;        // this CTA's half of one K block of a database tile
   static constexpr int kCore = kAResident + STAGES * kBBytes + 256;
   static constexpr int kCoreAligned = (kCore + 1023) / 1024 * 1024;
   static constexpr int kTotal = kCoreAligned + 1024;
 };
 
-template <int STAGES, class Epilogue>
+template <int STAGES, int KB, class Epilogue>
 __global__ void __launch_bounds__(gemm_threads<kAres2BlockN, Epilogue>(), 1)
 gemm_ares2_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                           const AresShape shape, const __grid_constant__ typename Epilogue::Params ep) {
-  using L = Ares2SmemLayout<STAGES>;
+  using L = Ares2SmemLayout<STAGES, KB>;
   constexpr int kEpiWarps = 4 * gemm_column_split<kAres2BlockN, Epilogue>();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -842,11 +843,11 @@ gemm_ares2_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gr
         a_phase ^= 1;
         if (leader) mbar_arrive_expect_tx(a_full, 2 * L::kAResident);
 #pragma unroll
-        for (int kb = 0; kb < kAresKB; ++kb)
+        for (int kb = 0; kb < KB; ++kb)
           tma_load_2d_2cta(&tmap_a, a_full_leader, smem_a + kb * L::kABytes, kb * 64, (mts * 2 + (int)crank) * kBlockM);
         for (int nt = nt0; nt < nt1; ++nt) {
 #pragma unroll
-          for (int kb = 0; kb < kAresKB; ++kb) {
+          for (int kb = 0; kb < KB; ++kb) {
             mbar_wait(&empty_bar[stage], phase ^ 1);
             if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * L::kBBytes);
             tma_load_2d_2cta(&tmap_b, mapa_u32(&full_bar[stage], 0), smem_b + stage * L::kBBytes, kb * 64,
@@ -875,7 +876,7 @@ gemm_ares2_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gr
           tc_fence_after();
           const uint32_t d_tmem = tmem_base + acc * kAres2BlockN;
 #pragma unroll
-          for (int kb = 0; kb < kAresKB; ++kb) {
+          for (int kb = 0; kb < KB; ++kb) {
             mbar_wait(&full_bar[stage], phase);
             tc_fence_after();
             const uint64_t adesc = umma_smem_desc_kmajor<128>(a_base + kb * L::kABytes);

@@ -118,19 +118,36 @@ __device__ __forceinline__ bool topk_better(float sa, int ia, float sb, int ib) 
   return sa > sb || (sa == sb && ia < ib);
 }
 
-// exact fp32 dot of the warp's query (8 values per lane in qv) with database row j
-__device__ __forceinline__ float warp_dot256(const float (&qv)[8], const float* __restrict__ db, long long j, int lane) {
-  const float4* r = reinterpret_cast<const float4*>(db + (size_t)j * 256) + lane * 2;
-  const float4 a = r[0], b = r[1];
-  float s = qv[0] * a.x + qv[1] * a.y + qv[2] * a.z + qv[3] * a.w + qv[4] * b.x + qv[5] * b.y + qv[6] * b.z + qv[7] * b.w;
+// One warp per fp32 dot product of two dim-wide rows (dim % 4 == 0, dim <= 128 * NV): lane l holds the NV float4 at
+// l * NV .. l * NV + NV - 1 of the row, zeros past dim (each adds +0). NV = ceil(dim / 128); at dim = 256 (NV = 2) this
+// is eight consecutive values per lane, the layout and summation order of the 256-wide kernels.
+template <int NV>
+__device__ __forceinline__ void warp_row_load(float (&v)[4 * NV], const float* __restrict__ row, int dim, int lane) {
+  const float4* r = reinterpret_cast<const float4*>(row) + lane * NV;
+#pragma unroll
+  for (int u = 0; u < NV; ++u) {
+    const float4 a = (dim == 128 * NV || lane * NV + u < dim / 4) ? r[u] : make_float4(0.f, 0.f, 0.f, 0.f);
+    v[4 * u] = a.x; v[4 * u + 1] = a.y; v[4 * u + 2] = a.z; v[4 * u + 3] = a.w;
+  }
+}
+
+// exact fp32 dot of the warp's query (warp_row_load layout in qv) with database row j
+template <int NV>
+__device__ __forceinline__ float warp_dot(const float (&qv)[4 * NV], const float* __restrict__ db, long long j, int dim, int lane) {
+  float dv[4 * NV];
+  warp_row_load<NV>(dv, db + (size_t)j * dim, dim, lane);
+  float s = qv[0] * dv[0];
+#pragma unroll
+  for (int i = 1; i < 4 * NV; ++i) s += qv[i] * dv[i];
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
   return s;
 }
 
 // One warp per query row: merge segment lists -> 64 approximate candidates -> exact re-score -> rank -> top k.
+template <int NV>
 __global__ void __launch_bounds__(256)
-topk_merge_rescore_kernel(const float* __restrict__ q, const float* __restrict__ db, long long n_q, long long n_db, int k,
+topk_merge_rescore_kernel(const float* __restrict__ q, const float* __restrict__ db, long long n_q, long long n_db, int dim, int k,
                           int n_segments, const float* __restrict__ part_s, const int* __restrict__ part_i, float margin,
                           float* __restrict__ out_s, long long* __restrict__ out_idx, int* __restrict__ flagged_rows,
                           float* __restrict__ flagged_tau, unsigned long long* __restrict__ flags /*[0] = flagged rows*/) {
@@ -170,17 +187,13 @@ topk_merge_rescore_kernel(const float* __restrict__ q, const float* __restrict__
   const int i_last = __shfl_sync(0xffffffffu, ci[1], 31);
 
   // ---- exact re-score ----
-  float qv[8];
-  {
-    const float4* r = reinterpret_cast<const float4*>(q + (size_t)row * 256) + lane * 2;
-    const float4 a = r[0], b = r[1];
-    qv[0] = a.x; qv[1] = a.y; qv[2] = a.z; qv[3] = a.w; qv[4] = b.x; qv[5] = b.y; qv[6] = b.z; qv[7] = b.w;
-  }
+  float qv[4 * NV];
+  warp_row_load<NV>(qv, q + (size_t)row * dim, dim, lane);
   float es[2] = {-INFINITY, -INFINITY};
   for (int c = 0; c < kTopKCand; ++c) {
     const int idx = __shfl_sync(0xffffffffu, ci[c >> 5], c & 31);
     if (idx < 0) continue;  // warp-uniform
-    const float s = warp_dot256(qv, db, idx, lane);
+    const float s = warp_dot<NV>(qv, db, idx, dim, lane);
     if (lane == (c & 31)) es[c >> 5] = s;
   }
   // ---- rank by (exact score desc, index asc) ----
@@ -224,8 +237,9 @@ topk_merge_rescore_kernel(const float* __restrict__ q, const float* __restrict__
 constexpr int kTopKSlices = 16;
 constexpr int kTopKBatch = 8192;
 
+template <int NV>
 __global__ void __launch_bounds__(256)
-topk_fallback_scan_kernel(const float* __restrict__ q, const float* __restrict__ db, long long n_db, int k, long long batch0,
+topk_fallback_scan_kernel(const float* __restrict__ q, const float* __restrict__ db, long long n_db, int dim, int k, long long batch0,
                           const int* __restrict__ flagged_rows, const float* __restrict__ flagged_tau,
                           const unsigned long long* __restrict__ flags, float* __restrict__ part_s, int* __restrict__ part_i) {
   __shared__ float ms[8 * 32];
@@ -236,16 +250,14 @@ topk_fallback_scan_kernel(const float* __restrict__ q, const float* __restrict__
   for (long long f = batch0 + blockIdx.y; f < nf && f < batch0 + kTopKBatch; f += gridDim.y) {
     const int row = flagged_rows[f];
     const float tau = flagged_tau[f];
-    float qv[8];
-    const float4* r = reinterpret_cast<const float4*>(q + (size_t)row * 256) + lane * 2;
-    const float4 a = r[0], b = r[1];
-    qv[0] = a.x; qv[1] = a.y; qv[2] = a.z; qv[3] = a.w; qv[4] = b.x; qv[5] = b.y; qv[6] = b.z; qv[7] = b.w;
+    float qv[4 * NV];
+    warp_row_load<NV>(qv, q + (size_t)row * dim, dim, lane);
     float ls = -INFINITY;       // this lane's entry of the warp's sorted list (lane 0 = best)
     int li = 0x7fffffff;
     float ws = -INFINITY;       // entry k-1 (the admission threshold), known to every lane
     int wi = 0x7fffffff;
     for (long long j = (long long)slice * 8 + warp; j < n_db; j += kTopKSlices * 8) {
-      const float sc = warp_dot256(qv, db, j, lane);
+      const float sc = warp_dot<NV>(qv, db, j, dim, lane);
       if (sc >= tau && topk_better(sc, (int)j, ws, wi)) {   // warp-uniform
         const int pos = __popc(__ballot_sync(0xffffffffu, topk_better(ls, li, sc, (int)j)));
         const float us = __shfl_up_sync(0xffffffffu, ls, 1);
@@ -315,7 +327,7 @@ struct TopKWs {
   int n_segments;
   long long rows_padded;
 };
-inline TopKWs topk_ws_layout(int64_t n_q, int64_t n_db) {
+inline TopKWs topk_ws_layout(int64_t n_q, int64_t n_db, int dim) {
   TopKWs L{};
   size_t off = 0;
   auto take = [&](size_t bytes) {
@@ -340,8 +352,8 @@ inline TopKWs topk_ws_layout(int64_t n_q, int64_t n_db) {
   L.n_segments = seg;
   L.rows_padded = m_tiles * 128;
   const int64_t batch = std::min<int64_t>(n_q, kTopKBatch);
-  L.qbf = take((size_t)n_q * 512);
-  L.dbbf = take((size_t)n_db * 512);
+  L.qbf = take((size_t)n_q * 2 * dim);    // bf16 screen copies, 2 * dim bytes per row
+  L.dbbf = take((size_t)n_db * 2 * dim);
   L.part_s = take((size_t)L.rows_padded * seg * kTopKCand * 4);
   L.part_i = take((size_t)L.rows_padded * seg * kTopKCand * 4);
   L.flagged_rows = take((size_t)n_q * 4);
@@ -352,18 +364,18 @@ inline TopKWs topk_ws_layout(int64_t n_q, int64_t n_db) {
   L.total = off;
   return L;
 }
-inline size_t topk_workspace_bytes(int64_t n_q, int64_t n_db, int k) {
+inline size_t topk_workspace_bytes(int64_t n_q, int64_t n_db, int k, int dim) {
   (void)k;
   if (n_q <= 0 || n_db <= 0) return 0;
-  return topk_ws_layout(n_q, n_db).total;
+  return topk_ws_layout(n_q, n_db, dim).total;
 }
 
-inline int topk_run(const float* q, const float* db, int64_t n_q, int64_t n_db, int k, float margin, float* out_s,
-                    int64_t* out_idx, unsigned long long* flags_out, uint8_t* ws, cudaStream_t st, std::string* err) {
-  const TopKWs L = topk_ws_layout(n_q, n_db);
-  const bool self = (q == db && n_q == n_db);
-  __nv_bfloat16* qbf = reinterpret_cast<__nv_bfloat16*>(ws + L.qbf);
-  __nv_bfloat16* dbbf = self ? qbf : reinterpret_cast<__nv_bfloat16*>(ws + L.dbbf);
+// Exact stages after the screen: merge + re-score, then the fallback scan of the flagged rows, kTopKBatch at a time. The
+// number of flagged rows is only known on the device, so every possible batch is launched and the blocks of a batch past the
+// count exit at once (no host synchronisation; a batch with nothing to do costs two empty launches).
+template <int NV>
+inline void topk_exact(const float* q, const float* db, int64_t n_q, int64_t n_db, int dim, int k, float margin, const TopKWs& L,
+                       uint8_t* ws, float* out_s, int64_t* out_idx, cudaStream_t st) {
   float* part_s = reinterpret_cast<float*>(ws + L.part_s);
   int* part_i = reinterpret_cast<int*>(ws + L.part_i);
   int* flagged_rows = reinterpret_cast<int*>(ws + L.flagged_rows);
@@ -371,39 +383,56 @@ inline int topk_run(const float* q, const float* db, int64_t n_q, int64_t n_db, 
   float* fb_s = reinterpret_cast<float*>(ws + L.fb_s);
   int* fb_i = reinterpret_cast<int*>(ws + L.fb_i);
   unsigned long long* flags = reinterpret_cast<unsigned long long*>(ws + L.flags);
+  topk_merge_rescore_kernel<NV><<<(unsigned)((n_q * 32 + 255) / 256), 256, 0, st>>>(
+      q, db, n_q, n_db, dim, k, L.n_segments, part_s, part_i, margin, out_s, reinterpret_cast<long long*>(out_idx), flagged_rows,
+      flagged_tau, flags);
+  const long long batch_rows = std::min<long long>(n_q, kTopKBatch);
+  for (long long b0 = 0; b0 < n_q; b0 += kTopKBatch) {
+    topk_fill_kernel<<<device_sm_count() * 4, 256, 0, st>>>(fb_i, batch_rows * kTopKSlices * kTopKMaxK, -1, flags, b0);
+    topk_fallback_scan_kernel<NV><<<dim3(kTopKSlices, (unsigned)std::min<long long>(batch_rows, 2 * device_sm_count())), 256, 0, st>>>(
+        q, db, n_db, dim, k, b0, flagged_rows, flagged_tau, flags, fb_s, fb_i);
+    topk_fallback_rank_kernel<<<(unsigned)std::min<long long>(batch_rows, 2 * device_sm_count()), 128, 0, st>>>(
+        k, b0, flagged_rows, flags, fb_s, fb_i, out_s, reinterpret_cast<long long*>(out_idx));
+  }
+}
+
+inline int topk_run(const float* q, const float* db, int64_t n_q, int64_t n_db, int dim, int k, float margin, float* out_s,
+                    int64_t* out_idx, unsigned long long* flags_out, uint8_t* ws, cudaStream_t st, std::string* err) {
+  const TopKWs L = topk_ws_layout(n_q, n_db, dim);
+  const bool self = (q == db && n_q == n_db);
+  __nv_bfloat16* qbf = reinterpret_cast<__nv_bfloat16*>(ws + L.qbf);
+  __nv_bfloat16* dbbf = self ? qbf : reinterpret_cast<__nv_bfloat16*>(ws + L.dbbf);
+  float* part_s = reinterpret_cast<float*>(ws + L.part_s);
+  int* part_i = reinterpret_cast<int*>(ws + L.part_i);
+  unsigned long long* flags = reinterpret_cast<unsigned long long*>(ws + L.flags);
   auto ck = [&](cudaError_t e, const char* what) {
     if (e != cudaSuccess) { *err = std::string(what) + ": " + cudaGetErrorString(e); return true; }
     return false;
   };
   if (ck(cudaMemsetAsync(flags, 0, 64, st), "memset")) return 1;
-  f32_to_bf16_kernel<<<(unsigned)((n_q * 32 + 255) / 256), 256, 0, st>>>(q, qbf, n_q * 32);
-  if (!self) f32_to_bf16_kernel<<<(unsigned)((n_db * 32 + 255) / 256), 256, 0, st>>>(db, dbbf, n_db * 32);
+  const long long q8 = n_q * dim / 8, db8 = n_db * dim / 8;   // 8 elements per thread
+  f32_to_bf16_kernel<<<(unsigned)((q8 + 255) / 256), 256, 0, st>>>(q, qbf, q8);
+  if (!self) f32_to_bf16_kernel<<<(unsigned)((db8 + 255) / 256), 256, 0, st>>>(db, dbbf, db8);
+  // unpadded bf16 rows (inner extent dim, pitch 2 * dim bytes): TMA zero-fills the columns past dim in the last K block. The
+  // screen streams A and B through one ring of 3 stages of one K block each, so its shared memory does not depend on dim.
   CUtensorMap ta, tb;
-  if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, 256, 256, 128, 64) || make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, 256, 256, 256, 64)) {
+  if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, dim, dim, 128, 64) || make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, dim, dim, 256, 64)) {
     *err = "tensor map encode failed";
     return 1;
   }
-  GemmShape s = plain_shape(n_q, 0, 256, 256, 64, 1);
+  GemmShape s = plain_shape(n_q, 0, (dim + 63) / 64 * 64, 256, 64, 1);
   s.n_tiles = (int)((n_db + 255) / 256);
   s.row_resident = 1;
   s.n_segments = L.n_segments;
-  s.b_prefetch_tiles = (size_t)n_db * 512 > ((size_t)160 << 20) ? g_topk_prefetch : 0;   // database tiles from HBM: see gemm_sm100.cuh
+  s.b_prefetch_tiles = (size_t)n_db * 2 * dim > ((size_t)160 << 20) ? g_topk_prefetch : 0;   // database tiles from HBM: see gemm_sm100.cuh
   EpiTopK::Params ep{};
   ep.q_rows = n_q; ep.db_rows = n_db; ep.n_segments = L.n_segments; ep.part_s = part_s; ep.part_i = part_i;
   if (ck((launch_gemm<256, 64, 3, EpiTopK>(ta, tb, s, ep, st)), "screen launch")) return 1;
-  topk_merge_rescore_kernel<<<(unsigned)((n_q * 32 + 255) / 256), 256, 0, st>>>(q, db, n_q, n_db, k, L.n_segments, part_s, part_i, margin,
-                                                                               out_s, reinterpret_cast<long long*>(out_idx), flagged_rows,
-                                                                               flagged_tau, flags);
-  // Exact fallback for the flagged rows, kTopKBatch at a time. The number of flagged rows is only known on the device, so
-  // every possible batch is launched and the blocks of a batch past the count exit at once (no host synchronisation; a
-  // batch with nothing to do costs two empty launches).
-  const long long batch_rows = std::min<long long>(n_q, kTopKBatch);
-  for (long long b0 = 0; b0 < n_q; b0 += kTopKBatch) {
-    topk_fill_kernel<<<device_sm_count() * 4, 256, 0, st>>>(fb_i, batch_rows * kTopKSlices * kTopKMaxK, -1, flags, b0);
-    topk_fallback_scan_kernel<<<dim3(kTopKSlices, (unsigned)std::min<long long>(batch_rows, 2 * device_sm_count())), 256, 0, st>>>(
-        q, db, n_db, k, b0, flagged_rows, flagged_tau, flags, fb_s, fb_i);
-    topk_fallback_rank_kernel<<<(unsigned)std::min<long long>(batch_rows, 2 * device_sm_count()), 128, 0, st>>>(
-        k, b0, flagged_rows, flags, fb_s, fb_i, out_s, reinterpret_cast<long long*>(out_idx));
+  switch ((dim + 127) / 128) {
+    case 1: topk_exact<1>(q, db, n_q, n_db, dim, k, margin, L, ws, out_s, out_idx, st); break;
+    case 2: topk_exact<2>(q, db, n_q, n_db, dim, k, margin, L, ws, out_s, out_idx, st); break;
+    case 3: topk_exact<3>(q, db, n_q, n_db, dim, k, margin, L, ws, out_s, out_idx, st); break;
+    case 4: topk_exact<4>(q, db, n_q, n_db, dim, k, margin, L, ws, out_s, out_idx, st); break;
   }
   if (ck(cudaMemcpyAsync(flags_out, flags, 16, cudaMemcpyDeviceToDevice, st), "copy flags") || ck(cudaGetLastError(), "top-k kernels")) return 1;
   return 0;

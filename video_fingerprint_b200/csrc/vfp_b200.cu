@@ -1065,6 +1065,20 @@ size_t frame_bytes_of(int frame_dtype) {
   return (size_t)12288 * (frame_dtype == VFP_FRAME_BF16 ? 2 : frame_dtype == VFP_FRAME_F32 ? 4 : 1);
 }
 
+// Embedding widths the search accepts: the rule of vfp_pair_stats (every fp32 row is 16-byte aligned for float4 loads and
+// every bf16 screen row is a whole number of 32-byte sectors). The screen runs ceil(dim / 64) K blocks of 64 columns.
+bool search_dim_ok(int dim) { return dim >= 16 && dim <= 512 && dim % 16 == 0; }
+
+// Stages of the CTA-pair join kernel's database ring: 8 up to KB = 6; above that the resident query rows (16 KB per K block)
+// leave room for 14 - KB stages of 16 KB within the 227 KB a block may have.
+template <int KB>
+cudaError_t launch_join_ares(bool pairs, const CUtensorMap& ta, const CUtensorMap& tb, const AresShape& s,
+                             const EpiJoinThreshold::Params& ep, cudaStream_t st) {
+  if (pairs) return launch_gemm_ares2<(KB <= 6 ? 8 : 14 - KB), KB, EpiJoinThreshold>(ta, tb, s, ep, st);
+  if constexpr (KB <= 4) return launch_gemm_ares<5, KB, EpiJoinThreshold>(ta, tb, s, ep, st);
+  return cudaErrorInvalidValue;   // 32 KB of resident query rows per K block: KB > 4 takes the streamed kernel
+}
+
 }  // namespace
 
 extern "C" {
@@ -1117,27 +1131,34 @@ int vfp_forward_clips(const vfp_weights* w, const void* const* clip_frames_host,
 // ---------------------------------------------------------------------------------------------
 // similarity join
 // ---------------------------------------------------------------------------------------------
-size_t vfp_join_workspace_bytes(int64_t n_q, int64_t n_db, int64_t candidate_capacity) {
-  if (n_q <= 0 || n_db <= 0) return 0;
+size_t vfp_join_workspace_bytes_dim(int64_t n_q, int64_t n_db, int64_t candidate_capacity, int dim) {
+  if (n_q <= 0 || n_db <= 0 || !search_dim_ok(dim)) return 0;
   if (candidate_capacity < 1024) candidate_capacity = 1024;
-  return align_up((size_t)n_q * 512, 1024) + align_up((size_t)n_db * 512, 1024) +
+  return align_up((size_t)n_q * 2 * dim, 1024) + align_up((size_t)n_db * 2 * dim, 1024) +
          3 * align_up((size_t)candidate_capacity * 4, 1024) + 1024;
+}
+size_t vfp_join_workspace_bytes(int64_t n_q, int64_t n_db, int64_t candidate_capacity) {
+  return vfp_join_workspace_bytes_dim(n_q, n_db, candidate_capacity, 256);
 }
 
 int vfp_join_threshold(const float* q, const float* db, int64_t n_q, int64_t n_db, int dim, int64_t q_row0, float thr,
                        float screen_margin, int32_t* out_i, int32_t* out_j, float* out_s, int64_t capacity,
                        uint64_t* counts_out, void* workspace, size_t workspace_bytes, void* stream) {
   if (!q || !db || !out_i || !out_j || !out_s || !counts_out || !workspace) return fail("vfp_join_threshold: null argument");
-  if (dim != 256) return fail("vfp_join_threshold: dim must be 256");
+  if (!search_dim_ok(dim))
+    return fail("vfp_join_threshold: dim " + std::to_string(dim) + " is not supported (16 <= dim <= 512, dim % 16 == 0)");
   if (n_q <= 0 || n_db <= 0) return fail("vfp_join_threshold: empty operand");
   if (n_q > 0x7fffff00LL || n_db > 0x7fffff00LL || q_row0 + n_q > 0x7fffff00LL) return fail("vfp_join_threshold: more than 2^31 rows");
   if (!(screen_margin >= 0.0f)) return fail("vfp_join_threshold: screen_margin must be >= 0");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   const bool self_join = (q == db && n_q == n_db);
-  const size_t q_bytes = align_up((size_t)n_q * 512, 1024), db_bytes = align_up((size_t)n_db * 512, 1024);
+  const int kb = (dim + 63) / 64;
+  const size_t row_bytes = (size_t)2 * dim;   // one bf16 screen row
+  const size_t q_bytes = align_up((size_t)n_q * row_bytes, 1024), db_bytes = align_up((size_t)n_db * row_bytes, 1024);
   const size_t fixed = q_bytes + db_bytes + 1024;
-  if (workspace_bytes < fixed + 3 * 4096) return fail("vfp_join_threshold: workspace too small; see vfp_join_workspace_bytes");
+  if (workspace_bytes < fixed + 3 * 4096)
+    return fail("vfp_join_threshold: workspace too small for dim " + std::to_string(dim) + "; see vfp_join_workspace_bytes_dim");
   const int64_t cand_cap = (int64_t)((workspace_bytes - fixed) / 3 / 1024 * 1024 / 4);
   __nv_bfloat16* qbf = reinterpret_cast<__nv_bfloat16*>(ws);
   __nv_bfloat16* dbbf = self_join ? qbf : reinterpret_cast<__nv_bfloat16*>(ws + q_bytes);
@@ -1149,18 +1170,21 @@ int vfp_join_threshold(const float* q, const float* db, int64_t n_q, int64_t n_d
 
   VFP_CUDA(cudaMemsetAsync(cand_count, 0, 8, st));
   VFP_CUDA(cudaMemsetAsync(counts, 0, 16, st));
-  f32_to_bf16_kernel<<<(unsigned)((n_q * 32 + 255) / 256), 256, 0, st>>>(q, qbf, n_q * 32);
-  if (!self_join) f32_to_bf16_kernel<<<(unsigned)((n_db * 32 + 255) / 256), 256, 0, st>>>(db, dbbf, n_db * 32);
+  const long long q8 = n_q * dim / 8, db8 = n_db * dim / 8;   // 8 elements per thread
+  f32_to_bf16_kernel<<<(unsigned)((q8 + 255) / 256), 256, 0, st>>>(q, qbf, q8);
+  if (!self_join) f32_to_bf16_kernel<<<(unsigned)((db8 + 255) / 256), 256, 0, st>>>(db, dbbf, db8);
   // a self join's score matrix is symmetric: screen the upper triangle only, the re-score kernel emits both orders
   const int tri = (self_join && g_join_symmetric) ? 1 : 0;
   EpiJoinThreshold::Params ep{};
   ep.thr = thr - screen_margin;
   ep.q_rows = n_q; ep.db_rows = n_db; ep.q_row0 = q_row0;
   ep.out_i = cand_i; ep.out_j = cand_j; ep.out_s = cand_s; ep.count = cand_count; ep.capacity = cand_cap;
+  // The screen operands are the unpadded bf16 rows: the tensor maps have an inner extent of dim columns and a 2 * dim-byte
+  // pitch, and TMA zero-fills the columns past dim in the last 64-column K block.
   CUtensorMap ta, tb;
-  if (g_join_kernel >= 1) {   // A-resident, panel-major schedule (gemm_sm100.cuh); 2 = CTA pairs (cta_group::2 UMMAs)
-    if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, 256, 256, 128, 64) ||
-        make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, 256, 256, 128, 64))
+  if (g_join_kernel == 2 || (g_join_kernel == 1 && kb <= 4)) {   // A-resident, panel-major schedule (gemm_sm100.cuh); 2 = CTA pairs (cta_group::2 UMMAs)
+    if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, dim, dim, 128, 64) ||
+        make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, dim, dim, 128, 64))
       return fail("vfp_join_threshold: tensor map encode failed");
     const bool pairs = g_join_kernel == 2;
     AresShape s{};
@@ -1177,17 +1201,27 @@ int vfp_join_threshold(const float* q, const float* db, int64_t n_q, int64_t n_d
     s.tri = tri;
     s.q_row0 = 0;   // tri compares LOCAL row and column indices: q and db are the same matrix
     ep.tri = tri;
-    if (pairs) VFP_CUDA((launch_gemm_ares2<8, EpiJoinThreshold>(ta, tb, s, ep, st)));
-    else VFP_CUDA((launch_gemm_ares<5, EpiJoinThreshold>(ta, tb, s, ep, st)));
+    cudaError_t e = cudaErrorInvalidValue;
+    switch (kb) {
+      case 1: e = launch_join_ares<1>(pairs, ta, tb, s, ep, st); break;
+      case 2: e = launch_join_ares<2>(pairs, ta, tb, s, ep, st); break;
+      case 3: e = launch_join_ares<3>(pairs, ta, tb, s, ep, st); break;
+      case 4: e = launch_join_ares<4>(pairs, ta, tb, s, ep, st); break;
+      case 5: e = launch_join_ares<5>(pairs, ta, tb, s, ep, st); break;
+      case 6: e = launch_join_ares<6>(pairs, ta, tb, s, ep, st); break;
+      case 7: e = launch_join_ares<7>(pairs, ta, tb, s, ep, st); break;
+      case 8: e = launch_join_ares<8>(pairs, ta, tb, s, ep, st); break;
+    }
+    VFP_CUDA(e);
   } else {
-    if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, 256, 256, 128, 64) ||
-        make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, 256, 256, 256, 64))
+    if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, dim, dim, 128, 64) ||
+        make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, dim, dim, 256, 64))
       return fail("vfp_join_threshold: tensor map encode failed");
-    GemmShape s = plain_shape(n_q, 0, 256, 256, 64, 32);
+    GemmShape s = plain_shape(n_q, 0, kb * 64, 256, 64, 32);
     s.n_tiles = (int)((n_db + 255) / 256);
     // L2 prefetch of the database tiles: +22 % at 2 M rows, +14 % at 1 M, but -7 % while the bf16 database (512 B per row)
     // still fits the 126 MB L2 (262 144 rows), where it is only extra traffic
-    s.b_prefetch_tiles = (size_t)n_db * 512 > ((size_t)160 << 20) ? g_join_prefetch : 0;
+    s.b_prefetch_tiles = (size_t)n_db * row_bytes > ((size_t)160 << 20) ? g_join_prefetch : 0;
     ep.tri = tri;   // this kernel visits every tile; the epilogue still drops what lies below the diagonal
     VFP_CUDA((launch_gemm<256, 64, 4, EpiJoinThreshold>(ta, tb, s, ep, st)));
   }
@@ -1202,20 +1236,25 @@ int vfp_join_threshold(const float* q, const float* db, int64_t n_q, int64_t n_d
 // ---------------------------------------------------------------------------------------------
 // flat inner-product top-k
 // ---------------------------------------------------------------------------------------------
-size_t vfp_topk_workspace_bytes(int64_t n_q, int64_t n_db, int k) { return topk_workspace_bytes(n_q, n_db, k); }
+size_t vfp_topk_workspace_bytes_dim(int64_t n_q, int64_t n_db, int k, int dim) {
+  return search_dim_ok(dim) ? topk_workspace_bytes(n_q, n_db, k, dim) : 0;
+}
+size_t vfp_topk_workspace_bytes(int64_t n_q, int64_t n_db, int k) { return topk_workspace_bytes(n_q, n_db, k, 256); }
 
 int vfp_topk_ip(const float* q, const float* db, int64_t n_q, int64_t n_db, int dim, int k, float screen_margin,
                 float* out_s, int64_t* out_idx, uint64_t* flags_out, void* workspace, size_t workspace_bytes,
                 void* stream) {
   if (!q || !db || !out_s || !out_idx || !flags_out || !workspace) return fail("vfp_topk_ip: null argument");
-  if (dim != 256) return fail("vfp_topk_ip: dim must be 256");
+  if (!search_dim_ok(dim))
+    return fail("vfp_topk_ip: dim " + std::to_string(dim) + " is not supported (16 <= dim <= 512, dim % 16 == 0)");
   if (k <= 0 || k > 32) return fail("vfp_topk_ip: k must be in [1, 32]");
   if (n_q <= 0 || n_db <= 0) return fail("vfp_topk_ip: empty operand");
   if (n_db < k) return fail("vfp_topk_ip: k exceeds the number of database rows");
   if (n_q > 0x7fffff00LL || n_db > 0x7fffff00LL) return fail("vfp_topk_ip: more than 2^31 rows");
-  if (workspace_bytes < topk_workspace_bytes(n_q, n_db, k)) return fail("vfp_topk_ip: workspace too small; see vfp_topk_workspace_bytes");
+  if (workspace_bytes < topk_workspace_bytes(n_q, n_db, k, dim))
+    return fail("vfp_topk_ip: workspace too small for dim " + std::to_string(dim) + "; see vfp_topk_workspace_bytes_dim");
   std::string err;
-  const int rc = topk_run(q, db, n_q, n_db, k, screen_margin, out_s, out_idx, reinterpret_cast<unsigned long long*>(flags_out),
+  const int rc = topk_run(q, db, n_q, n_db, dim, k, screen_margin, out_s, out_idx, reinterpret_cast<unsigned long long*>(flags_out),
                           static_cast<uint8_t*>(workspace), static_cast<cudaStream_t>(stream), &err);
   if (rc) return fail("vfp_topk_ip: " + err);
   return 0;

@@ -26,7 +26,7 @@ import torch
 from . import _native
 from .model import create_model
 
-EMBED_DIM = 256
+MAX_SEARCH_DIM = 512
 _BF16_DOT_BOUND = 2.0 ** -8  # |<q,d> - <bf16(q),bf16(d)>| <= 2^-8 |q||d| (two roundings of 2^-9 each, Cauchy-Schwarz)
 
 
@@ -42,6 +42,31 @@ def _as_device_f32(x, device=None) -> torch.Tensor:
     return x.float().contiguous()
 
 
+def _search_operands(db, q=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Device fp32 operands of the join and the top-k search: `db` (n_db, dim) and `q` (n_q, dim), `q` is `db` when None.
+    Raises ValueError, before anything is copied or launched, unless both are 2-D with the same width of 1 to 512 columns.
+    The library takes widths that are multiples of 16; any other width is zero-padded to the next one in the device copy.
+    Every added product is +0, so scores are those of the unpadded rows up to summation order, and so is the screen bound
+    (padding changes no norm)."""
+    shapes = [("db", tuple(db.shape))] + ([] if q is None else [("q", tuple(q.shape))])
+    for name, shape in shapes:
+        if len(shape) != 2:
+            raise ValueError(f"{name} must be a 2-D (rows, dim) array, got shape {shape}")
+    dim = shapes[0][1][1]
+    if q is not None and shapes[1][1][1] != dim:
+        raise ValueError(f"q and db must have the same width, got {shapes[1][1][1]} and {dim}")
+    if not 1 <= dim <= MAX_SEARCH_DIM:
+        raise ValueError(f"embedding width {dim} is not supported (1 to {MAX_SEARCH_DIM} columns)")
+    db = _as_device_f32(db)
+    q = db if q is None else _as_device_f32(q, db.device)
+    pad = -dim % 16
+    if pad:
+        self_search = q is db
+        db = torch.nn.functional.pad(db, (0, pad))
+        q = db if self_search else torch.nn.functional.pad(q, (0, pad))
+    return db, q
+
+
 def screen_margin(q: torch.Tensor, db: torch.Tensor) -> float:
     """Bound on the bf16 tensor-core screen error for these operands (see include/vfp_b200.h)."""
     nq = float(torch.linalg.vector_norm(q, dim=1).max())
@@ -55,15 +80,14 @@ _MAX_CANDIDATES = 1 << 26  # screen candidates buffered per native call (12 byte
 def threshold_join_device(
     db: torch.Tensor, thr: float, q: Optional[torch.Tensor] = None, q_row0: int = 0, capacity: Optional[int] = None
 ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """All (i, j, s) with <q_i, db_j> >= thr (fp32), as device tensors in no particular order.
+    """All (i, j, s) with <q_i, db_j> >= thr (fp32), as device tensors in no particular order. `db` is (n_db, dim) and `q`
+    (n_q, dim), `q` = `db` when None, for any width dim of 1 to 512 (see `_search_operands`).
     i is offset by q_row0 (global row index of a row-block shard). Retries with a larger buffer on overflow; when a
     low threshold or a heavily duplicated corpus produces more candidates than `_MAX_CANDIDATES`, the query rows are
     split into blocks (the reference degrades the same way, one row at a time, fingerprint.py:497-499)."""
+    db, q = _search_operands(db, q)
     lib = _native.load()
-    db = _as_device_f32(db)
-    q = db if q is None else _as_device_f32(q, db.device)
-    if db.dim() != 2 or db.shape[1] != EMBED_DIM or q.shape[1] != EMBED_DIM:
-        raise ValueError("embeddings must be (n, 256)")
+    dim = db.shape[1]
     margin = screen_margin(q, db)
     dev = db.device
 
@@ -73,13 +97,13 @@ def threshold_join_device(
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
             while True:
-                ws = torch.empty(lib.vfp_join_workspace_bytes(n_q, n_db, cand_cap), dtype=torch.uint8, device=dev)
+                ws = torch.empty(lib.vfp_join_workspace_bytes_dim(n_q, n_db, cand_cap, dim), dtype=torch.uint8, device=dev)
                 out_i = torch.empty(cap, dtype=torch.int32, device=dev)
                 out_j = torch.empty(cap, dtype=torch.int32, device=dev)
                 out_s = torch.empty(cap, dtype=torch.float32, device=dev)
                 counts = torch.zeros(2, dtype=torch.int64, device=dev)
                 rc = lib.vfp_join_threshold(
-                    C.c_void_p(qb.data_ptr()), C.c_void_p(db.data_ptr()), n_q, n_db, EMBED_DIM, int(row0), float(thr), float(margin),
+                    C.c_void_p(qb.data_ptr()), C.c_void_p(db.data_ptr()), n_q, n_db, dim, int(row0), float(thr), float(margin),
                     C.c_void_p(out_i.data_ptr()), C.c_void_p(out_j.data_ptr()), C.c_void_p(out_s.data_ptr()), cap,
                     C.c_void_p(counts.data_ptr()), C.c_void_p(ws.data_ptr()), ws.numel(), C.c_void_p(stream),
                 )
@@ -124,8 +148,8 @@ def duplicate_pairs(db, thr: float) -> Tuple[np.ndarray, np.ndarray, np.ndarray]
     with at least two hits. A row whose only hit is itself can neither seed a group (`len(similar) > 1`, :502) nor be marked
     by one, and at a million videos such rows are all but a few percent of the pair list - so they are dropped and the rest
     is ordered on the device (one bincount and one sort over the pair list) instead of on the host: 1 M embeddings, 1.08 M
-    pairs: D2H + lexsort + grouping 300 ms -> a few ms next to the 175 ms join."""
-    db = _as_device_f32(db)
+    pairs: D2H + lexsort + grouping 300 ms -> a few ms next to the 175 ms join. `db` is (n, dim), 1 <= dim <= 512."""
+    db, _ = _search_operands(db)
     n = db.shape[0]
     i, j, s = threshold_join_device(db, thr)
     i64 = i.to(torch.int64)
@@ -137,25 +161,25 @@ def duplicate_pairs(db, thr: float) -> Tuple[np.ndarray, np.ndarray, np.ndarray]
 
 
 def topk_inner_product(q, db, k: int) -> Tuple[np.ndarray, np.ndarray]:
-    """Exact flat-IP top-k: (scores (n_q,k) fp32 descending, indices (n_q,k) int64, ties by ascending index)."""
+    """Exact flat-IP top-k: (scores (n_q,k) fp32 descending, indices (n_q,k) int64, ties by ascending index). `q` (n_q, dim)
+    and `db` (n_db, dim) for any width dim of 1 to 512."""
     S, I = topk_inner_product_device(q, db, k)
     return S.cpu().numpy(), I.cpu().numpy()
 
 
 def topk_inner_product_device(q, db, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    db, q = _search_operands(db, q)
     lib = _native.load()
-    db = _as_device_f32(db)
-    q = db if q is None else _as_device_f32(q, db.device)
-    n_q, n_db = q.shape[0], db.shape[0]
+    n_q, n_db, dim = q.shape[0], db.shape[0], db.shape[1]
     k = min(int(k), n_db)
     dev = db.device
     with torch.cuda.device(dev):
-        ws = torch.empty(lib.vfp_topk_workspace_bytes(n_q, n_db, k), dtype=torch.uint8, device=dev)
+        ws = torch.empty(lib.vfp_topk_workspace_bytes_dim(n_q, n_db, k, dim), dtype=torch.uint8, device=dev)
         S = torch.empty((n_q, k), dtype=torch.float32, device=dev)
         I = torch.empty((n_q, k), dtype=torch.int64, device=dev)
         flags = torch.zeros(2, dtype=torch.int64, device=dev)
         rc = lib.vfp_topk_ip(
-            C.c_void_p(q.data_ptr()), C.c_void_p(db.data_ptr()), n_q, n_db, EMBED_DIM, k, float(screen_margin(q, db)),
+            C.c_void_p(q.data_ptr()), C.c_void_p(db.data_ptr()), n_q, n_db, dim, k, float(screen_margin(q, db)),
             C.c_void_p(S.data_ptr()), C.c_void_p(I.data_ptr()), C.c_void_p(flags.data_ptr()), C.c_void_p(ws.data_ptr()),
             ws.numel(), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream),
         )

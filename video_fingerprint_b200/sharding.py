@@ -4,7 +4,7 @@ follows (SURVEY.md section 8e):
 
 * forward: clips are independent units -> length-balanced (LPT) partition over ranks, weights replicated,
   NO collective while fingerprinting;
-* join: ONE all-gather of the (n_r, 256) fp32 embedding shards, started first and overlapped with the join of the
+* join: ONE all-gather of the (n_r, dim) fp32 embedding shards, started first and overlapped with the join of the
   rank's rows against its OWN columns; the other column ranges follow once the gather has landed (`q_row0` and a column
   offset make the pair indices global);
 * top-k: queries are sharded the same way, the database is the all-gathered matrix -> no merge step;
@@ -150,7 +150,7 @@ class _RowGather:
 def sharded_threshold_join_device(
     local_embeddings: torch.Tensor, thr: float, group=None, join_fn: Optional[Callable] = None
 ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, int]:
-    """Row-block sharded all-pairs join, device part. `local_embeddings` is this rank's (n_r, 256) shard, shards being
+    """Row-block sharded all-pairs join, device part. `local_embeddings` is this rank's (n_r, dim) shard, shards being
     consecutive in rank order. The all-gather of the shards is started first and runs (NCCL, NVLink) WHILE the rank joins
     its rows against its own columns - the one block that needs no remote data; the two remaining column ranges follow
     when the gather has landed. The score matrix is symmetric, so every block of it is computed by ONE rank, which also
