@@ -7,7 +7,7 @@ tests/golden/make_golden_3d.py produces by running the UNMODIFIED reference modu
 """
 from __future__ import annotations
 
-from typing import Dict, List
+from typing import Dict, List, Optional
 
 import torch
 import torch.nn.functional as F
@@ -40,9 +40,13 @@ def make_state_dict_3d(seed: int, frame_stride: int = 16, embedding_dim: int = 2
     return sd
 
 
-def forward3d_oracle(sd: Dict[str, torch.Tensor], video: torch.Tensor, frame_stride: int) -> torch.Tensor:
-    """model.py:468-509 in eval mode. video: (B, T, 3, H, W) or (B, 3, T, H, W) fp32 in [0, 1]."""
-    x = video.float()
+def forward3d_oracle(sd: Dict[str, torch.Tensor], video: torch.Tensor, frame_stride: int, stages: Optional[dict] = None,
+                     dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    """model.py:468-509 in eval mode. video: (B, T, 3, H, W) or (B, 3, T, H, W) in [0, 1]. `dtype`: the precision of the
+    weights, frames and arithmetic (float64 for the high-precision reference). `stages` receives the projector's ReLU hidden
+    `head_h` and its pre-normalisation output `head_e`."""
+    sd = {k: (v.to(dtype) if v.is_floating_point() else v) for k, v in sd.items()}
+    x = video.to(dtype)
     if x.dim() == 5 and x.shape[2] == 3:
         x = x.permute(0, 2, 1, 3, 4)
     T = x.shape[2]
@@ -62,6 +66,8 @@ def forward3d_oracle(sd: Dict[str, torch.Tensor], video: torch.Tensor, frame_str
     combined = (tf * attn).sum(dim=2) + tf.mean(dim=2)
     h = F.relu(F.linear(combined, sd["projector.0.weight"], sd["projector.0.bias"]))   # Dropout inactive in eval
     e = F.linear(h, sd["projector.3.weight"], sd["projector.3.bias"])
+    if stages is not None:
+        stages["head_h"], stages["head_e"] = h, e
     return F.normalize(e, p=2, dim=1)
 
 

@@ -115,18 +115,24 @@ def adaptive_pooling(sd, x: torch.Tensor) -> torch.Tensor:
     return torch.cat([avg, mx, weighted], dim=1)
 
 
-def project_and_normalise(sd, pooled: torch.Tensor) -> torch.Tensor:
-    """(B,3C) -> unit-norm (B,D).  model.py:219-224, 292-294."""
+def project_and_normalise(sd, pooled: torch.Tensor, stages: Optional[dict] = None) -> torch.Tensor:
+    """(B,3C) -> unit-norm (B,D).  model.py:219-224, 292-294. Records the ReLU hidden `head_h` and the pre-normalisation
+    output `head_e` in `stages`."""
     h = F.relu(F.linear(pooled, sd["final_projection.0.weight"], sd["final_projection.0.bias"]))
     e = F.linear(h, sd["final_projection.3.weight"], sd["final_projection.3.bias"])
+    if stages is not None:
+        stages["head_h"], stages["head_e"] = h, e
     return e / e.norm(dim=1, keepdim=True).clamp_min(1e-12)
 
 
 @torch.no_grad()
-def forward_oracle(sd: Dict[str, torch.Tensor], video: torch.Tensor, stages: Optional[dict] = None) -> torch.Tensor:
-    """Reference forward on a dense batch (B,T,3,64,64) (or (B,3,T,H,W), see model.py:283)."""
-    sd = {k: (v.float() if v.is_floating_point() else v) for k, v in sd.items()}
-    video = video.float()
+def forward_oracle(sd: Dict[str, torch.Tensor], video: torch.Tensor, stages: Optional[dict] = None,
+                   dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    """Reference forward on a dense batch (B,T,3,64,64) (or (B,3,T,H,W), see model.py:283). `dtype`: the precision of every
+    weight, frame, the checkpoint's positional table and all arithmetic (fp32 is the reference's own; float64 gives the
+    high-precision reference the kernels are measured against)."""
+    sd = {k: (v.to(dtype) if v.is_floating_point() else v) for k, v in sd.items()}
+    video = video.to(dtype)
     if video.dim() == 5 and video.shape[1] == 3:  # the reference's layout sniff, quirk included
         video = video.permute(0, 2, 1, 3, 4)
     B, T = video.shape[:2]
@@ -148,7 +154,7 @@ def forward_oracle(sd: Dict[str, torch.Tensor], video: torch.Tensor, stages: Opt
     pooled = adaptive_pooling(sd, x)
     if stages is not None:
         stages["pooled"] = pooled
-    return project_and_normalise(sd, pooled)
+    return project_and_normalise(sd, pooled, stages)
 
 
 def subsample_indices(total_frames: int, max_frames: int = 500) -> List[int]:

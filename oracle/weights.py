@@ -82,8 +82,10 @@ def state_spec(spatial_dim=128, temporal_dim=256, embedding_dim=256, num_attenti
     return spec
 
 
-def make_state_dict(seed: int, style: str = "default") -> Dict[str, torch.Tensor]:
+def make_state_dict(seed: int, style: str = "default", **arch) -> Dict[str, torch.Tensor]:
+    """Seeded checkpoint of `state_spec(**arch)`: `arch` may set spatial_dim, embedding_dim and num_attention_blocks."""
     assert style in ("default", "stress")
+    assert set(arch) <= {"spatial_dim", "embedding_dim", "num_attention_blocks"}, sorted(arch)
     g = torch.Generator().manual_seed(seed)
     stress = style == "stress"
     sd: Dict[str, torch.Tensor] = {}
@@ -91,7 +93,7 @@ def make_state_dict(seed: int, style: str = "default") -> Dict[str, torch.Tensor
     def uni(shape, lo, hi):
         return torch.rand(shape, generator=g) * (hi - lo) + lo
 
-    for key, shape, kind in state_spec():
+    for key, shape, kind in state_spec(**arch):
         if kind == "w":
             fan_in = 1
             for d in shape[1:]:

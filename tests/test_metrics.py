@@ -68,6 +68,41 @@ def test_device_metrics_match_reference_golden(name):
     close(metrics.compute_discrimination_metrics(E, ids), GOLD[name]["discrimination"], name)
 
 
+def grid_embeddings(seed, n_videos, clips_per_video, sigma, dim):
+    """make_metric_embeddings at `dim`, rounded to multiples of 2^-8: every product is then a multiple of 2^-16 and every
+    partial sum of a dot product of these near-unit rows stays below 2 in magnitude, so each score is exact in fp32 whatever
+    the summation order, and rank-derived values cannot depend on it."""
+    E, ids = mo.make_metric_embeddings(seed, n_videos, clips_per_video, sigma, dim=dim)
+    return np.round(E * 256) / np.float32(256), ids
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dim", [1, 3, 8, 100, 129, 500, 512])
+def test_device_metrics_any_width_match_oracle(dim):
+    """Widths that are not a multiple of 16 are zero-padded on the device; the values must be the oracle's at that width."""
+    from video_fingerprint_b200 import metrics
+
+    for seed, n_videos, cpv, sigma in (mo.METRIC_CASES["ragged"], mo.METRIC_CASES["pairs_noisy"]):
+        E, ids = grid_embeddings(seed, n_videos, cpv, sigma, dim)
+        close(metrics.compute_retrieval_metrics(E, ids), mo.retrieval_metrics(E, ids), f"dim{dim}")
+        close(metrics.compute_discrimination_metrics(torch.from_numpy(E), ids), mo.discrimination_metrics(E, ids), f"dim{dim}")
+
+
+def test_metrics_reject_malformed_input_before_the_device():
+    from video_fingerprint_b200 import metrics
+
+    E, ids = mo.make_metric_embeddings(3, 10, 2, 0.05, dim=8)
+    for fn in (metrics.compute_retrieval_metrics, metrics.compute_discrimination_metrics):
+        with pytest.raises(ValueError, match="2-D"):
+            fn(E[0], ids[:1])
+        with pytest.raises(ValueError, match="2-D"):
+            fn(E.reshape(4, 5, 8), ids[:4])
+        with pytest.raises(ValueError, match="one video id per embedding"):
+            fn(E, ids[:-1])
+        with pytest.raises(ValueError, match="one video id per embedding"):
+            fn(torch.from_numpy(E), ids.reshape(-1, 2))
+
+
 @pytest.mark.gpu
 def test_device_metrics_ties_ragged_and_degenerate():
     from video_fingerprint_b200 import metrics

@@ -49,23 +49,28 @@ def _positives(video_ids: np.ndarray) -> Tuple[np.ndarray, np.ndarray, np.ndarra
 
 
 def _device_pass(embeddings, video_ids, thresholds: Sequence[float]):
-    _native.require_cuda()
-    lib = _native.load()
     if isinstance(embeddings, torch.Tensor):
         E = embeddings.detach()
     else:
         E = torch.from_numpy(np.ascontiguousarray(embeddings, dtype=np.float32))
-    E = E.float().contiguous()
+    if E.dim() != 2:
+        raise ValueError(f"embeddings must be 2-D (n, dim), got shape {tuple(E.shape)}")
+    ids_np = np.asarray(video_ids)
+    if ids_np.ndim != 1 or len(ids_np) != E.shape[0]:
+        raise ValueError(f"one video id per embedding: {E.shape[0]} embeddings, video_ids of shape {ids_np.shape}")
+    if len(thresholds) > _MAX_THRESHOLDS:
+        raise ValueError(f"at most {_MAX_THRESHOLDS} thresholds per pass")
+    _native.require_cuda()
+    lib = _native.load()
+    E = E.float()
     if not E.is_cuda:
         E = E.cuda()
-    ids_np = np.asarray(video_ids)
+    # the pair kernels take rows of a multiple of 16 floats; zero columns add fmaf(0, 0, acc) = acc, so scores and ranks of
+    # any width 1 .. 512 are those of the unpadded rows
+    E = torch.nn.functional.pad(E, (0, -E.shape[1] % 16)).contiguous()
     _, ids_np = np.unique(ids_np, return_inverse=True)      # any hashable id -> dense int32
     ids_np = ids_np.astype(np.int32)
     n, dim = E.shape
-    if len(ids_np) != n:
-        raise ValueError("one video id per embedding")
-    if len(thresholds) > _MAX_THRESHOLDS:
-        raise ValueError(f"at most {_MAX_THRESHOLDS} thresholds per pass")
     row_ptr, pair_i, pos = _positives(ids_np)
     m = int(row_ptr[-1])
     dev = E.device
