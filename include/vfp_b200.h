@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define VFP_ABI_VERSION 6
+#define VFP_ABI_VERSION 7
 
 /* frame element types accepted by vfp_forward (planar (T,3,64,64) frames as produced by
  * _preprocess_frames, fingerprint.py:186-214; U8 values are scaled by 1/255 on the device) */
@@ -68,7 +68,7 @@ int vfp_weights_embedding_dim(const vfp_weights* w);
 
 /* Device workspace needed to push `frames_per_pass` frames (and up to `clips_per_pass` clips) through
  * the network in one pass. vfp_forward splits its input into passes that fit the workspace it is given;
- * the minimum useful value is the longest clip. About 9 KB per frame plus the frame encoder's scratch for one conv pass
+ * the minimum useful value is the longest clip. About 7.5 KB per frame plus the frame encoder's scratch for one conv pass
  * (48 KB per frame for min(frames_per_pass, 65 536) frames, + 1 GB that only fp32 frames use); the conv-pass size follows
  * vfp_set_tuning key 3, so size and call under the same setting. */
 size_t vfp_forward_workspace_bytes(int64_t frames_per_pass, int64_t clips_per_pass);
@@ -218,17 +218,11 @@ int vfp_profile_num_stages(void);
 const char* vfp_profile_stage_name(int i);
 int vfp_profile_read(double* stage_ms, int n_stages, uint64_t* launches, int reset);
 
-/* Tuning knobs for experiments (process-wide; defaults in parentheses). key 0: frames per conv1+conv2 pass of the two-kernel
- * stem (16384, >= 64); key 1: conv1+conv2 stem: 2 = fused kernel, conv1 as TS-mode tcgen05 UMMA (default for u8 / bf16 frames),
- * 0 = two kernels (always used for fp32 frames); key 2: 1 = hang diagnosis mode (see vfp_debug_hang_log), 0 = watchdog traps
- * (default); key 3: frames per conv pass (64..262144, default 65536); key 5 / key 6: L2 prefetch distance in column tiles of the
- * one-CTA join kernel / the top-k screen for databases larger than L2 (0 = off); key 7: programmatic dependent launch between
- * the forward's kernels (0); key 8: cap on the CTAs of persistent kernels (0 = one per SM); key 9: conv passes in flight on
- * separate streams (1); key 10: join kernel, 0 = one CTA per tile, 1 = A-resident, 2 = A-resident CTA pairs (2); key 11:
- * self joins compute the upper triangle and mirror the pairs (1); key 12: join panel width in column tiles (512); key 13:
- * TMA multicast of the conv3 / conv4 filter tile across a CTA pair, bit mask (0); key 14: 1 = both MLP linears in one kernel (1);
- * key 15: CTA-pair GEMM, bit 0 conv4, bit 1 QKV / out-projection (1); key 16: conv3 with its filters in tensor memory (1);
- * key 17: attention on tcgen05 (1) or the mma.sync twin kept for cross-checks (0).
+/* Tuning knobs for experiments (process-wide; defaults in parentheses). key 1: conv1+conv2 stem: 2 = fused kernel, conv1 as
+ * TS-mode tcgen05 UMMA (default for u8 / bf16 frames), 0 = two kernels (always used for fp32 frames and unaligned vfp_forward
+ * buffers); key 2: 1 = hang diagnosis mode (see vfp_debug_hang_log), 0 = watchdog traps (default); key 3: frames per conv pass
+ * (64..262144, default 65536); key 9: conv passes in flight on separate streams (1); key 17: attention on tcgen05 (1) or the
+ * mma.sync twin kept for cross-checks (0). Any other key, or a value out of range, is rejected with 1.
  * Every setting produces the same results up to fp32 summation order (scripts/dev_tuning_parity.py). */
 int vfp_set_tuning(int key, long long value);
 

@@ -1,6 +1,6 @@
 """Similarity join and top-k search across embedding widths, on one GPU.
 
-    python scripts/dev_join_widths.py                       # width sweep: join, top-k, join kernel choice above 256
+    python scripts/dev_join_widths.py                       # width sweep: join, top-k
     python scripts/dev_join_widths.py --ab OTHER_ROOT       # width 256: this tree against another checkout, alternating
     python scripts/dev_join_widths.py --dump OUT.npz        # seeded width-256 outputs (tests/golden/search_dim256.npz)
 
@@ -102,30 +102,18 @@ def time_ms(fn, reps: int) -> list:
     return out
 
 
-def join_record(vfp, dim: int, n: int, reps: int, key10=None) -> dict:
-    from video_fingerprint_b200 import _native
-
+def join_record(vfp, dim: int, n: int, reps: int) -> dict:
     X = unit_rows(n, dim, seed=dim)
-    lib = _native.load()
-    if key10 is not None:
-        lib.vfp_set_tuning(10, key10)
     res = {}
-    try:
-        ms = time_ms(lambda: res.update(out=vfp.threshold_join_device(X, 0.95)), reps)
-    finally:
-        if key10 is not None:
-            lib.vfp_set_tuning(10, 2)
+    ms = time_ms(lambda: res.update(out=vfp.threshold_join_device(X, 0.95)), reps)
     med = float(np.median(ms))
     pairs = n * n                 # every ordered pair, the count of np.dot(E, E.T)
     screened = n * (n + 1) // 2   # a self join screens the upper triangle only
     kb = -(-dim // 64)
-    rec = {"case": "join", "dim": dim, "rows": n, "thr": 0.95, "ms_median": round(med, 3), "ms": [round(x, 3) for x in ms],
-           "result_pairs": int(res["out"][0].numel()), "gpairs_per_s": round(pairs / med / 1e6, 1),
-           "executed_tflops": round(2 * screened * 64 * kb / med / 1e9, 1),
-           "algorithmic_tflops": round(2 * screened * dim / med / 1e9, 1)}
-    if key10 is not None:
-        rec["join_kernel_key10"] = key10
-    return rec
+    return {"case": "join", "dim": dim, "rows": n, "thr": 0.95, "ms_median": round(med, 3), "ms": [round(x, 3) for x in ms],
+            "result_pairs": int(res["out"][0].numel()), "gpairs_per_s": round(pairs / med / 1e6, 1),
+            "executed_tflops": round(2 * screened * 64 * kb / med / 1e9, 1),
+            "algorithmic_tflops": round(2 * screened * dim / med / 1e9, 1)}
 
 
 def topk_record(vfp, dim: int, n_db: int, n_q: int, k: int, reps: int) -> dict:
@@ -203,9 +191,6 @@ def main() -> None:
         return
     for dim in WIDTHS:
         emit(join_record(vfp, dim, args.join_rows, args.reps))
-    for dim in (256, 384, 512):   # the kernel choice above 256: CTA-pair A-resident (key 10 = 2) against streamed (0)
-        for key in (0, 2):
-            emit(join_record(vfp, dim, args.join_rows, args.reps, key10=key))
     for dim in WIDTHS:
         emit(topk_record(vfp, dim, args.topk_db, args.topk_q, 20, args.reps))
 

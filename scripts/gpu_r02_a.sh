@@ -15,12 +15,9 @@ except Exception as e:
     print("$name: no line", e)
 PY
 }
-ab old      --tuning 7=0 --pipelines 1 --frames-per-pass 1048576
-ab pdl      --tuning 7=1 --pipelines 1 --frames-per-pass 1048576
+ab old      --pipelines 1 --frames-per-pass 1048576
 ab p2_128k  --pipelines 2 --frames-per-pass 131072
 ab p2_64k   --pipelines 2 --frames-per-pass 65536
 ab p3_64k   --pipelines 3 --frames-per-pass 65536
-ab p2_half  --pipelines 2 --frames-per-pass 131072 --tuning 8=74
-ab p2_nopdl --pipelines 2 --frames-per-pass 131072 --tuning 7=0
 timeout 900 python bench.py --steps 10 --warmup 3 > $O/r02a_bench_n1.json 2> $O/r02a_bench_n1.err; echo "bench exit $?"
 tail -c 3000 $O/r02a_bench_n1.json

@@ -12,5 +12,4 @@ except Exception as e:
     print("$name: no line", e)
 PY
 }
-ab ffn1
-ab ffn0 --tuning 14=0
+ab base

@@ -1,8 +1,8 @@
 #!/bin/bash
-# L2-sized conv passes with and without programmatic dependent launch (verdict item 3)
+# L2-sized conv passes (verdict item 3)
 cd "$(dirname "$0")/.." || exit 1
 mkdir -p gpurun_out; O=gpurun_out
-echo "# bench.py --forward-only --steps 5 --warmup 3, 10 000 clips x 64 frames; key 3 = frames per conv pass, key 7 = programmatic dependent launch" > $O/r02p2_table.txt
+echo "# bench.py --forward-only --steps 5 --warmup 3, 10 000 clips x 64 frames; key 3 = frames per conv pass" > $O/r02p2_table.txt
 for t in ${VARIANTS:-"3=16384" "3=32768" "3=65536"}; do
   args=""; for kv in $t; do args="$args --tuning $kv"; done
   timeout 600 python bench.py --forward-only --steps 5 --warmup 3 $args > $O/r02p2.json 2> $O/r02p2.err; rc=$?

@@ -152,7 +152,7 @@ def abi_clips(lib, m, clips, ws_bytes, code=_native.FRAME_U8, ptrs=None, pitches
     return rc, emb.t[: n * 1024].view(torch.float32).view(n, 256).clone(), feats.t[: total * 1024].view(torch.float32).view(total, 256).clone(), (ws, emb, feats)
 
 
-def test_pass_splitting_through_the_abi(model):
+def test_conv_pass_splitting_through_the_abi(model):
     lib = _native.load()
     buf = u8_frames(21, 900)
     clips = [buf[0:300], buf[::4][:120], buf[200:201], buf[100:400], u8_frames(22, 77), buf[3::2][:250], buf[0:300]]
@@ -162,7 +162,7 @@ def test_pass_splitting_through_the_abi(model):
     try:
         for conv_pass, pipes in [(None, 1), (64, 1), (64, 2), (128, 3), (64, 4)]:
             if conv_pass is not None:
-                assert lib.vfp_set_tuning(3, conv_pass) == 0 and lib.vfp_set_tuning(0, conv_pass) == 0
+                assert lib.vfp_set_tuning(3, conv_pass) == 0
             assert lib.vfp_set_tuning(9, pipes) == 0
             # just large enough for the longest clip (a pass of max_t frames may hold min(max_t, n) clips)
             tight = lib.vfp_forward_workspace_bytes(max_t, min(max_t, n))
@@ -185,7 +185,6 @@ def test_pass_splitting_through_the_abi(model):
                 assert torch.equal(feats, feats2.t[: total * 1024].view(torch.float32).view(total, 256))
     finally:
         lib.vfp_set_tuning(3, 65536)
-        lib.vfp_set_tuning(0, 16384)
         lib.vfp_set_tuning(9, 1)
 
 

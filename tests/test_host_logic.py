@@ -89,6 +89,15 @@ def test_library_exports_every_declared_symbol():
     assert _native.load().vfp_join_workspace_bytes(1000, 1000, 4096) >= 2 * 1000 * 512
 
 
+def test_tuning_keys_of_removed_paths_are_rejected():
+    lib = _native.load()
+    # former defaults of the keys whose alternative paths are gone: the library no longer knows them
+    for key, value in {0: 16384, 5: 16, 6: 0, 7: 0, 8: 0, 10: 2, 11: 1, 12: 512, 13: 0, 14: 1, 15: 1, 16: 1}.items():
+        assert lib.vfp_set_tuning(key, value) == 1, key
+    for key, value in {1: 2, 3: 65536, 9: 1, 17: 1}.items():   # key 2 needs a device
+        assert lib.vfp_set_tuning(key, value) == 0, key
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU behaviour")
 def test_product_path_fails_loudly_without_gpu():
     m = vfp.create_model("attention").eval()

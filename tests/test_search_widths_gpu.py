@@ -68,19 +68,6 @@ def check_topk(S, I, Q, DB, k):
         assert np.all(np.abs(full[np.arange(len(r)), I[r, c]] - full[np.arange(len(r)), wI[r, c]]) < 2e-6)
 
 
-class tuning:
-    """vfp_set_tuning(key, value) for the block, the default restored afterwards."""
-
-    def __init__(self, key, value, default):
-        self.key, self.value, self.default = key, value, default
-
-    def __enter__(self):
-        assert _native.load().vfp_set_tuning(self.key, self.value) == 0
-
-    def __exit__(self, *exc):
-        _native.load().vfp_set_tuning(self.key, self.default)
-
-
 def ptr(t):
     return C.c_void_p(t.data_ptr())
 
@@ -122,18 +109,16 @@ def raw_topk(Q, DB, k, dim=None, ws_dim=None):
 
 # ---------------------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("dim", [16, 32, 64, 96, 128, 192, 240, 256, 320, 384, 448, 512])
-def test_join_parity_across_widths(dim):
+def test_pair_join_parity_across_widths(dim):
     thr = 0.9
     E = planted(1500, dim, seed=dim, thr=thr)
     Q = np.ascontiguousarray(E[700:1100])
     want_self = join_oracle.threshold_pairs(E, thr)
     wi, wj, ws = join_oracle.threshold_pairs(E, thr, Q=Q)
     want_cross = (wi + 700, wj, ws)
-    for key in (0, 1, 2):   # streamed kernel, A-resident single CTA, A-resident CTA pairs (the default)
-        with tuning(10, key, 2):
-            n = assert_pairs_match(vfp.threshold_join(E, thr), want_self, thr)
-            assert n >= 1500 + 30
-            assert_pairs_match(vfp.threshold_join(E, thr, q=Q, q_row0=700), want_cross, thr)
+    n = assert_pairs_match(vfp.threshold_join(E, thr), want_self, thr)
+    assert n >= 1500 + 30
+    assert_pairs_match(vfp.threshold_join(E, thr, q=Q, q_row0=700), want_cross, thr)
 
 
 @pytest.mark.parametrize("dim", [32, 128, 512])
@@ -180,19 +165,17 @@ def test_widths_off_the_multiple_of_16_are_zero_padded(dim):
         np.testing.assert_allclose(np.take_along_axis(full, I, axis=1), wS, atol=1e-5, rtol=0)
 
 
-def test_width_256_is_bitwise_the_earlier_build(golden_dir):
+def test_width_256_pair_join_is_bitwise_the_earlier_build(golden_dir):
     spec = importlib.util.spec_from_file_location("dev_join_widths", os.path.join(ROOT, "scripts", "dev_join_widths.py"))
     dev = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(dev)
     gold = np.load(os.path.join(golden_dir, "search_dim256.npz"))
     inputs = dev.golden_inputs()
     assert str(gold["inputs_sha256"]) == dev.inputs_sha256(inputs)
-    for key in (0, 1, 2):
-        with tuning(10, key, 2):
-            got = dev.golden_outputs(vfp, inputs)
-        for name, arr in got.items():
-            assert arr.dtype == gold[name].dtype and arr.shape == gold[name].shape, name
-            assert np.array_equal(arr.view(np.uint8), gold[name].view(np.uint8)), (key, name)
+    got = dev.golden_outputs(vfp, inputs)
+    for name, arr in got.items():
+        assert arr.dtype == gold[name].dtype and arr.shape == gold[name].shape, name
+        assert np.array_equal(arr.view(np.uint8), gold[name].view(np.uint8)), name
 
 
 @pytest.mark.parametrize("dim", [128, 512])

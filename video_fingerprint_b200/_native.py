@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, _LIB_NAME)
 LIB_PATH = os.environ.get("VFP_B200_LIB", LIB_PATH)  # development aid: load an experimental build
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 FRAME_U8, FRAME_BF16, FRAME_F32, FRAME_U8_HWC = 0, 1, 2, 3
 
 # every symbol include/vfp_b200.h declares (tests check the library exports exactly these)

@@ -59,7 +59,6 @@ __global__ void __launch_bounds__(kAtcThreads, 2) attention_tc_kernel(const __gr
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(s_full + 5);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  pdl_launch_dependents();
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&p.tmap_qkv);
     for (int i = 0; i < kAtcStages; ++i) {
@@ -81,7 +80,6 @@ __global__ void __launch_bounds__(kAtcThreads, 2) attention_tc_kernel(const __gr
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
 
   if (warp == 0) {
     // ------------------------------ TMA producer ------------------------------

@@ -1,7 +1,7 @@
 // conv3 (64 -> 128 channels, 3x3 stride 2, 16x16 -> 8x8, model.py:107-109) with the FILTERS IN TENSOR MEMORY.
 //
-// The generic kernel runs this layer with the channels on M and four frames' pixels on N (SWAP mode): every UMMA then streams
-// 4 KB of filters and 8 KB of pixels from shared memory, and every K block is refilled by TMA with 16 KB of filters + 32 KB of
+// The generic GEMM kernel ran this layer with the channels on M and four frames' pixels on N: every UMMA then streamed
+// 4 KB of filters and 8 KB of pixels from shared memory, and every K block was refilled by TMA with 16 KB of filters + 32 KB of
 // pixels: 96 B/clk of operand reads + 96 B/clk of fill against a 128 B/clk shared-memory port - the layer sat at 54 % tensor
 // utilisation (ncu) with the port as the wall (multicasting the filter tile across a CTA pair did not help: the bytes still
 // land in every CTA's shared memory). The filters are only 128 x 576 bf16 = 288 TMEM columns, so here they are written to
@@ -59,7 +59,6 @@ __global__ void __launch_bounds__(kC3Threads, 1) conv3_ts_kernel(const __grid_co
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_full + 2);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  pdl_launch_dependents();
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&p.tmap_in);
     tma_prefetch_desc(&p.tmap_out);
@@ -99,7 +98,6 @@ __global__ void __launch_bounds__(kC3Threads, 1) conv3_ts_kernel(const __grid_co
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  pdl_wait();   // the filters are static; the pixels come from the previous kernel
 
   if (warp == 0) {
     // ------------------------------ TMA producer ------------------------------

@@ -295,63 +295,6 @@ struct EpiBiasActTma : EpiDefaults {
 };
 
 // -------------------------------------------------------------------------------------------
-// Epilogue of the SWAP (channels-on-M) convolutions: the thread owns output CHANNEL `row` and receives 32 consecutive
-// PIXELS per chunk. y = relu(acc + bias[channel]) is written transposed into the [pixel][channel] staging tile
-// (64-byte rows, SWIZZLE_64B, one 2-byte store per pixel; the 32 lanes of a warp fill one 64-byte row per
-// instruction) and stored by the TMA unit as a 32-pixel x 32-channel box of the NHWC output.
-// -------------------------------------------------------------------------------------------
-struct EpiConvTransposedTma : EpiDefaults {
-  struct Params {
-    alignas(64) CUtensorMap tmap_out;  // [pixels][C_out] bf16, box 32 channels x 32 pixels, SWIZZLE_64B
-    const float* bias;                 // [C_out]
-    int c_out;                         // valid channels (<= 128)
-    int pixels_per_tile;               // MT * 128
-  };
-  static constexpr int kChunkBytes = 2048;
-  static constexpr int kBuffers = 2;
-  static constexpr int kExtraSmemBytes = 8 * kBuffers * kChunkBytes;
-  uint8_t* stage;
-  int buf;
-  float bias_row;    // the thread's accumulator row = its output channel never changes: one load for the whole kernel
-  int bias_for;
-  __device__ __forceinline__ void setup(const Params&, uint8_t* extra, int warp_slot, int) {
-    stage = extra + warp_slot * (kBuffers * kChunkBytes);
-    buf = 0;
-    bias_for = -1;
-    bias_row = 0.0f;
-  }
-  __device__ __forceinline__ void finish(const Params&, int lane) {
-    if (lane == 0) tma_store_wait_read<0>();
-  }
-  __device__ __forceinline__ void begin(const Params&, int, int, int) {}
-  __device__ __forceinline__ void end(const Params&, int, int, int) {}
-  __device__ __forceinline__ void chunk(const Params& p, int mts, int col0, int row, uint32_t (&v)[32], int) {
-    const int ch0 = row & ~31;           // first channel of this warp's lane quarter
-    if (ch0 >= p.c_out) return;          // warp-uniform: conv2 has only 64 of the 128 accumulator rows
-    const int lane = row & 31;
-    if (bias_for != row) { bias_row = __ldg(p.bias + row); bias_for = row; }
-    const float b = bias_row;
-    uint8_t* dst = stage + buf * kChunkBytes;
-    if (lane == 0) tma_store_wait_read<kBuffers - 1>();
-    __syncwarp();
-    uint8_t* col = dst + (lane & 7) * 2;
-    const int chunk = lane >> 3;
-#pragma unroll
-    for (int i = 0; i < 32; ++i) {
-      const float y = fmaxf(__uint_as_float(v[i]) + b, 0.0f);
-      *reinterpret_cast<__nv_bfloat16*>(col + i * 64 + ((chunk ^ ((i >> 1) & 3)) << 4)) = __float2bfloat16(y);
-    }
-    fence_proxy_async_smem();
-    __syncwarp();
-    if (lane == 0) {
-      tma_store_2d(&p.tmap_out, dst, ch0, mts * p.pixels_per_tile + col0);
-      tma_store_commit();
-    }
-    buf ^= 1;
-  }
-};
-
-// -------------------------------------------------------------------------------------------
 // conv4 epilogue: relu(acc + bias), then the 4x4 global average pool. A tile holds 8 frames x 16
 // pixels, so each half-warp (16 lanes) is exactly one frame; a halving butterfly leaves lane j of
 // the half-warp with the sums of columns 2j, 2j+1 of the chunk.

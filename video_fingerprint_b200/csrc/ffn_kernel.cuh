@@ -101,7 +101,6 @@ __global__ void __launch_bounds__(kFfnThreads, 1) ffn_pair_kernel(const __grid_c
   const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
   const int my_tiles = p.pair_tiles > pair ? (p.pair_tiles - pair + n_pairs - 1) / n_pairs : 0;
   const int n_chunks = my_tiles * kFfnChunks;   // global chunk sequence of this pair
-  pdl_launch_dependents();
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&p.tmap_x);
@@ -138,7 +137,6 @@ __global__ void __launch_bounds__(kFfnThreads, 1) ffn_pair_kernel(const __grid_c
   cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
 
   if (warp == 0) {
     // ------------------------------ TMA producer (both CTAs) ------------------------------

@@ -1,4 +1,4 @@
-// Host launch helpers: per-device kernel configuration, programmatic dependent launch, gemm_tcgen05_kernel grids.
+// Host launch helpers: per-device kernel configuration, kernel launches, gemm_tcgen05_kernel grids.
 #pragma once
 #include <atomic>
 #include <mutex>
@@ -32,18 +32,6 @@ inline int device_sm_count() {
   return n;
 }
 
-// Upper bound on the CTAs a persistent kernel launches (vfp_set_tuning key 8; 0 = one per SM). Two pipelines that
-// run side by side on different streams can each be given part of the GPU this way.
-inline std::atomic<int>& persistent_cta_limit() {
-  static std::atomic<int> v{0};
-  return v;
-}
-inline int persistent_grid() {
-  const int lim = persistent_cta_limit().load(std::memory_order_relaxed);
-  const int sms = device_sm_count();
-  return (lim > 0 && lim < sms) ? lim : sms;
-}
-
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-DEVICE property of a kernel, so "already configured" is
 // remembered per (kernel, device ordinal) - a process-wide flag breaks the second GPU of a process.
 inline cudaError_t ensure_dynamic_smem(const void* kernel, int bytes) {
@@ -62,18 +50,6 @@ inline cudaError_t ensure_dynamic_smem(const void* kernel, int bytes) {
   return e;
 }
 
-// Programmatic dependent launch (vfp_set_tuning key 7): every kernel of the forward chain executes
-// griddepcontrol.launch_dependents at its top and griddepcontrol.wait before it touches memory, so the next
-// kernel's CTAs are scheduled - and run their prologue (barrier init, TMEM allocation, descriptor prefetch) - while
-// the tail of the current kernel drains. Kernels launched this way MUST call pdl_wait() (sm100_primitives.cuh).
-// OFF by default: measured on B200 over 10 000 x 64-frame clips it changes nothing or costs up to 2 % (39.2-39.9 ms per
-// step with it, 38.6-38.9 without, profiles/r02_ab_schedule.txt) - the forward is 160 long launches per step, their
-// tails are not where the time goes.
-inline std::atomic<int>& pdl_enabled() {
-  static std::atomic<int> v{0};
-  return v;
-}
-
 template <class... KArgs, class... Args>
 inline cudaError_t launch_kernel_cluster(int cluster, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
                                          Args&&... args) {
@@ -82,13 +58,8 @@ inline cudaError_t launch_kernel_cluster(int cluster, void (*kernel)(KArgs...), 
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   int n = 0;
-  if (pdl_enabled().load(std::memory_order_relaxed)) {
-    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
   if (cluster > 1) {
     attr[n].id = cudaLaunchAttributeClusterDimension;
     attr[n].val.clusterDim.x = (unsigned)cluster;
@@ -105,23 +76,19 @@ inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block
   return launch_kernel_cluster(1, kernel, grid, block, smem, stream, std::forward<Args>(args)...);
 }
 
-// MCAST = 2: clusters of two CTAs share the B tile (tb must then be a tensor map with a box of BLOCK_N / 2 rows); not
-// available for the row-resident schedule.
-template <int BLOCK_N, int BLOCK_K, int STAGES, class Epi, int MT = 1, bool SWAP = false, int MCAST = 1>
+template <int BLOCK_N, int BLOCK_K, int STAGES, class Epi, int MT = 1>
 inline cudaError_t launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const GemmShape& shape,
                                const typename Epi::Params& ep, cudaStream_t stream) {
   using L = GemmSmemLayout<BLOCK_N, BLOCK_K, STAGES, MT>;
   constexpr int kSmem = L::kTotal + Epi::kExtraSmemBytes;
   static_assert(kSmem <= 232448, "shared memory budget");
-  auto kernel = gemm_tcgen05_kernel<BLOCK_N, BLOCK_K, STAGES, Epi, MT, SWAP, MCAST>;
+  auto kernel = gemm_tcgen05_kernel<BLOCK_N, BLOCK_K, STAGES, Epi, MT>;
   if (cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), kSmem); e != cudaSuccess) return e;
-  if (MCAST > 1 && (shape.row_resident || shape.b_prefetch_tiles)) return cudaErrorInvalidValue;
-  const int m_super = ((shape.m_tiles + MT - 1) / MT + MCAST - 1) / MCAST;   // (pairs of) super-tiles
+  const int m_super = (shape.m_tiles + MT - 1) / MT;   // super-tiles
   const int total = shape.row_resident ? m_super * shape.n_segments : m_super * shape.n_tiles;
   if (total <= 0) return cudaSuccess;
-  const int clusters = persistent_grid() / MCAST;
-  const int grid = (total < clusters ? total : clusters) * MCAST;
-  return launch_kernel_cluster(MCAST, kernel, dim3(grid), dim3(gemm_threads<BLOCK_N, Epi>()), kSmem, stream, ta, tb, shape, ep);
+  const int grid = total < device_sm_count() ? total : device_sm_count();
+  return launch_kernel(kernel, dim3(grid), dim3(gemm_threads<BLOCK_N, Epi>()), kSmem, stream, ta, tb, shape, ep);
 }
 
 template <int BLOCK_N, int BLOCK_K, int STAGES, int KB, class Epi>
@@ -135,22 +102,8 @@ inline cudaError_t launch_gemm_bres(const CUtensorMap& ta, const CUtensorMap& tb
   if (cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), kSmem); e != cudaSuccess) return e;
   const long long total = (long long)shape.m_tiles * shape.n_tiles;
   if (total <= 0) return cudaSuccess;
-  const int grid = total < persistent_grid() ? (int)total : persistent_grid();
+  const int grid = total < device_sm_count() ? (int)total : device_sm_count();
   return launch_kernel(kernel, dim3(grid), dim3(gemm_threads<BLOCK_N, Epi>()), kSmem, stream, ta, tb, shape, ep);
-}
-
-template <int STAGES, int KB, class Epi>
-inline cudaError_t launch_gemm_ares(const CUtensorMap& ta, const CUtensorMap& tb, const AresShape& shape,
-                                    const typename Epi::Params& ep, cudaStream_t stream) {
-  using L = AresSmemLayout<STAGES, KB>;
-  constexpr int kSmem = L::kTotal + Epi::kExtraSmemBytes;
-  static_assert(kSmem <= 232448, "shared memory budget");
-  auto kernel = gemm_ares_tcgen05_kernel<STAGES, KB, Epi>;
-  if (cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), kSmem); e != cudaSuccess) return e;
-  const long long total = (long long)shape.m_super * shape.n_panels;
-  if (total <= 0) return cudaSuccess;
-  const int grid = total < persistent_grid() ? (int)total : persistent_grid();
-  return launch_kernel(kernel, dim3(grid), dim3(gemm_threads<kAresBlockN, Epi>()), kSmem, stream, ta, tb, shape, ep);
 }
 
 template <int STAGES, int KB, class Epi>
@@ -163,7 +116,7 @@ inline cudaError_t launch_gemm_ares2(const CUtensorMap& ta, const CUtensorMap& t
   if (cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), kSmem); e != cudaSuccess) return e;
   const long long total = (long long)shape.m_super * shape.n_panels;
   if (total <= 0) return cudaSuccess;
-  const int pairs = persistent_grid() / 2;
+  const int pairs = device_sm_count() / 2;
   const int grid = 2 * (total < pairs ? (int)total : pairs);
   return launch_kernel_cluster(2, kernel, dim3(grid), dim3(gemm_threads<kAres2BlockN, Epi>()), kSmem, stream, ta, tb, shape, ep);
 }
@@ -177,10 +130,10 @@ inline cudaError_t launch_gemm_pair(const CUtensorMap& ta, const CUtensorMap& tb
   static_assert(kSmem <= 232448, "shared memory budget");
   auto kernel = gemm_pair_tcgen05_kernel<BLOCK_K, STAGES, Epi>;
   if (cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(kernel), kSmem); e != cudaSuccess) return e;
-  if (shape.row_resident || shape.b_prefetch_tiles) return cudaErrorInvalidValue;
+  if (shape.row_resident) return cudaErrorInvalidValue;
   const long long total = (long long)((shape.m_tiles + 1) / 2) * shape.n_tiles;
   if (total <= 0) return cudaSuccess;
-  const int pairs = persistent_grid() / 2;
+  const int pairs = device_sm_count() / 2;
   const int grid = 2 * (total < pairs ? (int)total : pairs);
   return launch_kernel_cluster(2, kernel, dim3(grid), dim3(gemm_threads<256, Epi>()), kSmem, stream, ta, tb, shape, ep);
 }
@@ -198,7 +151,6 @@ inline GemmShape plain_shape(long long M, int N, int K, int block_n, int block_k
   s.h_mul = 0;
   s.row_resident = 0;
   s.n_segments = 1;
-  s.b_prefetch_tiles = 0;
   return s;
 }
 
@@ -211,22 +163,6 @@ inline void conv_taps_strided(GemmShape* s, int cblocks_per_tap) {
     s->tap_w[kb] = (signed char)(kw - 1);
     s->tap_h[kb] = (signed char)(kh - 1);
   }
-}
-
-// The same convolution over a space-to-depth input [frame][H/2][W/2][(sh*2+sw)*C + c]: it becomes a 2x2 /
-// stride-1 window over cells, every tap reads ONE dense channel slice of a cell (no strided traversal).
-// tap k in {0,1,2} -> input row 2*o + k - 1 = cell (o + d), sub-row s with (d, s) = (-1,1), (0,0), (0,1).
-inline void conv_taps_space_to_depth(GemmShape* s, int cblocks_per_subpixel) {
-  s->h_mul = 1;
-  const int d[3] = {-1, 0, 0}, sub[3] = {1, 0, 1};
-  int kb = 0;
-  for (int kh = 0; kh < 3; ++kh)
-    for (int kw = 0; kw < 3; ++kw)
-      for (int cb = 0; cb < cblocks_per_subpixel; ++cb, ++kb) {
-        s->tap_c_blk[kb] = (signed char)((sub[kh] * 2 + sub[kw]) * cblocks_per_subpixel + cb);
-        s->tap_w[kb] = (signed char)d[kw];
-        s->tap_h[kb] = (signed char)d[kh];
-      }
 }
 
 }  // namespace vfp

@@ -37,7 +37,6 @@ struct GemmShape {
   // row-reducing epilogue can keep per-row state across them. Concurrent CTAs stream the same columns -> L2 reuse.
   int row_resident;
   int n_segments;
-  int b_prefetch_tiles;  // L2-prefetch the B column tile this many tiles ahead (0 = off)
   // A operand addressing
   int a_conv;           // 0: rows are GEMM rows; 1: 4-D box (C, W, H, frame) over an NHWC activation tensor
   int tiles_per_frame;  // conv: row tiles per frame (>=1) ...
@@ -116,30 +115,15 @@ struct GemmSmemLayout {
 // UMMAs that accumulate into the SAME TMEM tile issue back to back only every ~180 cycles (measured: 24 dependent
 // M128 N64 K16 instructions take 4300 cycles), which starves narrow tiles (N=64: 32 cycles of work per
 // instruction). Round-robin over MT independent accumulators hides that latency.
-//
-// SWAP: the roles of the two shared-memory tiles are exchanged in the UMMA: the B-region tile (weights, 128 rows =
-// output channels, rows past C_out zero-filled by TMA) becomes the M operand and the MT x 128 activation rows become
-// the N operand (N = 256 for MT = 2). An SS-mode UMMA costs ~128 cycles however narrow N is (the 128 x 16 A slice is
-// streamed from shared memory), so a conv with C_out = 64 / 128 as the N dimension uses only 25 % / 50 % of the
-// tensor pipe; with the channels on M and 256 pixels on N it is 50 % / 100 %. The accumulator then holds
-// [channel][pixel] and the epilogue transposes while staging for the TMA store.
-//
-// MCAST = 2: the kernel runs as clusters of two CTAs that work on neighbouring row (super-)tiles of the SAME column tile
-// in lock step. The B tile (filters / weights) of every K block is then fetched from L2 once per PAIR: each CTA loads
-// half of its rows with a multicast TMA that writes both CTAs' shared memory (tmap_b must have a box of BLOCK_N / 2 rows).
-// A stage is released by a multicast tcgen05.commit that arrives at both CTAs' empty barriers (count 2).
-template <int BLOCK_N, int BLOCK_K, int STAGES, class Epilogue, int MT = 1, bool SWAP = false, int MCAST = 1>
+template <int BLOCK_N, int BLOCK_K, int STAGES, class Epilogue, int MT = 1>
 __global__ void __launch_bounds__(gemm_threads<BLOCK_N, Epilogue>(), 1)
 gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                     const GemmShape shape_in, const __grid_constant__ typename Epilogue::Params ep) {
-  static_assert(MCAST == 1 || MCAST == 2, "cluster size");
   using L = GemmSmemLayout<BLOCK_N, BLOCK_K, STAGES, MT>;
   static_assert(BLOCK_N % 32 == 0 && BLOCK_N >= 32 && BLOCK_N <= 256, "BLOCK_N");
   static_assert(BLOCK_K == 64 || BLOCK_K == 32 || BLOCK_K == 16, "BLOCK_K");
-  static_assert(SWAP ? (BLOCK_N == 128 && MT * 128 <= 256) : (2 * MT * BLOCK_N <= 512), "TMEM: two accumulator buffers");
-  constexpr int kAccCols = SWAP ? MT * kBlockM : MT * BLOCK_N;  // columns of one accumulator buffer
-  constexpr int kEpiTiles = SWAP ? 1 : MT;                      // accumulator tiles the epilogue walks per CTA tile
-  constexpr int kEpiCols = SWAP ? MT * kBlockM : BLOCK_N;       // columns of one such tile
+  static_assert(2 * MT * BLOCK_N <= 512, "TMEM: two accumulator buffers");
+  constexpr int kAccCols = MT * BLOCK_N;  // columns of one accumulator buffer
   constexpr uint32_t kTmemCols = (2 * kAccCols <= 32) ? 32 : (2 * kAccCols <= 64) ? 64 : (2 * kAccCols <= 128) ? 128
                                  : (2 * kAccCols <= 256) ? 256 : 512;
 
@@ -156,21 +140,17 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  pdl_launch_dependents();
   // the tile walk runs over super-tiles of MT row tiles
   GemmShape shape = shape_in;
   const int m_tiles_real = shape_in.m_tiles;
-  shape.m_tiles = ((shape_in.m_tiles + MT - 1) / MT + MCAST - 1) / MCAST;   // the walk runs over (pairs of) super-tiles
-  const int crank = MCAST > 1 ? (int)cluster_ctarank() : 0;
-  const int walk_cta = blockIdx.x / MCAST, walk_n = gridDim.x / MCAST;
-  constexpr uint16_t kMcastMask = (uint16_t)((1u << MCAST) - 1u);
+  shape.m_tiles = (shape_in.m_tiles + MT - 1) / MT;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_a);
     tma_prefetch_desc(&tmap_b);
     for (int i = 0; i < STAGES; ++i) {
       mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], MCAST);
+      mbar_init(&empty_bar[i], 1);
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&acc_full[i], 1);
@@ -184,21 +164,18 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   }
   tc_fence_before();
   __syncthreads();
-  if constexpr (MCAST > 1) cluster_sync_all();   // the peer's barriers are initialised before anything is multicast at them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();   // everything above overlapped the previous kernel's tail; its results are needed from here on
 
   if (warp == 0) {
     // ------------------------------ TMA producer ------------------------------
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      TileWalk walk(shape, walk_cta, walk_n);
+      TileWalk walk(shape, blockIdx.x, gridDim.x);
       int mts, nt;
       bool first, last;
       while (walk.next(mts, nt, first, last)) {
-        mts = mts * MCAST + crank;
         int frame0[MT], oh0[MT];
 #pragma unroll
         for (int sub = 0; sub < MT; ++sub) {
@@ -214,16 +191,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
             }
           }
         }
-        // A B operand much larger than L2 (a database of >= 10^6 rows in the join) comes from HBM the first time a column
-        // tile is touched, and the ~32 CTAs that share the tile all stall on that one fetch (measured: 1 241 TFLOP/s with a
-        // 134 MB database, 852 with 512 MB). The CTA that owns the group's first row tile pulls the column tile
-        // `b_prefetch_tiles` ahead into L2 (row-resident schedule of the top-k search: every 8th row tile does, the CTAs of
-        // one column segment walk the same columns at about the same time).
-        if (shape.b_prefetch_tiles > 0 && (mts * MT) % (shape.row_resident ? 8 : shape.group_m) == 0) {
-          const int pnt = nt + shape.b_prefetch_tiles;
-          if (pnt < shape.n_tiles)
-            for (int kb = 0; kb < shape.k_blocks; ++kb) tma_prefetch_l2_2d(&tmap_b, kb * BLOCK_K, pnt * BLOCK_N);
-        }
         for (int kb = 0; kb < shape.k_blocks; ++kb) {
           mbar_wait(&empty_bar[stage], phase ^ 1);
           mbar_arrive_expect_tx(&full_bar[stage], L::kStageBytes);
@@ -237,12 +204,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
               tma_load_2d(&tmap_a, &full_bar[stage], dst, kb * BLOCK_K, (mts * MT + sub) * kBlockM);
             }
           }
-          if constexpr (MCAST > 1) {   // my half of the B rows, written into both CTAs of the pair
-            tma_load_2d_mcast(&tmap_b, &full_bar[stage], smem_b + stage * L::kBBytes + crank * (L::kBBytes / MCAST), kb * BLOCK_K,
-                              nt * BLOCK_N + crank * (BLOCK_N / MCAST), kMcastMask);
-          } else {
-            tma_load_2d(&tmap_b, &full_bar[stage], smem_b + stage * L::kBBytes, kb * BLOCK_K, nt * BLOCK_N);
-          }
+          tma_load_2d(&tmap_b, &full_bar[stage], smem_b + stage * L::kBBytes, kb * BLOCK_K, nt * BLOCK_N);
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
       }
@@ -250,11 +212,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   } else if (warp == 1) {
     // ------------------------------ UMMA issuer ------------------------------
     if (lane == 0) {
-      constexpr uint32_t idesc = SWAP ? umma_idesc_bf16(kBlockM, MT * kBlockM) : umma_idesc_bf16(kBlockM, BLOCK_N);
+      constexpr uint32_t idesc = umma_idesc_bf16(kBlockM, BLOCK_N);
       int stage = 0;
       uint32_t phase = 0;
       int local = 0;
-      TileWalk walk(shape, walk_cta, walk_n);
+      TileWalk walk(shape, blockIdx.x, gridDim.x);
       int mts, nt;
       bool first, last;
       for (; walk.next(mts, nt, first, last); ++local) {
@@ -271,18 +233,13 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
 #pragma unroll
           for (int k = 0; k < BLOCK_K / 16; ++k) {
             // advancing 16 bf16 along K = 32 bytes = 2 units of the (addr >> 4) field
-            if constexpr (SWAP) {
-              const uint64_t pxdesc = umma_smem_desc_kmajor<L::kRowBytes>(a_base);  // MT*128 activation rows = N
-              umma_bf16(d_tmem, bdesc + 2 * k, pxdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
-            } else {
 #pragma unroll
-              for (int sub = 0; sub < MT; ++sub) {
-                const uint64_t adesc = umma_smem_desc_kmajor<L::kRowBytes>(a_base + sub * L::kABytes);
-                umma_bf16(d_tmem + sub * BLOCK_N, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
-              }
+            for (int sub = 0; sub < MT; ++sub) {
+              const uint64_t adesc = umma_smem_desc_kmajor<L::kRowBytes>(a_base + sub * L::kABytes);
+              umma_bf16(d_tmem + sub * BLOCK_N, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
             }
           }
-          if constexpr (MCAST > 1) umma_commit_mcast(&empty_bar[stage], kMcastMask); else umma_commit(&empty_bar[stage]);
+          umma_commit(&empty_bar[stage]);
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
         umma_commit(&acc_full[acc]);
@@ -291,12 +248,12 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   } else {
     // ------------------------------ epilogue ------------------------------
     constexpr int kSplit = gemm_column_split<BLOCK_N, Epilogue>();
-    constexpr int kColsPerWarp = kEpiCols / kSplit;
+    constexpr int kColsPerWarp = BLOCK_N / kSplit;
     const int quarter = warp & 3;  // TMEM lane quarter this warp may touch
     const int row = quarter * 32 + lane;
     const int col_begin = ((warp - 2) >> 2) * kColsPerWarp;
     int local = 0;
-    TileWalk walk(shape, walk_cta, walk_n);
+    TileWalk walk(shape, blockIdx.x, gridDim.x);
     int mts, nt;
     bool first, last;
     Epilogue epi;
@@ -304,16 +261,15 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     epi.setup(ep, extra_smem, warp - 2, lane);
     epi.set_block_n(BLOCK_N);
     for (; walk.next(mts, nt, first, last); ++local) {
-      mts = mts * MCAST + crank;
       const int acc = local & 1;
       const uint32_t acc_phase = (local >> 1) & 1;
       if (first) epi.item_begin(ep, mts, walk.seg, row, extra_smem);
       mbar_wait(&acc_full[acc], acc_phase);
       tc_fence_after();
 #pragma unroll 1
-      for (int sub = 0; sub < kEpiTiles; ++sub) {
-        const int mt = SWAP ? mts : mts * MT + sub;  // SWAP: the epilogue sees the super-tile (MT*128 pixel columns)
-        if (!SWAP && mt >= m_tiles_real) break;      // warp-uniform
+      for (int sub = 0; sub < MT; ++sub) {
+        const int mt = mts * MT + sub;
+        if (mt >= m_tiles_real) break;  // warp-uniform
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + acc * kAccCols + sub * BLOCK_N;
         epi.begin(ep, mt, nt, row);
 #pragma unroll 1
@@ -323,7 +279,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
             uint32_t v[32];
             tmem_ld_32x32(taddr + c, v);
             tmem_ld_wait();
-            epi.chunk(ep, mt, SWAP ? c : nt * BLOCK_N + c, row, v, pass);
+            epi.chunk(ep, mt, nt * BLOCK_N + c, row, v, pass);
           }
         }
         epi.end(ep, mt, nt, row);
@@ -339,7 +295,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   __syncwarp();
   tc_fence_before();
   __syncthreads();
-  if constexpr (MCAST > 1) cluster_sync_all();   // my last multicast commits target the peer's barriers: it must still be there
   if (warp == 1) {
     tc_fence_after();
     tmem_dealloc(tmem_base, kTmemCols);
@@ -386,7 +341,6 @@ gemm_bres_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  pdl_launch_dependents();
   const long long total = (long long)shape.m_tiles * shape.n_tiles;
   const long long per = (total + gridDim.x - 1) / gridDim.x;
   const long long u0 = (long long)blockIdx.x * per;
@@ -415,7 +369,6 @@ gemm_bres_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();   // everything above overlapped the previous kernel's tail; its results are needed from here on
 
   if (warp == 0) {
     if (lane == 0) {
@@ -535,33 +488,30 @@ gemm_bres_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
 }
 
 // =================================================================================================
-// A-resident, panel-major variant for the all-pairs similarity join (vfp_join_threshold).
+// A-resident, panel-major schedule of the all-pairs similarity join (vfp_join_threshold).
 // The plain kernel above re-fetches BOTH operands for every 128 x 256 tile: 192 KB per 2 048 MMA cycles = 94 B/clk per SM,
 // above what L2 -> SM delivers, so the join ran at 0.59-0.75 of the tensor peak. Here a work item is
 //      (a super-tile of kAresMT x 128 query rows) x (one PANEL of database column tiles),
-// the query super-tile (all four K blocks, 128 KB) is loaded ONCE per item and stays in shared memory, and only the
-// database streams through the ring in 128-row x 64-column blocks: 64 KB per 2 048 MMA cycles = 32 B/clk. UMMAs are
-// M128 N128 K16 (64 cycles each, the tensor pipe's full rate), two independent accumulators per column tile (one per
-// query sub-tile), TMEM double buffered: 2 x 2 x 128 = 512 columns.
+// the query super-tile (all K blocks) is loaded ONCE per item and stays in shared memory, and only the database streams
+// through the ring in blocks of 64 columns.
 // Items are numbered PANEL-MAJOR and dealt round-robin, so at any time all CTAs work inside the same one or two panels:
 // a panel (<= 65 536 database rows = 32 MB of bf16) is read from HBM once and then served from L2 however far the CTAs
 // drift apart; a row-major order would let 148 CTAs stream 148 different parts of a database that does not fit L2.
 // `tri` (self joins): S is symmetric, so column tiles that lie entirely below the diagonal of the item's rows are
 // skipped; the epilogue keeps j >= i and the re-score kernel emits the mirrored pair.
 // =================================================================================================
-// KB (template parameter of both kernels) = resident K blocks of 64 columns, ceil(dim / 64): 4 for the 256-wide embeddings the
+// KB (template parameter of the kernel) = resident K blocks of 64 columns, ceil(dim / 64): 4 for the 256-wide embeddings the
 // models produce by default. Columns past dim in the last block are zero-filled by the TMA unit and add +0 to every score.
 constexpr int kAresMT = 2;
-constexpr int kAresBlockN = 128;
 
 struct AresShape {
   int m_super;        // super-tiles of kAresMT * 128 query rows
-  int n_tiles;        // database column tiles of 128 rows
+  int n_tiles;        // database column tiles of block_n rows
   int panel_tiles;    // column tiles per panel
   int n_panels;
   int tri;            // 1: skip column tiles strictly below the diagonal
   long long q_row0;   // global index of query row 0 (position of the diagonal)
-  int block_n;        // database rows per column tile (128: single-CTA kernel, 256: CTA-pair kernel)
+  int block_n;        // database rows per column tile (kAres2BlockN)
 };
 
 struct AresWalk {
@@ -584,181 +534,11 @@ struct AresWalk {
   }
 };
 
-template <int STAGES, int KB>
-struct AresSmemLayout {
-  static constexpr int kABytes = kBlockM * 128;                      // one K block of one 128-row sub-tile
-  static constexpr int kAResident = kAresMT * KB * kABytes;          // 32 KB per K block (128 KB at KB = 4)
-  static constexpr int kBBytes = kAresBlockN * 128;                  // one K block of a database tile
-  static constexpr int kCore = kAResident + STAGES * kBBytes + 256;
-  static constexpr int kCoreAligned = (kCore + 1023) / 1024 * 1024;
-  static constexpr int kTotal = kCoreAligned + 1024;
-};
-
-template <int STAGES, int KB, class Epilogue>
-__global__ void __launch_bounds__(gemm_threads<kAresBlockN, Epilogue>(), 1)
-gemm_ares_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
-                         const AresShape shape, const __grid_constant__ typename Epilogue::Params ep) {
-  using L = AresSmemLayout<STAGES, KB>;
-  constexpr int kAccCols = kAresMT * kAresBlockN;   // 256 columns per accumulator buffer
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* smem_a = smem;
-  uint8_t* smem_b = smem + L::kAResident;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L::kAResident + STAGES * L::kBBytes);
-  uint64_t* full_bar = bars;
-  uint64_t* empty_bar = bars + STAGES;
-  uint64_t* acc_full = bars + 2 * STAGES;
-  uint64_t* acc_empty = bars + 2 * STAGES + 2;
-  uint64_t* a_full = bars + 2 * STAGES + 4;
-  uint64_t* a_empty = bars + 2 * STAGES + 5;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 6);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  pdl_launch_dependents();
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmap_a);
-    tma_prefetch_desc(&tmap_b);
-    for (int i = 0; i < STAGES; ++i) {
-      mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&acc_full[i], 1);
-      mbar_init(&acc_empty[i], 4 * gemm_column_split<kAresBlockN, Epilogue>());
-    }
-    mbar_init(a_full, 1);
-    mbar_init(a_empty, 1);
-    fence_mbar_init();
-  }
-  if (warp == 1) {
-    tmem_alloc(tmem_slot, 512);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
-
-  if (warp == 0) {
-    // ------------------------------ TMA producer ------------------------------
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0, a_phase = 0;
-      AresWalk walk(shape, blockIdx.x, gridDim.x);
-      int mts, nt0, nt1;
-      while (walk.next(mts, nt0, nt1)) {
-        mbar_wait(a_empty, a_phase ^ 1);   // the previous item's UMMAs have read the resident query tile
-        a_phase ^= 1;
-        mbar_arrive_expect_tx(a_full, L::kAResident);
-#pragma unroll
-        for (int sub = 0; sub < kAresMT; ++sub)
-#pragma unroll
-          for (int kb = 0; kb < KB; ++kb)
-            tma_load_2d(&tmap_a, a_full, smem_a + (sub * KB + kb) * L::kABytes, kb * 64, (mts * kAresMT + sub) * kBlockM);
-        for (int nt = nt0; nt < nt1; ++nt) {
-#pragma unroll
-          for (int kb = 0; kb < KB; ++kb) {
-            mbar_wait(&empty_bar[stage], phase ^ 1);
-            mbar_arrive_expect_tx(&full_bar[stage], L::kBBytes);
-            tma_load_2d(&tmap_b, &full_bar[stage], smem_b + stage * L::kBBytes, kb * 64, nt * kAresBlockN);
-            if (++stage == STAGES) { stage = 0; phase ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ------------------------------ UMMA issuer ------------------------------
-    if (lane == 0) {
-      constexpr uint32_t idesc = umma_idesc_bf16(kBlockM, kAresBlockN);
-      int stage = 0, local = 0;
-      uint32_t phase = 0, a_phase = 0;
-      AresWalk walk(shape, blockIdx.x, gridDim.x);
-      int mts, nt0, nt1;
-      const uint32_t a_base = smem_u32(smem_a);
-      while (walk.next(mts, nt0, nt1)) {
-        mbar_wait(a_full, a_phase);
-        a_phase ^= 1;
-        tc_fence_after();
-        for (int nt = nt0; nt < nt1; ++nt, ++local) {
-          const int acc = local & 1;
-          mbar_wait(&acc_empty[acc], ((local >> 1) & 1) ^ 1);
-          tc_fence_after();
-          const uint32_t d_tmem = tmem_base + acc * kAccCols;
-#pragma unroll
-          for (int kb = 0; kb < KB; ++kb) {
-            mbar_wait(&full_bar[stage], phase);
-            tc_fence_after();
-            const uint64_t bdesc = umma_smem_desc_kmajor<128>(smem_u32(smem_b + stage * L::kBBytes));
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-#pragma unroll
-              for (int sub = 0; sub < kAresMT; ++sub) {
-                const uint64_t adesc = umma_smem_desc_kmajor<128>(a_base + (sub * KB + kb) * L::kABytes);
-                umma_bf16(d_tmem + sub * kAresBlockN, adesc + 2 * k, bdesc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
-              }
-            }
-            umma_commit(&empty_bar[stage]);
-            if (++stage == STAGES) { stage = 0; phase ^= 1; }
-          }
-          umma_commit(&acc_full[acc]);
-        }
-        umma_commit(a_empty);   // arrives when every UMMA of this item has completed
-      }
-    }
-  } else {
-    // ------------------------------ epilogue ------------------------------
-    constexpr int kSplit = gemm_column_split<kAresBlockN, Epilogue>();
-    constexpr int kColsPerWarp = kAresBlockN / kSplit;
-    const int quarter = warp & 3;
-    const int row = quarter * 32 + lane;
-    const int col_begin = ((warp - 2) >> 2) * kColsPerWarp;
-    int local = 0;
-    AresWalk walk(shape, blockIdx.x, gridDim.x);
-    int mts, nt0, nt1;
-    Epilogue epi;
-    epi.setup(ep, smem + L::kCoreAligned, warp - 2, lane);
-    while (walk.next(mts, nt0, nt1)) {
-      for (int nt = nt0; nt < nt1; ++nt, ++local) {
-        const int acc = local & 1;
-        mbar_wait(&acc_full[acc], (local >> 1) & 1);
-        tc_fence_after();
-#pragma unroll 1
-        for (int sub = 0; sub < kAresMT; ++sub) {
-          const int mt = mts * kAresMT + sub;
-          const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + acc * kAccCols + sub * kAresBlockN;
-          epi.begin(ep, mt, nt, row);
-#pragma unroll 1
-          for (int c = col_begin; c < col_begin + kColsPerWarp; c += 32) {
-            uint32_t v[32];
-            tmem_ld_32x32(taddr + c, v);
-            tmem_ld_wait();
-            epi.chunk(ep, mt, nt * kAresBlockN + c, row, v, 0);
-          }
-          epi.end(ep, mt, nt, row);
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&acc_empty[acc]);
-      }
-    }
-    epi.finish(ep, lane);
-  }
-
-  __syncwarp();
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
 // =================================================================================================
 // CTA-pair version of the A-resident join kernel (tcgen05 cta_group::2). An SS-mode UMMA streams both operands from shared
 // memory: (128 + N) rows x 32 B per instruction, i.e. 128 B/clk at M128 N128 - the whole shared-memory port, with the TMA
-// fill (32 B/clk here) on top; that is what held the single-CTA kernel at 0.74 of the tensor peak. A pair of CTAs issues
+// fill (32 B/clk) on top; that is what held a single-CTA version of this schedule (M128 N128 UMMAs, 256 resident query
+// rows) at 0.74 of the tensor peak. A pair of CTAs issues
 // ONE UMMA of M = 256, N = 256: each SM computes its 128 query rows against all 256 database rows but keeps only 128 of
 // them (16 KB per K block) in its own shared memory and reads the peer's half over the pair link: 64 B/clk of operand
 // reads + 32 B/clk of fill per SM.
@@ -802,7 +582,6 @@ gemm_ares2_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gr
   const int lane = threadIdx.x & 31;
   const uint32_t crank = cluster_ctarank();
   const bool leader = crank == 0;
-  pdl_launch_dependents();
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_a);
     tma_prefetch_desc(&tmap_b);
@@ -827,7 +606,6 @@ gemm_ares2_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gr
   cluster_sync_all();   // both CTAs' barriers and TMEM exist before any cross-CTA traffic
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
   const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
 
   if (warp == 0) {
@@ -979,7 +757,6 @@ gemm_pair_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
   const int lane = threadIdx.x & 31;
   const uint32_t crank = cluster_ctarank();
   const bool leader = crank == 0;
-  pdl_launch_dependents();
   GemmShape shape = shape_in;
   const int m_tiles_real = shape_in.m_tiles;
   shape.m_tiles = (shape_in.m_tiles + 1) / 2;   // the walk runs over pairs of row tiles
@@ -1007,7 +784,6 @@ gemm_pair_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
   cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
 
   if (warp == 0) {
     // ------------------------------ TMA producer (both CTAs) ------------------------------

@@ -27,13 +27,6 @@ __device__ __forceinline__ bool elect_one() {
   return pred != 0;
 }
 
-// Programmatic dependent launch: launch_dependents lets the next kernel of the stream be scheduled as soon as every CTA of
-// this grid has issued it (or exited); wait blocks until the PREVIOUS grid has completed and its memory is visible.
-// Both are no-ops for a kernel launched without the programmatic-serialization attribute. Every kernel that may be
-// launched with the attribute must execute pdl_wait() before its first access to memory another kernel produced.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
 // Device-visible error word: kernels write a nonzero code and trap instead of spinning forever.
 // (a hung kernel on a shared box costs a strike; a trapped one only costs the call.)
 __device__ unsigned int g_vfp_device_error = 0;
@@ -183,14 +176,6 @@ __device__ __forceinline__ void tma_load_4d(const CUtensorMap* m, uint64_t* bar,
       : "memory");
 }
 
-// Multicast variant: the box lands at the same shared-memory offset of every CTA of the cluster named in `cta_mask`, and each of
-// those CTAs' mbarrier (same offset) receives the complete_tx for the bytes written into ITS shared memory.
-__device__ __forceinline__ void tma_load_2d_mcast(const CUtensorMap* m, uint64_t* bar, void* dst, int c0, int c1, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask)
-      : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -258,13 +243,6 @@ __device__ __forceinline__ void umma_commit_2cta(uint64_t* bar, uint16_t cta_mas
                : "memory");
 }
 
-// TMA prefetch of a 2-D tile into L2 only (no shared-memory destination, no completion to wait for)
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* m, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0),
-               "r"(c1)
-               : "memory");
-}
-
 // TMA tiled store (shared -> global), bulk-group completion
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* src, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
@@ -313,13 +291,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
 // Arrive on an mbarrier once all previously issued UMMAs of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-// The same arrival delivered to the mbarrier at this offset in every CTA of `cta_mask` (a stage that holds multicast data is
-// free only when EVERY CTA that received it has consumed it).
-__device__ __forceinline__ void umma_commit_mcast(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(cta_mask)
                : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }

@@ -159,7 +159,6 @@ __global__ void __launch_bounds__(kStemThreads, 1) stem_ts_kernel(const __grid_c
 
   const int tid = threadIdx.x;
   const int warp = tid >> 5, lane = tid & 31;
-  pdl_launch_dependents();
   // a conv pass is at most 16384 frames, so 32-bit counters are enough everywhere below
   const int n_local = (p.n_frames > blockIdx.x) ? (int)((p.n_frames - blockIdx.x + gridDim.x - 1) / gridDim.x) : 0;
   const int n_tiles = 4 * n_local, n_units = 2 * n_local;
@@ -203,7 +202,6 @@ __global__ void __launch_bounds__(kStemThreads, 1) stem_ts_kernel(const __grid_c
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t plane_bytes = p.frame_dtype == kFrameBF16 ? 8192u : 4096u;
-  pdl_wait();   // the previous conv pass (conv3 still reads the c2 buffer this kernel overwrites) must have completed
 
   // ------------------------------ transposers: raw planes -> HWC tile (warp 2 and WG5, ltid 0 .. 159) ------------------------------
   auto transposer_role = [&](int ltid) {

@@ -27,8 +27,6 @@ struct FrameSrc {
 // frame encoder's loaders read (the frames themselves need not be packed).
 __global__ void token_map_kernel(const int* __restrict__ cu, const FrameSrc* __restrict__ src, int n_clips, int n_tokens,
                                  int* __restrict__ tok_pos, int* __restrict__ tok_len, unsigned long long* __restrict__ frame_addr) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= n_tokens) return;
   int lo = 0, hi = n_clips;  // find v with cu[v] <= t < cu[v+1]
@@ -57,8 +55,6 @@ add_layernorm_bf16_kernel(float* __restrict__ x, const __nv_bfloat16* __restrict
                           const __nv_bfloat16* __restrict__ delta2 /*nullable, added after delta*/,
                           const float* __restrict__ gamma, const float* __restrict__ beta, __nv_bfloat16* __restrict__ y,
                           int n_tokens, int write_x) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp >= n_tokens) return;
@@ -118,8 +114,6 @@ __global__ void __launch_bounds__(256)
 add_convert_bf16_kernel(float* __restrict__ x, const __nv_bfloat16* __restrict__ delta /*nullable*/,
                         const __nv_bfloat16* __restrict__ delta2 /*nullable, added after delta*/, __nv_bfloat16* __restrict__ xbf,
                         long long n8) {
-  pdl_launch_dependents();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n8) return;
   float4* xr = reinterpret_cast<float4*>(x) + 2 * i;
@@ -232,7 +226,6 @@ __global__ void __launch_bounds__(kTc2Threads, 2) temporal_conv_tma_kernel(const
   uint64_t* full = reinterpret_cast<uint64_t*>(masks + 64);                                  // [2] tile rows + masks have landed
   uint64_t* empty = full + 2;                                                               // [2] 8 compute warps are done with the tile
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  pdl_launch_dependents();
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&p.tmap_x);
     mbar_init(&full[0], 1);
@@ -250,7 +243,6 @@ __global__ void __launch_bounds__(kTc2Threads, 2) temporal_conv_tma_kernel(const
                              __ldg(p.w + (2 * 11 + tap) * kDim + o), __ldg(p.w + (3 * 11 + tap) * kDim + o));
   }
   __syncthreads();
-  pdl_wait();
   if (warp == 8) {
     // ---- producer: one TMA box per tile; lane i works out which taps of token i stay inside the token's own clip ----
     int it = 0;
@@ -375,8 +367,6 @@ __global__ void __launch_bounds__(kAttThreads, 3)
 attention_fa_kernel(const __nv_bfloat16* __restrict__ qkv, const int4* __restrict__ items /*{first query token, clip start, clip end, 0}*/,
                     __nv_bfloat16* __restrict__ out, int n_tokens) {
   extern __shared__ __align__(16) uint8_t att_smem[];
-  pdl_launch_dependents();
-  pdl_wait();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = lane >> 2, tig = lane & 3;
   const int4 item = __ldg(items + blockIdx.x);
@@ -534,8 +524,6 @@ attention_fa_kernel(const __nv_bfloat16* __restrict__ qkv, const int4* __restric
 __global__ void __launch_bounds__(256)
 temporal_pool_kernel(const float* __restrict__ x, const float* __restrict__ logits, const int* __restrict__ cu,
                      float* __restrict__ pooled /*[clips][768]*/, __nv_bfloat16* __restrict__ pooled_bf /*same, bf16*/) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int clip = blockIdx.x, c = threadIdx.x;
   const int t0 = cu[clip], T = cu[clip + 1] - t0;
   float sum = 0.f, mx = -INFINITY, m = -INFINITY, l = 0.f, ws = 0.f;
@@ -575,8 +563,6 @@ final_projection_kernel(const float* __restrict__ pooled, const float* __restric
   __shared__ float sp[kClips][3 * kDim];
   __shared__ float sh[kClips][kDim];
   __shared__ float red[kClips][8];
-  pdl_launch_dependents();
-  pdl_wait();
   const int c0 = blockIdx.x * kClips;
   const int tid = threadIdx.x;
   for (int i = tid; i < kClips * 3 * kDim; i += 256) {

@@ -18,11 +18,6 @@
 
 namespace vfp {
 
-// L2 prefetch distance (column tiles) of the top-k screen for databases that do not fit L2 (vfp_set_tuning key 6). Off by
-// default: measured no effect (65 536 queries x 4 M rows: 464 ms with 0, 4, 8, 16 or 32) - the screen is bound by its
-// candidate-list epilogue, not by the database fetch, unlike the threshold join (+22 % there).
-static int g_topk_prefetch = 0;
-
 constexpr int kTopKCand = 64;        // approximate candidates kept per query row
 constexpr int kTopKMaxK = 32;
 constexpr int kTopKMaxSegments = 32;
@@ -424,7 +419,6 @@ inline int topk_run(const float* q, const float* db, int64_t n_q, int64_t n_db, 
   s.n_tiles = (int)((n_db + 255) / 256);
   s.row_resident = 1;
   s.n_segments = L.n_segments;
-  s.b_prefetch_tiles = (size_t)n_db * 2 * dim > ((size_t)160 << 20) ? g_topk_prefetch : 0;   // database tiles from HBM: see gemm_sm100.cuh
   EpiTopK::Params ep{};
   ep.q_rows = n_q; ep.db_rows = n_db; ep.n_segments = L.n_segments; ep.part_s = part_s; ep.part_i = part_i;
   if (ck((launch_gemm<256, 64, 3, EpiTopK>(ta, tb, s, ep, st)), "screen launch")) return 1;

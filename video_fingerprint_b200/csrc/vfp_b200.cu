@@ -53,11 +53,11 @@ constexpr float kBnEps = 1e-5f;
 // ---------------------------------------------------------------------------------------------
 enum Stage : int {
   kStConv1 = 0, kStConv2, kStConv3, kStConv4, kStTokEmbed, kStTemporalConv, kStLayerNorm, kStQkv, kStAttention,
-  kStOutProj, kStMlp1, kStMlp2, kStPoolGemm, kStPool, kStFinal, kStMisc, kStStemFused, kStFfn, kNumStages
+  kStOutProj, kStPoolGemm, kStPool, kStFinal, kStMisc, kStStemFused, kStFfn, kNumStages
 };
 const char* const kStageNames[kNumStages] = {"conv1_stem", "conv2_igemm", "conv3_igemm", "conv4_igemm_pool", "token_embed_gemm",
                                              "temporal_conv", "layernorm", "qkv_gemm", "attention", "out_proj_gemm",
-                                             "mlp1_gemm_gelu", "mlp2_gemm", "pool_logits_gemm", "temporal_pool",
+                                             "pool_logits_gemm", "temporal_pool",
                                              "final_projection", "misc", "stem_fused", "ffn_fused"};
 struct Profiler {
   bool enabled = false;
@@ -105,8 +105,7 @@ struct AttnBlockWeights {
   float *ln1_w, *ln1_b, *ln2_w, *ln2_b;
   __nv_bfloat16 *wqkv, *wo, *w1, *w2;
   float *bqkv, *bo, *b1, *b2;
-  CUtensorMap tm_qkv, tm_o, tm_w1, tm_w2;
-  CUtensorMap tm_qkv_h, tm_o_h;       // the same weights with boxes of 128 rows: CTA-pair GEMM (one CTA's half of a 256-row tile)
+  CUtensorMap tm_qkv, tm_o;
   CUtensorMap tm_w1_ffn, tm_w2_ffn;   // fused feed-forward kernel: boxes of 128 rows x 64 columns (one CTA's half of a 256-row block)
 };
 
@@ -121,8 +120,8 @@ struct vfp_weights {
   float* c1_bias = nullptr;
   __nv_bfloat16 *c2_w = nullptr, *c3_w = nullptr, *c4_w = nullptr;
   float *c2_b = nullptr, *c3_b = nullptr, *c4_b = nullptr;
-  CUtensorMap tm_c2, tm_c3, tm_c4;
-  CUtensorMap tm_c3h, tm_c4h;   // the same filters with boxes of half the rows: multicast loads of CTA pairs
+  CUtensorMap tm_c2;
+  CUtensorMap tm_c4h;   // conv4 filters with boxes of half the rows: one CTA's half of the CTA-pair GEMM's B tile
   __nv_bfloat16* c2f_w = nullptr;  // conv2 weights in the K order of the fused stem kernel
   CUtensorMap tm_c2f;
   __nv_bfloat16* c1ts_w = nullptr;  // conv1 weights stacked for the TS-mode stem kernel: [64 = (sw, c_out)][128 = (kh, 24 window values)]
@@ -239,14 +238,17 @@ int prep_f32(vfp_weights* w, const float* src, size_t n, float** dev) {
 
 // ---------------------------------------------------------------------------------------------
 // forward workspace. Two regions with different granularity:
-//   * the TOKEN region holds one "token pass" (up to all clips of the call): 8.5 KB per frame/token. The token
+//   * the TOKEN region holds one "token pass" (up to all clips of the call): 7.5 KB per frame/token. The token
 //     GEMMs, LayerNorm, attention, pooling and the head each run ONCE per token pass, so their launches are large;
 //   * the CONV region holds the activations of one "conv pass" (up to 65 536 frames by default, 48 KB per frame, plus 64 KB
 //     per frame for 16 384 frames of conv1 output that only the two-kernel stem uses): the frame encoder walks the token
 //     pass in such slices and only leaves the 512 B/frame pooled features behind.
 // ---------------------------------------------------------------------------------------------
 constexpr int64_t kConvPassFrames = 262144;  // workspace is sized for this many frames per conv pass (48 KB per frame)
-constexpr int64_t kStemPassFrames = 16384;   // ... and for this many frames of conv1 output (64 KB per frame, two-kernel stem only)
+// ... and for this many frames of conv1 output (64 KB per frame, two-kernel stem only), which steps through a conv pass in
+// sub-passes of this size. Measured on B200 (10k x 64-frame clips): 512 -> 71.3 ms/step, 1024 -> 62.9, 2048 -> 60.7,
+// 4096 -> 58.9, 16384 -> 55.8: short L2-sized sub-passes lose more to small launches than they save in HBM traffic.
+constexpr int64_t kStemPassFrames = 16384;
 // frames actually walked per conv pass (vfp_set_tuning key 3, <= kConvPassFrames). Every launch of the three persistent
 // frame-encoder kernels costs ~13-16 us that do not scale with its size (cluster launch, TMEM allocation, the filters' trip
 // into tensor memory, pipeline ramp and drain), so passes are LARGE: 10 000 x 64-frame clips take 32.9 ms per step with
@@ -254,27 +256,14 @@ constexpr int64_t kStemPassFrames = 16384;   // ... and for this many frames of 
 // enough to keep c2 / c3 in the 126 MB L2 (2 048 - 4 096 frames) lose far more to those fixed costs than they save in
 // HBM traffic: 36.3 - 39.4 ms, 35.1 - 36.7 with programmatic dependent launch.
 int64_t g_conv_pass_frames = 65536;
-// conv1+conv2 sub-pass. Measured on B200 (10k x 64-frame clips): 512 -> 71.3 ms/step, 1024 -> 62.9, 2048 -> 60.7,
-// 4096 -> 58.9, 16384 -> 55.8: short L2-sized sub-passes lose more to small launches than they save in HBM traffic.
-int64_t g_stem_pass_frames = kStemPassFrames;
 // conv1+conv2 in one kernel (stem_ts_kernel.cuh: conv1's output stays in shared memory as conv2's UMMA operand).
 // Measured on B200 (10k x 64-frame clips): 13.3 ms vs 13.4 + 12.9 ms for the two HBM-bound kernels, so it is the
 // default for u8 / bf16 frames; vfp_set_tuning(1, 0) selects the two-kernel path (always used for fp32 frames).
 int g_fused_stem = 2;
-int g_join_prefetch = 16;  // vfp_set_tuning key 5: column tiles of L2 prefetch distance in the join (0 = off)
-// Measured (10 000 clips): conv4 5.19 -> 4.9 ms on pairs; QKV 1.25 -> 1.91 and the out-projection 0.48 -> 0.64 ms (their K = 256
-// weight block is better kept resident in shared memory, gemm_bres_tcgen05_kernel), hence bit 1 is off by default.
 int g_attention_tc = 1;    // key 17: attention on tcgen05 (attention_tc_kernel.cuh) instead of the mma.sync kernel
-int g_conv3_ts = 1;         // key 16: conv3 with its filters in tensor memory (TS-mode UMMAs) instead of the generic SWAP kernel
-int g_pair_gemm = 1;        // key 15: bit 0 conv4, bit 1 QKV / out-projection on CTA pairs (gemm_pair_tcgen05_kernel)
-int g_ffn_mode = 1;         // key 14: 0 = two GEMM launches, 1 = fused feed-forward kernel on CTA pairs
-int g_conv_mcast = 0;       // key 13: bit 0 conv3, bit 1 conv4 run as CTA pairs that share the filter tile through multicast TMA
-int g_join_kernel = 2;      // key 10: 0 = the generic tile kernel, 1 = A-resident panel-major kernel, 2 = the same on CTA pairs (cta_group::2)
-int g_join_symmetric = 1;   // key 11: self joins screen the upper triangle only
-int g_join_panel_tiles = 512;  // key 12: database column tiles (of 128 rows) per L2 panel
 
 struct TokenWs {
-  size_t cu, frame_src, att_items, frame_addr, tok_pos, tok_len, feat, xa, xb, xn, qkv, att, delta, delta2, h, logits, xbf, pooled, pooled_bf, head_h, total;
+  size_t cu, frame_src, att_items, frame_addr, tok_pos, tok_len, feat, xa, xb, xn, qkv, att, delta, delta2, logits, xbf, pooled, pooled_bf, head_h, total;
 };
 struct ConvWs {
   size_t c1, c2, c3, total;
@@ -302,7 +291,6 @@ TokenWs token_ws_layout(int64_t F, int64_t C) {
   L.att = take((size_t)F * kDim * 2);
   L.delta = take((size_t)F * kDim * 2);
   L.delta2 = take((size_t)F * kDim * 2);
-  L.h = take((size_t)F * 4 * kDim * 2);
   L.logits = take((size_t)F * kDim * 4);
   L.xbf = take((size_t)F * kDim * 2);
   L.pooled = take((size_t)C * 3 * kDim * 4);
@@ -369,21 +357,9 @@ int vfp_device_sm_count(void) {
 }
 
 int vfp_set_tuning(int key, long long value) {
-  if (key == 0 && value >= 64 && value <= kStemPassFrames) { g_stem_pass_frames = value; return 0; }
   if (key == 1 && (value == 0 || value == 2)) { g_fused_stem = (int)value; return 0; }
-  if (key == 5 && value >= 0 && value <= 4096) { g_join_prefetch = (int)value; return 0; }
-  if (key == 6 && value >= 0 && value <= 4096) { g_topk_prefetch = (int)value; return 0; }
   if (key == 3 && value >= 64 && value <= kConvPassFrames) { g_conv_pass_frames = value; return 0; }
-  if (key == 16 && value >= 0 && value <= 1) { g_conv3_ts = (int)value; return 0; }
   if (key == 17 && value >= 0 && value <= 1) { g_attention_tc = (int)value; return 0; }
-  if (key == 15 && value >= 0 && value <= 3) { g_pair_gemm = (int)value; return 0; }
-  if (key == 14 && value >= 0 && value <= 1) { g_ffn_mode = (int)value; return 0; }
-  if (key == 13 && value >= 0 && value <= 3) { g_conv_mcast = (int)value; return 0; }
-  if (key == 10 && value >= 0 && value <= 2) { g_join_kernel = (int)value; return 0; }
-  if (key == 11 && value >= 0 && value <= 1) { g_join_symmetric = (int)value; return 0; }
-  if (key == 12 && value >= 16 && value <= 65536) { g_join_panel_tiles = (int)value; return 0; }
-  if (key == 7 && value >= 0 && value <= 1) { pdl_enabled().store((int)value); return 0; }            // programmatic dependent launch
-  if (key == 8 && value >= 0 && value <= 4096) { persistent_cta_limit().store((int)value); return 0; }  // CTAs per persistent kernel (0 = all SMs)
   if (key == 9 && value >= 1 && value <= kMaxPipes) { g_forward_pipes = (int)value; return 0; }        // pipelines (internal streams) of vfp_forward
   if (key == 2) {  // hang diagnosis: timed-out mbarrier waits are logged and abandoned instead of trapping
     const int mode = value != 0;
@@ -622,12 +598,9 @@ int vfp_weights_create(const vfp_tensor_desc* tensors, int n_tensors, vfp_weight
       if (prep_dense_bf16(w, src, (size_t)it.n, it.dst)) return bail("");
     }
     if (make_tmap_rows_bf16(&a.tm_qkv, a.wqkv, 3 * kDim, kDim, kDim, 256, 64) ||
-        make_tmap_rows_bf16(&a.tm_o, a.wo, kDim, kDim, kDim, 256, 64) ||
-        make_tmap_rows_bf16(&a.tm_w1, a.w1, 4 * kDim, kDim, kDim, 256, 64) ||
-        make_tmap_rows_bf16(&a.tm_w2, a.w2, kDim, 4 * kDim, 4 * kDim, 256, 64))
+        make_tmap_rows_bf16(&a.tm_o, a.wo, kDim, kDim, kDim, 256, 64))
       return bail("tensor map encode failed (attention weights)");
-    if (make_tmap_rows_bf16(&a.tm_qkv_h, a.wqkv, 3 * kDim, kDim, kDim, 128, 64) || make_tmap_rows_bf16(&a.tm_o_h, a.wo, kDim, kDim, kDim, 128, 64) ||
-        make_tmap_rows_bf16(&a.tm_w1_ffn, a.w1, 4 * kDim, kDim, kDim, 128, 64) ||
+    if (make_tmap_rows_bf16(&a.tm_w1_ffn, a.w1, 4 * kDim, kDim, kDim, 128, 64) ||
         make_tmap_rows_bf16(&a.tm_w2_ffn, a.w2, kDim, 4 * kDim, 4 * kDim, 128, 64))
       return bail("tensor map encode failed (feed-forward weights)");
   }
@@ -666,9 +639,6 @@ int vfp_weights_create(const vfp_tensor_desc* tensors, int n_tensors, vfp_weight
   if (make_tmap_rows_bf16(&w->tm_c2, w->c2_w, 64, 384, 384, 64, 64) ||
       make_tmap_rows_bf16(&w->tm_c2f, w->c2f_w, 64, 320, 320, 64, 64) ||
       make_tmap_rows_bf16(&w->tm_c1ts, w->c1ts_w, 64, 128, 128, 64, 64) ||
-      make_tmap_rows_bf16(&w->tm_c3, w->c3_w, 128, 576, 576, 128, 64) ||
-      make_tmap_rows_bf16(&w->tm_c4, w->c4_w, 256, 1152, 1152, 256, 64) ||
-      make_tmap_rows_bf16(&w->tm_c3h, w->c3_w, 128, 576, 576, 64, 64) ||
       make_tmap_rows_bf16(&w->tm_c4h, w->c4_w, 256, 1152, 1152, 128, 64) ||
       make_tmap_rows_bf16(&w->tm_tok, w->wtok, kDim, 256, 256, 256, 64) ||
       make_tmap_rows_bf16(&w->tm_pool, w->wpool, kDim, kDim, kDim, 256, 64))
@@ -696,8 +666,6 @@ int encode_frames_pass(const vfp_weights* w, const unsigned long long* frame_add
   __nv_bfloat16* c1a = reinterpret_cast<__nv_bfloat16*>(conv_ws + L.c1);
   __nv_bfloat16* c2a = reinterpret_cast<__nv_bfloat16*>(conv_ws + L.c2);
   __nv_bfloat16* c3a = reinterpret_cast<__nv_bfloat16*>(conv_ws + L.c3);
-  // conv1 + conv2 can run in shorter "stem passes" (vfp_set_tuning key 0) so that conv1's output (64 KB per frame,
-  // the largest tensor of the forward) is still in L2 when conv2 reads it; by default one stem pass = the conv pass.
   CUtensorMap ta;
   // the fused stem streams raw frame planes with 16-byte bulk copies; fp32 frames (48 KB) do not fit its smem ring
   const bool fused = g_fused_stem && frame_dtype != VFP_FRAME_F32 && fused_ok;
@@ -710,12 +678,12 @@ int encode_frames_pass(const vfp_weights* w, const unsigned long long* frame_add
     sp.c2_bias = w->c2_b;
     VFP_CUDA(ensure_dynamic_smem(reinterpret_cast<const void*>(stem_ts_kernel), StemTsSmem::kTotal));
     g_prof.launches += 1;
-    const int grid = (int)std::min<int64_t>(F, persistent_grid());
+    const int grid = (int)std::min<int64_t>(F, device_sm_count());
     VFP_CUDA(launch_kernel(stem_ts_kernel, dim3(grid), dim3(kStemThreads), StemTsSmem::kTotal, st, sp));
     g_prof.mark(kStStemFused, st);
   }
-  for (int64_t s0 = 0; s0 < F && !fused; s0 += g_stem_pass_frames) {
-    const int64_t n = std::min<int64_t>(g_stem_pass_frames, F - s0);
+  for (int64_t s0 = 0; s0 < F && !fused; s0 += kStemPassFrames) {
+    const int64_t n = std::min<int64_t>(kStemPassFrames, F - s0);
     g_prof.launches += 2;
     {
       const long long grid = std::min<long long>(n, (long long)device_sm_count() * 10);
@@ -742,31 +710,16 @@ int encode_frames_pass(const vfp_weights* w, const unsigned long long* frame_add
     }
   }
   g_prof.launches += 2;
-  {  // conv3: 16x16x64 -> 8x8x128 through a stride-2 box, tile = 2 frames. (A weight-resident variant - launch_gemm_bres<128, 64, 3, 9>,
-     // all nine filter blocks in shared memory, M = 128 pixels - measured 2.01 ms vs 1.25 ms per 131 072 frames: the kernel is
-     // bound by the nine-fold L2 -> SM re-read of the input pixels, not by the weights.)
-    if (g_conv3_ts) {   // filters in tensor memory, three frames per tile (conv3_ts_kernel.cuh)
-      Conv3Params cp{};
-      if (make_tmap_nhwc_bf16(&cp.tmap_in, c2a, F, 16, 16, 64, 64, 8, 8, kC3Frames, 2) || make_tmap_out(&cp.tmap_out, c3a, (uint64_t)F * 64, 128, true))
-        return fail("tensor map encode failed (conv3)");
-      cp.w = w->c3_w; cp.bias = w->c3_b; cp.n_tiles = (int)((F + kC3Frames - 1) / kC3Frames);
-      VFP_CUDA(ensure_dynamic_smem(reinterpret_cast<const void*>(conv3_ts_kernel<7>), Conv3Smem<7>::kTotal));
-      VFP_CUDA(launch_kernel(conv3_ts_kernel<7>, dim3(std::min(cp.n_tiles, persistent_grid())), dim3(kC3Threads), Conv3Smem<7>::kTotal, st, cp));
-      g_prof.mark(kStConv3, st);
-    } else {
-    if (make_tmap_nhwc_bf16(&ta, c2a, F, 16, 16, 64, 64, 8, 8, 2, 2)) return fail("tensor map encode failed (conv3)");
-    GemmShape s{};
-    s.m_tiles = (int)((F + 1) / 2); s.n_tiles = 1; s.k_blocks = 9; s.group_m = 16; s.a_conv = 1;
-    s.tiles_per_frame = 1; s.frames_per_tile = 2; s.tile_out_rows = 8;
-    conv_taps_strided(&s, 1);
-    EpiConvTransposedTma::Params ep{};
-    if (make_tmap_out(&ep.tmap_out, c3a, (uint64_t)F * 64, 128, true)) return fail("tensor map encode failed (conv3 out)");
-    ep.bias = w->c3_b; ep.c_out = 128; ep.pixels_per_tile = 256;
-    // channels on M (128), four frames (256 pixels) on N
-    if (g_conv_mcast & 1) VFP_CUDA((launch_gemm<128, 64, 4, EpiConvTransposedTma, 2, true, 2>(ta, w->tm_c3h, s, ep, st)));
-    else VFP_CUDA((launch_gemm<128, 64, 4, EpiConvTransposedTma, 2, true>(ta, w->tm_c3, s, ep, st)));
+  {  // conv3: 16x16x64 -> 8x8x128 with its filters in tensor memory, three frames per tile (conv3_ts_kernel.cuh). (A weight-resident
+     // variant - launch_gemm_bres<128, 64, 3, 9>, all nine filter blocks in shared memory, M = 128 pixels - measured 2.01 ms vs
+     // 1.25 ms per 131 072 frames: the kernel is bound by the nine-fold L2 -> SM re-read of the input pixels, not by the weights.)
+    Conv3Params cp{};
+    if (make_tmap_nhwc_bf16(&cp.tmap_in, c2a, F, 16, 16, 64, 64, 8, 8, kC3Frames, 2) || make_tmap_out(&cp.tmap_out, c3a, (uint64_t)F * 64, 128, true))
+      return fail("tensor map encode failed (conv3)");
+    cp.w = w->c3_w; cp.bias = w->c3_b; cp.n_tiles = (int)((F + kC3Frames - 1) / kC3Frames);
+    VFP_CUDA(ensure_dynamic_smem(reinterpret_cast<const void*>(conv3_ts_kernel<7>), Conv3Smem<7>::kTotal));
+    VFP_CUDA(launch_kernel(conv3_ts_kernel<7>, dim3(std::min(cp.n_tiles, device_sm_count())), dim3(kC3Threads), Conv3Smem<7>::kTotal, st, cp));
     g_prof.mark(kStConv3, st);
-    }
   }
   {  // conv4: 8x8x128 -> 4x4x256 + ReLU + global average pool, tile = 8 frames
     if (make_tmap_nhwc_bf16(&ta, c3a, F, 8, 8, 128, 64, 4, 4, 8, 2)) return fail("tensor map encode failed (conv4)");
@@ -776,9 +729,8 @@ int encode_frames_pass(const vfp_weights* w, const unsigned long long* frame_add
     conv_taps_strided(&s, 2);
     EpiConvPool16::Params ep{};
     ep.bias = w->c4_b; ep.out_bf16 = feat_out; ep.frames = (int)F; ep.N = 256;
-    if (g_pair_gemm & 1) VFP_CUDA((launch_gemm_pair<64, 6, EpiConvPool16>(ta, w->tm_c4h, s, ep, st)));   // CTA pairs: one M256 N256 UMMA per K step
-    else if (g_conv_mcast & 2) VFP_CUDA((launch_gemm<256, 64, 4, EpiConvPool16, 1, false, 2>(ta, w->tm_c4h, s, ep, st)));
-    else VFP_CUDA((launch_gemm<256, 64, 4, EpiConvPool16>(ta, w->tm_c4, s, ep, st)));
+    // CTA pairs: one M256 N256 UMMA per K step. Measured (10 000 clips): 5.19 ms with one CTA per tile, 4.9 ms on pairs.
+    VFP_CUDA((launch_gemm_pair<64, 6, EpiConvPool16>(ta, w->tm_c4h, s, ep, st)));
     g_prof.mark(kStConv4, st);
   }
   return 0;
@@ -806,7 +758,6 @@ int forward_pass(const vfp_weights* w, const FrameSrc* src, int frame_dtype, boo
   __nv_bfloat16* att = reinterpret_cast<__nv_bfloat16*>(ws + L.att);
   __nv_bfloat16* delta = reinterpret_cast<__nv_bfloat16*>(ws + L.delta);     // attention out-projection of the current block
   __nv_bfloat16* delta_f = reinterpret_cast<__nv_bfloat16*>(ws + L.delta2);  // MLP output of the previous block
-  __nv_bfloat16* hbuf = reinterpret_cast<__nv_bfloat16*>(ws + L.h);
   float* logits = reinterpret_cast<float*>(ws + L.logits);
   __nv_bfloat16* xbf = reinterpret_cast<__nv_bfloat16*>(ws + L.xbf);
   float* pooled = reinterpret_cast<float*>(ws + L.pooled);
@@ -856,22 +807,18 @@ int forward_pass(const vfp_weights* w, const FrameSrc* src, int frame_dtype, boo
     }
     return 0;
   };
-  // bf16-output token GEMM, result written by the TMA unit (coalesced); act: 0 none, 2 gelu
+  // bf16-output token GEMM, result written by the TMA unit (coalesced); act: 0 none, 2 gelu. The whole 256x256 weight block of
+  // a column tile stays in shared memory: on CTA pairs (gemm_pair_tcgen05_kernel) QKV took 1.91 ms instead of 1.25 and the
+  // out-projection 0.64 instead of 0.48 (10 000 clips).
   auto token_gemm_bf16 = [&](const __nv_bfloat16* A, int64_t M, int K, const CUtensorMap& tb, int N, const float* bias, int act,
-                             __nv_bfloat16* out, const CUtensorMap* tb_half = nullptr) -> int {
+                             __nv_bfloat16* out) -> int {
     CUtensorMap tma;
     if (make_tmap_rows_bf16(&tma, A, (uint64_t)M, (uint64_t)K, (uint64_t)K, 128, 64)) return fail("tensor map encode failed (tokens)");
     EpiBiasActTma<true>::Params ep{};
     if (make_tmap_out(&ep.tmap_out, out, (uint64_t)M, (uint64_t)N, true)) return fail("tensor map encode failed (token out)");
     ep.bias = bias; ep.N = N; ep.act = act;
     GemmShape s = plain_shape(M, N, K, 256, 64, 32);
-    if (tb_half && (g_pair_gemm & 2)) {   // CTA pairs: one M256 N256 UMMA per K step, 32 KB per stage
-      VFP_CUDA((launch_gemm_pair<64, 6, EpiBiasActTma<true>>(tma, *tb_half, s, ep, st)));
-    } else if (K == 256) {
-      VFP_CUDA((launch_gemm_bres<256, 64, 4, 4, EpiBiasActTma<true>>(tma, tb, s, ep, st)));
-    } else {
-      VFP_CUDA((launch_gemm<256, 64, 4, EpiBiasActTma<true>>(tma, tb, s, ep, st)));
-    }
+    VFP_CUDA((launch_gemm_bres<256, 64, 4, 4, EpiBiasActTma<true>>(tma, tb, s, ep, st)));
     return 0;
   };
   {  // fp32 stream written through the TMA store path (row-per-thread fp32 stores touch 32 lines per instruction)
@@ -894,7 +841,7 @@ int forward_pass(const vfp_weights* w, const FrameSrc* src, int frame_dtype, boo
       if (make_tmap_rows_f32(&tp.tmap_x, bufs[blk], (uint64_t)F, kDim, kTc2Rows)) return fail("tensor map encode failed (temporal conv)");
       tp.tok_pos = tok_pos; tp.tok_len = tok_len; tp.w = w->tc_w[blk]; tp.bias = w->tc_b[blk]; tp.y = bufs[blk + 1];
       tp.n_tokens = (int)F; tp.n_tiles = (int)((F + kTc2Tok - 1) / kTc2Tok);
-      const int grid = std::min(tp.n_tiles, 2 * persistent_grid());
+      const int grid = std::min(tp.n_tiles, 2 * device_sm_count());
       VFP_CUDA(launch_kernel(temporal_conv_tma_kernel, dim3((unsigned)grid), dim3(kTc2Threads), kTc2SmemBytes, st, tp));
     }
     g_prof.mark(kStTemporalConv, st);
@@ -913,31 +860,26 @@ int forward_pass(const vfp_weights* w, const FrameSrc* src, int frame_dtype, boo
     const AttnBlockWeights& a = w->attn[b];
     VFP_CUDA(launch_kernel(add_layernorm_bf16_kernel, dim3(ln_grid), dim3(256), 0, st, xa, b > 0 ? delta : nullptr, b > 0 ? delta_f : nullptr, a.ln1_w, a.ln1_b, xn, (int)F, 1));
     g_prof.mark(kStLayerNorm, st);
-    if (token_gemm_bf16(xn, F, kDim, a.tm_qkv, 3 * kDim, a.bqkv, 0, qkv, &a.tm_qkv_h)) return 1;
+    if (token_gemm_bf16(xn, F, kDim, a.tm_qkv, 3 * kDim, a.bqkv, 0, qkv)) return 1;
     g_prof.mark(kStQkv, st);
     if (g_attention_tc) {
-      const int grid = std::min(atc.n_units, 2 * persistent_grid());
+      const int grid = std::min(atc.n_units, 2 * device_sm_count());
       VFP_CUDA(launch_kernel(attention_tc_kernel, dim3((unsigned)grid), dim3(kAtcThreads), kAtcSmemBytes, st, atc));
     } else {
       VFP_CUDA(launch_kernel(attention_fa_kernel, dim3((unsigned)n_items), dim3(kAttThreads), kAttSmemBytes, st, qkv, att_items, att, (int)F));
     }
     g_prof.mark(kStAttention, st);
-    if (token_gemm_bf16(att, F, kDim, a.tm_o, kDim, a.bo, 0, delta, &a.tm_o_h)) return 1;
+    if (token_gemm_bf16(att, F, kDim, a.tm_o, kDim, a.bo, 0, delta)) return 1;
     g_prof.mark(kStOutProj, st);
     VFP_CUDA(launch_kernel(add_layernorm_bf16_kernel, dim3(ln_grid), dim3(256), 0, st, xa, delta, (const __nv_bfloat16*)nullptr, a.ln2_w, a.ln2_b, xn, (int)F, 0));
     g_prof.mark(kStLayerNorm, st);
-    if (g_ffn_mode == 0) {
-      if (token_gemm_bf16(xn, F, kDim, a.tm_w1, 4 * kDim, a.b1, 2, hbuf)) return 1;
-      g_prof.mark(kStMlp1, st);
-      if (token_gemm_bf16(hbuf, F, 4 * kDim, a.tm_w2, kDim, a.b2, 0, delta_f)) return 1;
-      g_prof.mark(kStMlp2, st);
-    } else {   // both GEMMs in one kernel on CTA pairs, the hidden activation stays on the SM (ffn_kernel.cuh)
+    {   // both GEMMs in one kernel on CTA pairs, the hidden activation stays on the SM (ffn_kernel.cuh)
       FfnParams fp{};
       if (make_tmap_rows_bf16(&fp.tmap_x, xn, (uint64_t)F, kDim, kDim, 128, 64)) return fail("tensor map encode failed (feed-forward)");
       fp.tmap_w1 = a.tm_w1_ffn; fp.tmap_w2 = a.tm_w2_ffn;
       if (make_tmap_out(&fp.tmap_out, delta_f, (uint64_t)F, kDim, true)) return fail("tensor map encode failed (feed-forward out)");
       fp.b1 = a.b1; fp.b2 = a.b2; fp.M = (int)F; fp.pair_tiles = (int)((F + 255) / 256);
-      const int grid = 2 * std::min(fp.pair_tiles, persistent_grid() / 2);
+      const int grid = 2 * std::min(fp.pair_tiles, device_sm_count() / 2);
       VFP_CUDA(ensure_dynamic_smem(reinterpret_cast<const void*>(ffn_pair_kernel<5>), FfnSmem<5>::kTotal));
       VFP_CUDA(launch_kernel_cluster(2, ffn_pair_kernel<5>, dim3(grid), dim3(kFfnThreads), FfnSmem<5>::kTotal, st, fp));
       g_prof.mark(kStFfn, st);
@@ -1069,15 +1011,8 @@ size_t frame_bytes_of(int frame_dtype) {
 // every bf16 screen row is a whole number of 32-byte sectors). The screen runs ceil(dim / 64) K blocks of 64 columns.
 bool search_dim_ok(int dim) { return dim >= 16 && dim <= 512 && dim % 16 == 0; }
 
-// Stages of the CTA-pair join kernel's database ring: 8 up to KB = 6; above that the resident query rows (16 KB per K block)
-// leave room for 14 - KB stages of 16 KB within the 227 KB a block may have.
-template <int KB>
-cudaError_t launch_join_ares(bool pairs, const CUtensorMap& ta, const CUtensorMap& tb, const AresShape& s,
-                             const EpiJoinThreshold::Params& ep, cudaStream_t st) {
-  if (pairs) return launch_gemm_ares2<(KB <= 6 ? 8 : 14 - KB), KB, EpiJoinThreshold>(ta, tb, s, ep, st);
-  if constexpr (KB <= 4) return launch_gemm_ares<5, KB, EpiJoinThreshold>(ta, tb, s, ep, st);
-  return cudaErrorInvalidValue;   // 32 KB of resident query rows per K block: KB > 4 takes the streamed kernel
-}
+// Database column tiles (of kAres2BlockN = 256 rows) per L2 panel of the join: 65 536 rows, 32 MB of bf16 at dim 256.
+constexpr int kJoinPanelTiles = 256;
 
 }  // namespace
 
@@ -1174,57 +1109,46 @@ int vfp_join_threshold(const float* q, const float* db, int64_t n_q, int64_t n_d
   f32_to_bf16_kernel<<<(unsigned)((q8 + 255) / 256), 256, 0, st>>>(q, qbf, q8);
   if (!self_join) f32_to_bf16_kernel<<<(unsigned)((db8 + 255) / 256), 256, 0, st>>>(db, dbbf, db8);
   // a self join's score matrix is symmetric: screen the upper triangle only, the re-score kernel emits both orders
-  const int tri = (self_join && g_join_symmetric) ? 1 : 0;
+  const int tri = self_join ? 1 : 0;
   EpiJoinThreshold::Params ep{};
   ep.thr = thr - screen_margin;
   ep.q_rows = n_q; ep.db_rows = n_db; ep.q_row0 = q_row0;
   ep.out_i = cand_i; ep.out_j = cand_j; ep.out_s = cand_s; ep.count = cand_count; ep.capacity = cand_cap;
   // The screen operands are the unpadded bf16 rows: the tensor maps have an inner extent of dim columns and a 2 * dim-byte
   // pitch, and TMA zero-fills the columns past dim in the last 64-column K block.
+  // A-resident, panel-major schedule on CTA pairs (cta_group::2 UMMAs, gemm_sm100.cuh)
   CUtensorMap ta, tb;
-  if (g_join_kernel == 2 || (g_join_kernel == 1 && kb <= 4)) {   // A-resident, panel-major schedule (gemm_sm100.cuh); 2 = CTA pairs (cta_group::2 UMMAs)
-    if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, dim, dim, 128, 64) ||
-        make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, dim, dim, 128, 64))
-      return fail("vfp_join_threshold: tensor map encode failed");
-    const bool pairs = g_join_kernel == 2;
-    AresShape s{};
-    s.block_n = pairs ? kAres2BlockN : kAresBlockN;
-    s.m_super = (int)((n_q + kAresMT * kBlockM - 1) / (kAresMT * kBlockM));   // 256 query rows per work item in both kernels
-    s.n_tiles = (int)((n_db + s.block_n - 1) / s.block_n);
-    // a panel of <= 65 536 database rows (32 MB of bf16) stays in L2 while every query super-tile passes over it; small
-    // problems get shorter panels so that there are enough items to balance the SMs
-    int panel = g_join_panel_tiles * kAresBlockN / s.block_n;
-    const int workers = pairs ? persistent_grid() / 2 : persistent_grid();
-    while (panel > 8 && (long long)s.m_super * ((s.n_tiles + panel - 1) / panel) < 16LL * workers) panel /= 2;
-    s.panel_tiles = panel;
-    s.n_panels = (s.n_tiles + panel - 1) / panel;
-    s.tri = tri;
-    s.q_row0 = 0;   // tri compares LOCAL row and column indices: q and db are the same matrix
-    ep.tri = tri;
-    cudaError_t e = cudaErrorInvalidValue;
-    switch (kb) {
-      case 1: e = launch_join_ares<1>(pairs, ta, tb, s, ep, st); break;
-      case 2: e = launch_join_ares<2>(pairs, ta, tb, s, ep, st); break;
-      case 3: e = launch_join_ares<3>(pairs, ta, tb, s, ep, st); break;
-      case 4: e = launch_join_ares<4>(pairs, ta, tb, s, ep, st); break;
-      case 5: e = launch_join_ares<5>(pairs, ta, tb, s, ep, st); break;
-      case 6: e = launch_join_ares<6>(pairs, ta, tb, s, ep, st); break;
-      case 7: e = launch_join_ares<7>(pairs, ta, tb, s, ep, st); break;
-      case 8: e = launch_join_ares<8>(pairs, ta, tb, s, ep, st); break;
-    }
-    VFP_CUDA(e);
-  } else {
-    if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, dim, dim, 128, 64) ||
-        make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, dim, dim, 256, 64))
-      return fail("vfp_join_threshold: tensor map encode failed");
-    GemmShape s = plain_shape(n_q, 0, kb * 64, 256, 64, 32);
-    s.n_tiles = (int)((n_db + 255) / 256);
-    // L2 prefetch of the database tiles: +22 % at 2 M rows, +14 % at 1 M, but -7 % while the bf16 database (512 B per row)
-    // still fits the 126 MB L2 (262 144 rows), where it is only extra traffic
-    s.b_prefetch_tiles = (size_t)n_db * row_bytes > ((size_t)160 << 20) ? g_join_prefetch : 0;
-    ep.tri = tri;   // this kernel visits every tile; the epilogue still drops what lies below the diagonal
-    VFP_CUDA((launch_gemm<256, 64, 4, EpiJoinThreshold>(ta, tb, s, ep, st)));
+  if (make_tmap_rows_bf16(&ta, qbf, (uint64_t)n_q, dim, dim, 128, 64) ||
+      make_tmap_rows_bf16(&tb, dbbf, (uint64_t)n_db, dim, dim, 128, 64))
+    return fail("vfp_join_threshold: tensor map encode failed");
+  AresShape s{};
+  s.block_n = kAres2BlockN;
+  s.m_super = (int)((n_q + kAresMT * kBlockM - 1) / (kAresMT * kBlockM));   // 256 query rows per work item
+  s.n_tiles = (int)((n_db + s.block_n - 1) / s.block_n);
+  // a panel of <= 65 536 database rows (32 MB of bf16) stays in L2 while every query super-tile passes over it; small
+  // problems get shorter panels so that there are enough items to balance the SMs
+  int panel = kJoinPanelTiles;
+  const int workers = device_sm_count() / 2;
+  while (panel > 8 && (long long)s.m_super * ((s.n_tiles + panel - 1) / panel) < 16LL * workers) panel /= 2;
+  s.panel_tiles = panel;
+  s.n_panels = (s.n_tiles + panel - 1) / panel;
+  s.tri = tri;
+  s.q_row0 = 0;   // tri compares LOCAL row and column indices: q and db are the same matrix
+  ep.tri = tri;
+  // Stages of the database ring: 8 up to kb = 6; above that the resident query rows (16 KB per K block) leave room for
+  // 14 - kb stages of 16 KB within the 227 KB a block may have.
+  cudaError_t e = cudaErrorInvalidValue;
+  switch (kb) {
+    case 1: e = launch_gemm_ares2<8, 1, EpiJoinThreshold>(ta, tb, s, ep, st); break;
+    case 2: e = launch_gemm_ares2<8, 2, EpiJoinThreshold>(ta, tb, s, ep, st); break;
+    case 3: e = launch_gemm_ares2<8, 3, EpiJoinThreshold>(ta, tb, s, ep, st); break;
+    case 4: e = launch_gemm_ares2<8, 4, EpiJoinThreshold>(ta, tb, s, ep, st); break;
+    case 5: e = launch_gemm_ares2<8, 5, EpiJoinThreshold>(ta, tb, s, ep, st); break;
+    case 6: e = launch_gemm_ares2<8, 6, EpiJoinThreshold>(ta, tb, s, ep, st); break;
+    case 7: e = launch_gemm_ares2<7, 7, EpiJoinThreshold>(ta, tb, s, ep, st); break;
+    case 8: e = launch_gemm_ares2<6, 8, EpiJoinThreshold>(ta, tb, s, ep, st); break;
   }
+  VFP_CUDA(e);
   rescore_pairs_kernel<<<device_sm_count() * 4, 256, 0, st>>>(q, db, dim, q_row0, cand_i, cand_j, cand_count, cand_cap, thr,
                                                               out_i, out_j, out_s, counts, capacity, tri);
   // counts[1] = candidate count (device-side copy so the caller reads both with one transfer)
